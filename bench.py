@@ -26,6 +26,7 @@ One JSON line on stdout (rank 0).  With the default workload the line also carri
 c4 rollouts strong, c5 weak), so that the driver's BENCH / SCALE files see every config.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -269,6 +270,18 @@ class Workload:
     supports_f64 = False
     e2e_api = None
     units = 0  # units processed by THIS rank in one step
+    stateful = False  # a step advances a state that the next step reads
+
+    @classmethod
+    def reproducible(cls, args):
+        """Whether the timed steps start from the same inputs in every run with the same arguments.  The untimed warm-up
+        before them runs until the clock sampler has delivered samples, a run-dependent number of steps: a stateful step
+        is reproducible only when launched as a graph, whose input buffers restore_inputs() resets after that warm-up."""
+        return not cls.stateful or (cls.use_graph and args.launch != "stream" and hasattr(cls, "restore_inputs"))
+
+    def outputs(self):
+        """name -> device tensor: what a caller of the timed path received from the last step."""
+        raise NotImplementedError
 
     def __init__(self, args, rank, world, dev):
         self.args, self.rank, self.world, self.dev = args, rank, world, dev
@@ -329,6 +342,7 @@ class CartPoleStep(Workload):
     cpu_kind = "c2"
     supports_f64 = True
     inst_per_unit = 165.8  # 32 x smsp__inst_executed / envs, packed f32x2 (ncu, profiles/r02_ncu_full_c2.txt: 5 432 964 warp instructions per 2^20-env launch)
+    stateful = True
 
     def synth(self, seed):
         return synth_cartpole(self.n_envs, seed)
@@ -355,7 +369,11 @@ class CartPoleStep(Workload):
 
     def step(self, i):
         j = i % len(self.envs)
-        self.envs[j].step(self.acts[j])
+        self.out = self.envs[j].step(self.acts[j])
+
+    def outputs(self):
+        obs, reward, terminated = self.out[:3]
+        return {"obs": obs, "reward": reward, "terminated": terminated}
 
     def restore_inputs(self):
         """Put the synthetic states of SURVEY 8(d) back into the buffers the first timed step of every env reads (outside the
@@ -475,6 +493,9 @@ class Scoring(Workload):
 
     def step(self, i):
         self.out = self.env.get_batch_reward_terminal(self.obs, self.pre, self.act)
+
+    def outputs(self):
+        return {"reward": self.out[0], "terminated": self.out[1]}
 
     def setup_e2e(self):
         import torch
@@ -626,6 +647,7 @@ class ChargedBall(Workload):
     alg_fp64_ops = 20 + 4 * 20 + 10 + 2 * 10
     cpu_kind, cpu_sample = "c4", 1 << 20
     supports_f64 = True
+    stateful = True
 
     @classmethod
     def _total(cls, args):
@@ -710,6 +732,10 @@ class ScoringSweep(Workload):
         self.o1 = self.hop.get_batch_reward_terminal(*self.data[0])
         self.o2 = self.chee.get_batch_reward_terminal(*self.data[1])
         self.cp.unfreeze()
+
+    def outputs(self):
+        return {"hopper_reward": self.o1[0], "hopper_terminated": self.o1[1],
+                "halfcheetah_reward": self.o2[0], "halfcheetah_terminated": self.o2[1]}
 
     def setup_e2e(self):
         import torch
@@ -831,6 +857,7 @@ class CartPoleRollout(Workload):
     inst_per_unit = 185.8  # thread-level SASS instructions per env-step incl. in-kernel resets (ncu, profiles/r02_launches_rollout.csv; 247.1 before the spare reset samples)
     cpu_kind = "c2"
     e2e_max_steps = 5
+    stateful = True
 
     @classmethod
     def _horizon(cls, args):
@@ -926,6 +953,7 @@ class ChargedBallRollout(Workload):
     inst_per_unit = 139.7  # warp-level SASS instructions per env-step, all three divergent paths issued (ncu, profiles/r02_launches_c4_rollout.csv: mean of two consecutive 200-step launches, 128.1 from the reset state and 151.3 after it; 166.0 in round 1)
     cpu_kind, cpu_sample = "c4", 1 << 20
     e2e_max_steps = 5
+    stateful = True
 
     @classmethod
     def _total(cls, args):
@@ -1064,13 +1092,18 @@ class ClockSampler(threading.Thread):
         super().__init__(daemon=True)
         self.index, self.rows, self.stop_flag = index, [], False
         self.proc = None
-
-    def run(self):
-        try:
+        try:  # started here rather than in run(), so that finish() always finds the process it has to stop
             self.proc = subprocess.Popen(
                 ["nvidia-smi", f"--id={self.index}", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "20"],
                 stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True,
             )
+        except Exception:
+            pass
+
+    def run(self):
+        if self.proc is None:
+            return
+        try:
             for ln in self.proc.stdout:
                 if self.stop_flag:
                     break
@@ -1097,9 +1130,16 @@ class ClockSampler(threading.Thread):
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": mx or None, "reasons": sorted(reasons), "samples": len(sm)}
 
     def finish(self):
+        """Stop nvidia-smi and reap it: a child left unreaped when bench.py exits stays behind as a zombie.  Safe to call
+        more than once (run_ours also registers it with atexit, for runs that end in an error)."""
         self.stop_flag = True
         if self.proc is not None:
             self.proc.terminate()
+            try:
+                self.proc.wait(timeout=10)
+            except subprocess.TimeoutExpired:
+                self.proc.kill()
+                self.proc.wait()
 
 
 def measured_peaks():
@@ -1173,9 +1213,10 @@ def math_model(wl, units, seconds, sm_mhz, peak_gbs):
     return out
 
 
-def measure(wl, ctx, K, W, args, want_e2e=True):
+def measure(wl, ctx, K, W, args, want_e2e=True, keep_outputs=False):
     """One workload: W warm-up steps, exactly K timed steps (barrier + synchronize on both sides, CUDA events on the
-    launching stream, max over ranks), the dominant-kernel roofline, the end-to-end leg.  Returns the record."""
+    launching stream, max over ranks), the dominant-kernel roofline, the end-to-end leg.  Returns the record.
+    keep_outputs: copy the last timed step's outputs to the host as wl.last_outputs."""
     import torch
     import torch.distributed as dist
 
@@ -1279,6 +1320,8 @@ def measure(wl, ctx, K, W, args, want_e2e=True):
     torch.cuda.synchronize()
     if graph is None:
         launches = _lib.launch_count - launches0
+    if keep_outputs:  # before the e2e leg below steps the same envs again
+        wl.last_outputs = {k: v.cpu() for k, v in wl.outputs().items()}
     if world > 1:
         dist.barrier()
     ms_outer = ev0.elapsed_time(ev1)
@@ -1421,6 +1464,28 @@ def measure(wl, ctx, K, W, args, want_e2e=True):
     return rec
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(outs, directory):
+    """--dump-outputs: every output as <directory>/<name>.npy, float64 where the path computed float64, else float32 (flags
+    as 0 / 1).  Above DUMP_BYTES in all, the arrays are cut to one fixed, seeded sample of rows (the same rows of every array
+    with the same row count), so that runs with the same arguments can be compared output for output."""
+    arrays = {k: v.numpy() for k, v in outs.items()}
+    arrays = {k: a.astype(np.float64 if a.dtype == np.float64 else np.float32) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        rows = {}
+        for k, a in arrays.items():
+            n = a.shape[0]
+            if n not in rows:
+                rows[n] = np.sort(np.random.default_rng(0).choice(n, n * DUMP_BYTES // total, replace=False))
+            arrays[k] = a[rows[n]]
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), a)
+
+
 SECONDARY_N1 = [("c1", "f32"), ("c2_f64", "f64"), ("c3_hopper", "f32"), ("c3_halfcheetah", "f32"), ("c3_hopper_seq", "f32"),
                 ("c3_halfcheetah_seq", "f32"), ("c4", "f32"), ("c4_rollout", "f32"), ("c5", "f32"), ("c5_seq", "f32")]
 SECONDARY_MULTI = [("c4", "f32"), ("c4_rollout", "f32"), ("c5", "f32"), ("c5_seq", "f32")]
@@ -1455,11 +1520,14 @@ def run_ours(args):
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler is not None:
         sampler.start()
+        atexit.register(sampler.finish)
         time.sleep(0.3)
     ctx = Ctx(rank, world, local, dev, sampler)
     K, W = args.steps, max(args.warmup, 3)
     wl = WORKLOADS[args.workload](args, rank, world, dev)
-    line = measure(wl, ctx, K, W, args)
+    line = measure(wl, ctx, K, W, args, keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl.last_outputs, args.dump_outputs)
     # ---------------- CPU baseline on this box's host cores (bounded sample; oracle = the thing timed beside us)
     if rank == 0 and world == 1 and not args.no_cpu:
         n_s = wl.cpu_sample
@@ -1565,6 +1633,9 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--total-log2", type=int, default=0, help="c4 only: log2 of the total env count (default 26)")
     ap.add_argument("--horizon", type=int, default=None, help="rollout workloads: env-steps per launch (default 100; 32 with records)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them returned (rank 0's shard) as DIR/<name>.npy, "
+                         "at most 64 MB in all (a fixed, seeded sample of rows beyond that)")
     args = ap.parse_args()
     args.horizon_set = args.horizon is not None
     if args.horizon is None:
@@ -1572,6 +1643,12 @@ def main():
     args.secondary = args.workload is None and not args.no_secondary and args.impl == "ours" and args.dtype == "f32"
     if args.workload is None:
         args.workload = "c2"
+    if args.dump_outputs:
+        if args.impl != "ours":
+            raise SystemExit("bench.py: --dump-outputs writes what the GPU path computed (--impl ours)")
+        if not WORKLOADS[args.workload].reproducible(args):
+            raise SystemExit(f"bench.py: --dump-outputs: the timed steps of {args.workload} (launched this way) start from a state the "
+                             "untimed warm-up advanced by a run-dependent number of steps, so their outputs would differ from run to run")
     if args.steps is None:
         args.steps = 2000 if WORKLOADS[args.workload].use_graph else 20
         if args.impl == "reference":

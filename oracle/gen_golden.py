@@ -190,7 +190,9 @@ def gen_scoring():
 
 def gen_charged_ball():
     """Drive the reference helpers (charged_ball.py:54-82) on hand-built objects (the class is
-    not constructible, SURVEY.md 0.7).  24 envs x 256 steps per config, full state trajectories."""
+    not constructible, SURVEY.md 0.7).  24 envs x 256 steps per config, full state trajectories, of which the first
+    KEEP_STEPS steps of every third env are stored (a small file; envs 3 and 15 among them start fast)."""
+    KEEP_STEPS, KEEP_ENVS = 160, slice(0, 24, 3)
     out = {}
     for continuous in (False, True):
         for fr in (1, 3):
@@ -221,7 +223,8 @@ def gen_charged_ball():
                     circle[t + 1, e] = env.state["circle_state"]
                     free[t + 1, e] = env.state["free_state"]
             tag = f"{'cont' if continuous else 'disc'}_fr{fr}"
-            out[f"{tag}_action"] = actions
+            out[f"{tag}_action"] = actions[:KEEP_STEPS, KEEP_ENVS]
+            on, circle, free = on[: KEEP_STEPS + 1, KEEP_ENVS], circle[: KEEP_STEPS + 1, KEEP_ENVS], free[: KEEP_STEPS + 1, KEEP_ENVS]
             out[f"{tag}_on"] = on
             out[f"{tag}_circle"] = circle
             out[f"{tag}_free"] = free
