@@ -588,20 +588,23 @@ def score_seq(env, params: _lib.ScoringParams, obs_seq, action=None, group=None)
         raise ValueError(f"obs_seq must be [T+1, n, {d}], got {tuple(s.shape)}")
     T, n = s.shape[0] - 1, s.shape[1]
     needs_pre = family in (_lib.HOPPER, _lib.HALFCHEETAH)
-    sumsq = None
+    a = sumsq = None
     if needs_pre:
         if action is None:
             raise TypeError("get_batch_reward of this env needs the actions")
         a, _ = env._to_device(action, env.dtype)
         if a.shape[0] != T or a.shape[1] != n:
             raise ValueError(f"action must be [T={T}, n={n}, A], got {tuple(a.shape)}")
+    if (n * d * s.element_size()) % 16 != 0:
+        # rows of t >= 1 would lose the loader's alignment: score the flat views, whose pass computes the sum of squares
+        r, dn, _ = score(env, params, s[1:].reshape(T * n, d), s[:-1].reshape(T * n, d).clone(),
+                         a.reshape(T * n, -1) if needs_pre else None, group=group)
+        return r.reshape(T, n, 1), dn.reshape(T, n, 1), was_np
+    if needs_pre:
         sumsq = _sumsq(env, _aligned16(a), group)
     s = _aligned16(s)
     reward = torch.empty((T, n, 1), dtype=env.dtype, device=env.device)
     done = torch.empty((T, n, 1), dtype=torch.uint8, device=env.device)
-    if (n * d * s.element_size()) % 16 != 0:  # rows of t >= 1 would lose the loader's alignment: score the flat views
-        r, dn, _ = score(env, params, s[1:].reshape(T * n, d), s[:-1].reshape(T * n, d).clone(), a if needs_pre else None, group=group)
-        return r.reshape(T, n, 1), dn.reshape(T, n, 1), was_np
     env._call(
         "emei_reward_terminal_seq", s.data_ptr(), reward.data_ptr(), done.data_ptr(),
         env.stats.data_ptr() if getattr(env, "accumulate_scoring_stats", False) else None,
