@@ -15,6 +15,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .engine import HostStaging, action_rule
 
 
 class Freezable:
@@ -70,6 +71,17 @@ class EmeiEnv(Freezable):
         self._seed = 0
         self._reset_count = 0
         self._rollout_epoch = -1  # resets since the last explicit seed (0 = the seeded one): keys the rollout / noise streams
+
+    # ------------------------------------------------------------------ engine protocol (engine.py)
+    _engine = None  # the device-buffer owner of an env with a step kernel
+
+    def _ensure_engine(self):
+        """The env's engine, built on first use where the subclass builds it lazily; None: no dynamics kernel."""
+        return self._engine
+
+    def _next_obs_noise(self, advance: int = 1):
+        """NoiseParams of the next step call (obs_noise_params), or None: no state noise."""
+        return None
 
     # ------------------------------------------------------------------ device plumbing
     @property
@@ -214,8 +226,8 @@ class EmeiEnv(Freezable):
         Returns a dict with those records (if any) and ``stats``: device double[6] = [sum of rewards,
         #terminated, #truncated, #episodes finished, sum of finished returns, sum of finished lengths];
         ``rollout_info(stats)`` turns it into the reference's avg_reward / avg_length / total_episode_num."""
-        eng = getattr(self, "_ensure_engine", lambda: self._engine)()
-        if eng is None or not hasattr(eng, "rollout"):
+        eng = self._ensure_engine()
+        if eng is None:
             raise NotImplementedError(f"{type(self).__name__} has no fused rollout kernel")
         assert self.state is not None, "Call reset before using rollout."
         if actions is not None and not record:
@@ -237,29 +249,10 @@ class EmeiEnv(Freezable):
         rp.seed_action = (self._seed * 0xD1B54A32D192ED03 + 0x14057B7EF767814F + epoch * 0xE7037ED1A0B428DB) & 0xFFFFFFFFFFFFFFFF
         a = None
         if actions is not None:
-            # same dtype / range rules as step() (engine.normalise_action; base_control.py:62-66)
-            a, _ = self._to_device(actions)
-            cont = len(self.action_space.shape) > 0
-            if a.dtype == torch.bool:
-                a = a.view(torch.uint8)
-            if cont:
-                if a.dtype not in (torch.float32, torch.float64):
-                    a = a.to(torch.float32)
-            else:
-                if a.dtype.is_floating_point:
-                    raise AssertionError(f"actions of dtype {a.dtype} invalid: discrete action space needs integers")
-                if a.dtype not in (torch.uint8, torch.int32, torch.int64):
-                    a = a.to(torch.int64)
-            if getattr(self, "validate_actions", False):  # device-side range check: one sync, off by default
-                if cont:
-                    lo, hi = float(self.action_space.low.min()), float(self.action_space.high.max())
-                    ok = bool(((a >= lo) & (a <= hi)).all())
-                else:
-                    ok = bool(((a >= 0) & (a < self.action_space.n)).all())
-                assert ok, "teacher-forced actions outside the action space"
+            a = action_rule(self, self._to_device(actions)[0], len(self.action_space.shape) > 0)
         stats = torch.zeros(6, dtype=torch.float64, device=self.device)
         # obs_noise_params (mujoco_env.py:98-104): the step counter of the noise stream continues through the rollout
-        noise = getattr(self, "_next_obs_noise", lambda advance=1: None)(advance=int(horizon))
+        noise = self._next_obs_noise(advance=int(horizon))
         out = eng.rollout(rp, a, bool(record), stats, noise=noise)
         out["stats"] = stats
         return out
@@ -337,10 +330,6 @@ class EmeiEnv(Freezable):
         into pinned staging buffers, one stream synchronise.  The returned arrays are views of those
         staging buffers (valid until the next ``step_host``).  ``outputs``: subset of ("obs", "reward", "done") to
         download (default all, the reference's contract); the rest stays on the device and comes back as None."""
-        from .engine import HostStaging
-
-        if getattr(self, "_obs_noise_on", lambda: False)() and not hasattr(self._engine, "step_range"):
-            raise NotImplementedError("obs_noise_params != 0 with step_host: inverted pendulum only (emei_ip_step_noisy)")
         if getattr(self, "_staging", None) is None:
             self._staging = HostStaging(self)
         return self._staging.step(action, outputs)

@@ -5,6 +5,7 @@ HBM layout (DESIGN.md section 3):
   cart-pole / IP : state  [B,4] row-major (one 128-bit row per env), ping-pong pair of buffers;
                    IP keeps a separate obs buffer (theta wrapped) because the reference wraps only
                    the observation copy (inverted_pendulum.py:45-49).
+  I2P            : the same with [B,6] rows and obs buffers (RowStateEngine serves all three).
   charged ball   : on_circle uint8[B], circle [B,2], free [B,4] (= observation), updated in place.
   outputs        : reward [B,1] (engine dtype), done uint8[B,1] viewed as torch.bool.
 """
@@ -28,32 +29,37 @@ _ACTION_KIND = {
 }
 
 
-def normalise_action(env, action, continuous: bool) -> torch.Tensor:
-    """-> contiguous device tensor [num_envs] in one of the encodings of include/emei_b200.h.
-    Mirrors base_control.py:62-66 (int -> array; action_space.contains) for a batch."""
-    n = env.num_envs
-    if isinstance(action, (int, np.integer)) and not continuous:
-        action = torch.full((n,), int(action), dtype=torch.int64)
-    a, _ = env._to_device(action)
-    if a.numel() != n:
-        raise AssertionError(f"{action!r} ({type(action)}) invalid: expected {n} actions, got shape {tuple(a.shape)}")
-    a = a.reshape(n)
+def action_rule(env, a: torch.Tensor, continuous: bool) -> torch.Tensor:
+    """The dtype and range rule of every action entry point (base_control.py:62-66 for a batch): device tensor ``a`` of
+    any shape -> one of the encodings of include/emei_b200.h.  ``bool`` is read as its uint8 bytes."""
+    if a.dtype == torch.bool:
+        a = a.view(torch.uint8)
     if continuous:
         if a.dtype not in (torch.float32, torch.float64):
             a = a.to(torch.float32)
-    else:
-        if a.dtype.is_floating_point:
-            raise AssertionError(f"{action!r} ({type(action)}) invalid: discrete action space needs integers")
-        if a.dtype not in _ACTION_KIND:
-            a = a.to(torch.int64)
+    elif a.dtype.is_floating_point:
+        raise AssertionError(f"actions of dtype {a.dtype} invalid: discrete action space needs integers")
+    elif a.dtype not in _ACTION_KIND:
+        a = a.to(torch.int64)
     if env.validate_actions:  # device-side range check: one sync, off by default
         if continuous:
             lo, hi = float(env.action_space.low.min()), float(env.action_space.high.max())
             ok = bool(((a >= lo) & (a <= hi)).all())
         else:
             ok = bool(((a >= 0) & (a < env.action_space.n)).all())
-        assert ok, f"{action!r} ({type(action)}) invalid"
-    return a.contiguous()
+        assert ok, "actions outside the action space"
+    return a
+
+
+def normalise_action(env, action, continuous: bool, n: int) -> torch.Tensor:
+    """-> contiguous device tensor [n] of one step's actions for a batch of ``n`` rows (int -> array, as
+    base_control.py:62-66; then ``action_rule``)."""
+    if isinstance(action, (int, np.integer)) and not continuous:
+        action = torch.full((n,), int(action), dtype=torch.int64)
+    a, _ = env._to_device(action)
+    if a.numel() != n:
+        raise AssertionError(f"{action!r} ({type(action)}) invalid: expected {n} actions, got shape {tuple(a.shape)}")
+    return action_rule(env, a.reshape(n), continuous).contiguous()
 
 
 class StepOutputs:
@@ -66,8 +72,9 @@ class StepOutputs:
         self.done = [torch.empty((n, 1), dtype=torch.uint8, device=device) for _ in range(2)]
 
 
-class RolloutMixin:
-    """Episode bookkeeping buffers + the call of a fused T-step rollout entry point.
+class Engine:
+    """Base of the engines: episode bookkeeping buffers, the call of a fused T-step rollout entry point and the
+    freeze snapshots of the live state arrays (``_state_arrays``).
 
     float32 without state noise: the packed kernels (emei_cartpole_rollout_f32 / emei_charged_ball_rollout_f32).
     float64 (reference-exact), the inverted double pendulum and obs_noise_params: the reference-arithmetic kernels
@@ -142,28 +149,48 @@ class RolloutMixin:
             rec["timeouts"] = rec["timeouts"].view(torch.bool)
         return rec
 
+    # freeze/unfreeze: device-side copies of the live state arrays (base_control.py:32-36)
+    def snapshot(self) -> tuple:
+        snaps = tuple(torch.empty_like(t) for t in self._state_arrays())
+        self._copy(snaps, self._state_arrays())
+        return snaps
 
-class CartPoleEngine(RolloutMixin):
-    """cart-pole family + analytic inverted pendulum (emei_cartpole_step_*)."""
+    def restore(self, snaps: tuple):
+        self._alloc()
+        self._copy(self._state_arrays(), snaps)
+        self.has_state = True
 
-    def __init__(self, env, params: _lib.CartPoleParams, separate_obs: bool):
+    def _copy(self, dsts, srcs):
+        with torch.cuda.device(self.env.device):
+            for dst, src in zip(dsts, srcs):
+                _lib.call("emei_snapshot_copy", dst.data_ptr(), src.data_ptr(), src.numel() * src.element_size(), self.env._stream())
+
+
+class RowStateEngine(Engine):
+    """State [B, width], one row per env, in a ping-pong pair of buffers; ``separate_obs``: the observation goes to a
+    buffer pair of its own (the pendulums, whose observation wraps the angles), else it is the next state row."""
+
+    def __init__(self, env, params, width: int, separate_obs: bool, step_entry: str, noisy_entry: str):
         self.env = env
         self.params = params
-        self.separate_obs = separate_obs
         self.n = env.num_envs
-        self._bufs = None
-        self._obs = None
-        self._out = None
+        self.obs_dim = width
+        self.separate_obs = separate_obs
+        self._step_entry, self._noisy_entry = step_entry, noisy_entry
+        self._bufs = self._obs = self._out = None
         self._cur = 0
         self.has_state = False
 
     def _alloc(self):
         if self._bufs is None:
             dev, dt = self.env.device, self.env.dtype
-            self._bufs = [torch.empty((self.n, 4), dtype=dt, device=dev) for _ in range(2)]
+            self._bufs = [torch.empty((self.n, self.obs_dim), dtype=dt, device=dev) for _ in range(2)]
             if self.separate_obs:
-                self._obs = [torch.empty((self.n, 4), dtype=dt, device=dev) for _ in range(2)]
+                self._obs = [torch.empty((self.n, self.obs_dim), dtype=dt, device=dev) for _ in range(2)]
             self._out = StepOutputs(self.n, dt, dev)
+
+    def _state_arrays(self):
+        return [self._bufs[self._cur]]
 
     @property
     def state(self) -> Optional[torch.Tensor]:
@@ -172,64 +199,78 @@ class CartPoleEngine(RolloutMixin):
     def set_state(self, state):
         self._alloc()
         s, _ = self.env._to_device(state, self.env.dtype)
-        if tuple(s.shape) != (self.n, 4):
-            raise ValueError(f"state must have shape {(self.n, 4)}, got {tuple(s.shape)}")
+        if tuple(s.shape) != (self.n, self.obs_dim):
+            raise ValueError(f"state must have shape {(self.n, self.obs_dim)}, got {tuple(s.shape)}")
         self._bufs[self._cur].copy_(s)
         self.has_state = True
         self.new_episodes(reseed=False)
 
-    def step(self, action: torch.Tensor, copy_obs: bool, noise: Optional[_lib.NoiseParams] = None):
+    def _launch(self, lo: int, hi: int, src, dst, obs, action, reward, done, stats, noise):
+        """One step launch over rows [lo, hi) of the given arrays.  ``noise``: the step's NoiseParams
+        (obs_noise_params); a range draws the streams of its own global env ids."""
         env = self.env
+        self.params.action_kind = _ACTION_KIND[action.dtype]
+        # byte strides of the arrays, needed for a range only (a whole-batch step is on the host's per-call path)
+        es, ea, er = (src.element_size() * self.obs_dim, action.element_size(), reward.element_size()) if lo else (0, 0, 0)
+        args = (src.data_ptr() + lo * es, dst.data_ptr() + lo * es, (obs.data_ptr() + lo * es) if obs is not None else None,
+                action.data_ptr() + lo * ea, reward.data_ptr() + lo * er, done.data_ptr() + lo, stats, hi - lo,
+                ctypes.byref(self.params))
+        if noise is None:
+            env._call(self._step_entry, *args, env._stream())
+            return
+        if lo:
+            z = _lib.NoiseParams()
+            ctypes.memmove(ctypes.byref(z), ctypes.byref(noise), ctypes.sizeof(z))
+            z.env_offset = noise.env_offset + lo
+            noise = z
+        env._call(self._noisy_entry, *args, ctypes.byref(noise), env._stream())
+
+    def step(self, action: torch.Tensor, copy_obs: bool, noise: Optional[_lib.NoiseParams] = None):
+        """``step_range(0, n)`` + ``flip()``, with the outputs of ``copy_obs`` (fresh tensors) or the ping-pong buffers."""
         self._alloc()
-        src, dst = self._bufs[self._cur], self._bufs[1 - self._cur]
         nxt = 1 - self._cur
-        obs = None
-        if self.separate_obs:
-            obs = self._obs[nxt] if not copy_obs else torch.empty_like(src)
-        elif copy_obs:
-            obs = torch.empty_like(src)
+        src, dst = self._bufs[self._cur], self._bufs[nxt]
+        obs = self._obs[nxt] if self.separate_obs else None
         reward, done = self._out.reward[nxt], self._out.done[nxt]
         if copy_obs:
-            reward, done = torch.empty_like(reward), torch.empty_like(done)
-        self.params.action_kind = _ACTION_KIND[action.dtype]
-        ptrs = (src.data_ptr(), dst.data_ptr(), obs.data_ptr() if obs is not None else None, action.data_ptr(),
-                reward.data_ptr(), done.data_ptr(), env.stats.data_ptr(), self.n, ctypes.byref(self.params))
-        if noise is None:
-            env._call("emei_cartpole_step", *ptrs, env._stream())
-        else:  # obs_noise_params (mujoco_env.py:98-104): Gaussian state noise after every sub-step
-            env._call("emei_ip_step_noisy", *ptrs, ctypes.byref(noise), env._stream())
+            obs, reward, done = torch.empty_like(src), torch.empty_like(reward), torch.empty_like(done)
+        self._launch(0, self.n, src, dst, obs, action, reward, done, self.env.stats.data_ptr(), noise)
         self._cur = nxt
         return (obs if obs is not None else dst), reward, done.view(torch.bool)
 
     def step_range(self, lo: int, hi: int, action: torch.Tensor, reward: torch.Tensor, done: torch.Tensor, obs_out,
                    noise: Optional[_lib.NoiseParams] = None):
         """Launch the step kernel for envs [lo, hi) only (src -> dst of the CURRENT ping-pong pair, no flip):
-        the building block of the chunked host pipeline.  Call ``flip()`` once all ranges are launched.
-        ``noise``: the step's NoiseParams (obs_noise_params); the range draws the streams of its own global env ids."""
-        env = self.env
+        the building block of the chunked host pipeline (``step_host``).  Call ``flip()`` once all ranges are launched."""
         self._alloc()
-        src, dst = self._bufs[self._cur], self._bufs[1 - self._cur]
+        dst = self._bufs[1 - self._cur]
         if self.separate_obs and obs_out is None:
             obs_out = self._obs[1 - self._cur]
-        self.params.action_kind = _ACTION_KIND[action.dtype]
-        es, ea = src.element_size() * 4, action.element_size()
-        ptrs = (src.data_ptr() + lo * es, dst.data_ptr() + lo * es,
-                (obs_out.data_ptr() + lo * es) if obs_out is not None else None, action.data_ptr() + lo * ea,
-                reward.data_ptr() + lo * reward.element_size(), done.data_ptr() + lo, env.stats.data_ptr(), hi - lo,
-                ctypes.byref(self.params))
-        if noise is None:
-            env._call("emei_cartpole_step", *ptrs, env._stream())
-        else:
-            z = _lib.NoiseParams()
-            ctypes.memmove(ctypes.byref(z), ctypes.byref(noise), ctypes.sizeof(z))
-            z.env_offset = noise.env_offset + lo
-            env._call("emei_ip_step_noisy", *ptrs, ctypes.byref(z), env._stream())
+        self._launch(lo, hi, self._bufs[self._cur], dst, obs_out, action, reward, done, self.env.stats.data_ptr(), noise)
         return obs_out if obs_out is not None else dst
 
     def flip(self):
         self._cur = 1 - self._cur
 
-    # ---- fused T-step rollout (emei_cartpole_rollout_f32) ----------------------------------------
+    def next_obs_stateless(self, rows: torch.Tensor, action: torch.Tensor):
+        """get_batch_next_obs: one dynamics step from caller-supplied state rows (any batch size); the engine's own
+        state is untouched."""
+        env = self.env
+        b = rows.shape[0]
+        out = torch.empty_like(rows)
+        obs = torch.empty_like(rows) if self.separate_obs else None
+        reward = torch.empty((b, 1), dtype=env.dtype, device=env.device)
+        done = torch.empty((b, 1), dtype=torch.uint8, device=env.device)
+        self._launch(0, b, rows, out, obs, action, reward, done, None, None)
+        return obs if obs is not None else out
+
+
+class CartPoleEngine(RowStateEngine):
+    """cart-pole family (state = observation) + analytic inverted pendulum (emei_cartpole_step_* / emei_ip_step_noisy_*)."""
+
+    def __init__(self, env, params: _lib.CartPoleParams, separate_obs: bool):
+        RowStateEngine.__init__(self, env, params, 4, separate_obs, "emei_cartpole_step", "emei_ip_step_noisy")
+
     def rollout(self, rp: _lib.RolloutParams, actions, record: bool, rollout_stats: torch.Tensor, noise=None):
         self._alloc()
         state = self._bufs[self._cur]
@@ -240,43 +281,12 @@ class CartPoleEngine(RolloutMixin):
         return self._rollout("emei_cartpole_rollout_ref" + self.env._suffix, [state.data_ptr()], rp, actions, record, rollout_stats,
                              ref=True, extra=(z,))
 
-    def next_obs_stateless(self, obs: torch.Tensor, action: torch.Tensor):
-        """get_batch_next_obs: one dynamics step from caller-supplied observations (any batch size);
-        the engine's own state is untouched."""
-        env = self.env
-        b = obs.shape[0]
-        out = torch.empty_like(obs)
-        obs_out = torch.empty_like(obs) if self.separate_obs else None
-        reward = torch.empty((b, 1), dtype=env.dtype, device=env.device)
-        done = torch.empty((b, 1), dtype=torch.uint8, device=env.device)
-        self.params.action_kind = _ACTION_KIND[action.dtype]
-        env._call(
-            "emei_cartpole_step",
-            obs.data_ptr(), out.data_ptr(), obs_out.data_ptr() if obs_out is not None else None, action.data_ptr(),
-            reward.data_ptr(), done.data_ptr(), None, b, ctypes.byref(self.params), env._stream(),
-        )
-        return obs_out if obs_out is not None else out
 
-    # freeze/unfreeze: device-side snapshot of the live state buffer (base_control.py:32-36)
-    def snapshot(self):
-        src = self._bufs[self._cur]
-        snap = torch.empty_like(src)
-        with torch.cuda.device(self.env.device):
-            _lib.call("emei_snapshot_copy", snap.data_ptr(), src.data_ptr(), src.numel() * src.element_size(), self.env._stream())
-        return snap
+class I2PEngine(RowStateEngine):
+    """analytic inverted double pendulum (emei_i2p_step_*): state [B,6] + observation buffers."""
 
-    def restore(self, snap: torch.Tensor):
-        self._alloc()
-        dst = self._bufs[self._cur]
-        with torch.cuda.device(self.env.device):
-            _lib.call("emei_snapshot_copy", dst.data_ptr(), snap.data_ptr(), snap.numel() * snap.element_size(), self.env._stream())
-        self.has_state = True
-
-
-class I2PEngine(RolloutMixin):
-    """analytic inverted double pendulum (emei_i2p_step_*): state [B,6] ping-pong pair + observation buffers."""
-
-    obs_dim = 6
+    def __init__(self, env, params: _lib.I2PParams):
+        RowStateEngine.__init__(self, env, params, 6, True, "emei_i2p_step", "emei_i2p_step_noisy")
 
     def rollout(self, rp: _lib.RolloutParams, actions, record: bool, rollout_stats: torch.Tensor, noise=None):
         """emei_i2p_rollout_*: the four I2P tasks of zoo/conf/task/BI2P*.yaml through the collection loop of
@@ -289,107 +299,8 @@ class I2PEngine(RolloutMixin):
         return self._rollout("emei_i2p_rollout" + self.env._suffix, [state.data_ptr()], rp, actions, record, rollout_stats,
                              ref=True, extra=(Arr(*mean), Arr(*sigma), z))
 
-    def __init__(self, env, params: _lib.I2PParams):
-        self.env = env
-        self.params = params
-        self.n = env.num_envs
-        self._bufs = self._obs = self._out = None
-        self._cur = 0
-        self.has_state = False
 
-    def _alloc(self):
-        if self._bufs is None:
-            dev, dt = self.env.device, self.env.dtype
-            self._bufs = [torch.empty((self.n, 6), dtype=dt, device=dev) for _ in range(2)]
-            self._obs = [torch.empty((self.n, 6), dtype=dt, device=dev) for _ in range(2)]
-            self._out = StepOutputs(self.n, dt, dev)
-
-    @property
-    def state(self) -> Optional[torch.Tensor]:
-        return self._bufs[self._cur] if self.has_state else None
-
-    def set_state(self, state):
-        self._alloc()
-        s, _ = self.env._to_device(state, self.env.dtype)
-        if tuple(s.shape) != (self.n, 6):
-            raise ValueError(f"state must have shape {(self.n, 6)}, got {tuple(s.shape)}")
-        self._bufs[self._cur].copy_(s)
-        self.has_state = True
-        self.new_episodes(reseed=False)
-
-    def step(self, action: torch.Tensor, copy_obs: bool, noise: Optional[_lib.NoiseParams] = None):
-        env = self.env
-        self._alloc()
-        nxt = 1 - self._cur
-        src, dst = self._bufs[self._cur], self._bufs[nxt]
-        obs, reward, done = self._obs[nxt], self._out.reward[nxt], self._out.done[nxt]
-        if copy_obs:
-            obs, reward, done = torch.empty_like(obs), torch.empty_like(reward), torch.empty_like(done)
-        self.params.action_kind = _ACTION_KIND[action.dtype]
-        ptrs = (src.data_ptr(), dst.data_ptr(), obs.data_ptr(), action.data_ptr(), reward.data_ptr(), done.data_ptr(),
-                env.stats.data_ptr(), self.n, ctypes.byref(self.params))
-        if noise is None:
-            env._call("emei_i2p_step", *ptrs, env._stream())
-        else:
-            env._call("emei_i2p_step_noisy", *ptrs, ctypes.byref(noise), env._stream())
-        self._cur = nxt
-        return obs, reward, done.view(torch.bool)
-
-    def step_range(self, lo: int, hi: int, action: torch.Tensor, reward: torch.Tensor, done: torch.Tensor, obs_out,
-                   noise: Optional[_lib.NoiseParams] = None):
-        """Launch the step kernel for envs [lo, hi) only (src -> dst of the CURRENT ping-pong pair, no flip): the
-        building block of the chunked host pipeline (``step_host``).  Call ``flip()`` once all ranges are launched."""
-        env = self.env
-        self._alloc()
-        nxt = 1 - self._cur
-        src, dst = self._bufs[self._cur], self._bufs[nxt]
-        if obs_out is None:
-            obs_out = self._obs[nxt]
-        self.params.action_kind = _ACTION_KIND[action.dtype]
-        es, ea = src.element_size() * 6, action.element_size()
-        ptrs = (src.data_ptr() + lo * es, dst.data_ptr() + lo * es, obs_out.data_ptr() + lo * es, action.data_ptr() + lo * ea,
-                reward.data_ptr() + lo * reward.element_size(), done.data_ptr() + lo, env.stats.data_ptr(), hi - lo,
-                ctypes.byref(self.params))
-        if noise is None:
-            env._call("emei_i2p_step", *ptrs, env._stream())
-        else:
-            z = _lib.NoiseParams()
-            ctypes.memmove(ctypes.byref(z), ctypes.byref(noise), ctypes.sizeof(z))
-            z.env_offset = noise.env_offset + lo
-            env._call("emei_i2p_step_noisy", *ptrs, ctypes.byref(z), env._stream())
-        return obs_out
-
-    def flip(self):
-        self._cur = 1 - self._cur
-
-    def next_obs_stateless(self, obs: torch.Tensor, action: torch.Tensor):
-        """get_batch_next_obs: one dynamics step from caller-supplied STATES (the 6-d observation of this family
-        does not determine the state: inverted_double_pendulum.py:56-60 is not a bijection); engine untouched."""
-        b = obs.shape[0]
-        out, o2 = torch.empty_like(obs), torch.empty_like(obs)
-        r = torch.empty((b, 1), dtype=obs.dtype, device=obs.device)
-        d = torch.empty((b, 1), dtype=torch.uint8, device=obs.device)
-        self.params.action_kind = _ACTION_KIND[action.dtype]
-        self.env._call("emei_i2p_step", obs.data_ptr(), out.data_ptr(), o2.data_ptr(), action.data_ptr(), r.data_ptr(),
-                       d.data_ptr(), None, b, ctypes.byref(self.params), self.env._stream())
-        return o2
-
-    def snapshot(self):
-        src = self._bufs[self._cur]
-        snap = torch.empty_like(src)
-        with torch.cuda.device(self.env.device):
-            _lib.call("emei_snapshot_copy", snap.data_ptr(), src.data_ptr(), src.numel() * src.element_size(), self.env._stream())
-        return snap
-
-    def restore(self, snap: torch.Tensor):
-        self._alloc()
-        dst = self._bufs[self._cur]
-        with torch.cuda.device(self.env.device):
-            _lib.call("emei_snapshot_copy", dst.data_ptr(), snap.data_ptr(), snap.numel() * snap.element_size(), self.env._stream())
-        self.has_state = True
-
-
-class ChargedBallEngine(RolloutMixin):
+class ChargedBallEngine(Engine):
     """charged ball (emei_charged_ball_step_*): three state arrays updated in place."""
 
     # step_host: the observation is the `free` state array itself, so it needs a copy anyway and kernel-side stores of
@@ -466,21 +377,8 @@ class ChargedBallEngine(RolloutMixin):
     def flip(self):
         pass
 
-    def snapshot(self):
-        out = []
-        with torch.cuda.device(self.env.device):
-            for src in (self.on_circle, self.circle, self.free):
-                snap = torch.empty_like(src)
-                _lib.call("emei_snapshot_copy", snap.data_ptr(), src.data_ptr(), src.numel() * src.element_size(), self.env._stream())
-                out.append(snap)
-        return tuple(out)
-
-    def restore(self, snaps):
-        self._alloc()
-        with torch.cuda.device(self.env.device):
-            for dst, snap in zip((self.on_circle, self.circle, self.free), snaps):
-                _lib.call("emei_snapshot_copy", dst.data_ptr(), snap.data_ptr(), snap.numel() * snap.element_size(), self.env._stream())
-        self.has_state = True
+    def _state_arrays(self):
+        return [self.on_circle, self.circle, self.free]
 
 
 def _aligned16(t: torch.Tensor) -> torch.Tensor:
@@ -611,32 +509,6 @@ def score_seq(env, params: _lib.ScoringParams, obs_seq, action=None, group=None)
         sumsq.data_ptr() if sumsq is not None else None, n, T, ctypes.byref(params), env._stream(),
     )
     return reward, done.view(torch.bool), was_np
-
-
-def time_fused_scoring(env, obs, pre_obs, action, reps=10):
-    """CUDA-event duration (ms per launch) of the fused reward+terminal kernel alone, for the roofline
-    of bench.py: the sum-of-squares pre-pass runs once outside the timed launches."""
-    params = env._scoring_params()
-    b = obs.shape[0]
-    sumsq = torch.zeros(1, dtype=torch.float64, device=env.device)
-    ws = torch.zeros(_lib.SUMSQ_WORKSPACE_BYTES // 8, dtype=torch.float64, device=env.device)
-    env._call("emei_sumsq", action.data_ptr(), action.numel(), sumsq.data_ptr(), ws.data_ptr(), env._stream())
-    reward = torch.empty((b, 1), dtype=env.dtype, device=env.device)
-    done = torch.empty((b, 1), dtype=torch.uint8, device=env.device)
-
-    def launch():
-        env._call("emei_reward_terminal", obs.data_ptr(), pre_obs.data_ptr(), reward.data_ptr(), done.data_ptr(), None,
-                  sumsq.data_ptr(), b, ctypes.byref(params), env._stream())
-
-    launch()
-    torch.cuda.synchronize(env.device)
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for _ in range(reps):
-        launch()
-    e1.record()
-    torch.cuda.synchronize(env.device)
-    return e0.elapsed_time(e1) / reps
 
 
 ZERO_COPY_MAX_ENVS = 65536  # measured: scripts/probe_zero_copy_small.py, profiles/r02_zero_copy_small.txt
@@ -793,7 +665,7 @@ class HostStaging:
             self.a_host.copy_(a)  # host-side cast into the pinned staging buffer (uint8 / float32)
             a_src = self.a_host
         cur = torch.cuda.current_stream(env.device)
-        noise = getattr(env, "_next_obs_noise", lambda: None)()
+        noise = env._next_obs_noise()
         if noise is not None:  # obs_noise_params: the step counter changes every call, so nothing can be baked into a graph
             self._enqueue(a_src, noise)
             eng.flip()

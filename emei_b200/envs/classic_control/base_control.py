@@ -19,10 +19,12 @@ from typing import Optional
 import torch
 
 from ...core import EmeiEnv
+from ...engine import normalise_action, score
 
 
 class BaseControlEnv(EmeiEnv):
     metadata = {"render_modes": [], "render_fps": 50}
+    _continuous = False
 
     def __init__(
         self,
@@ -57,7 +59,6 @@ class BaseControlEnv(EmeiEnv):
             device=device,
             dtype=dtype,
         )
-        self._engine = None  # set by subclasses
 
     # ---- state access -------------------------------------------------------------------------
     @property
@@ -68,7 +69,7 @@ class BaseControlEnv(EmeiEnv):
     @state.setter
     def state(self, value):
         """Host- or device-supplied states (teacher forcing / set_state)."""
-        self._engine.set_state(value)
+        self._ensure_engine().set_state(value)
 
     # ---- freeze / unfreeze ----------------------------------------------------------------------
     def freeze(self) -> None:
@@ -86,17 +87,20 @@ class BaseControlEnv(EmeiEnv):
     def reset(self, *, seed: Optional[int] = None, options: Optional[dict] = None):
         self._reseed(seed)
         self.state = self.get_batch_init_state(self.num_envs)
-        if hasattr(self._engine, "new_episodes"):
-            self._engine.new_episodes(reseed=True)
+        self._engine.new_episodes(reseed=True)
         return self.state.clone(), {}
 
-    def _is_continuous(self) -> bool:
-        return len(self.action_space.shape) > 0
-
     def step(self, action):
-        from ...engine import normalise_action
-
         assert self.state is not None, "Call reset before using step method."
-        a = normalise_action(self, action, self._is_continuous())
+        a = normalise_action(self, action, self._continuous, self.num_envs)
         obs, reward, terminal = self._engine.step(a, self.copy_outputs)
         return obs, reward, terminal, False, {}
+
+    # ---- scoring (the reward and terminal of both families depend on obs only) ------------------------
+    def get_batch_reward(self, obs, pre_obs=None, action=None, state=None, pre_state=None):
+        r, _, was_np = score(self, self._scoring_params(), obs)
+        return self._ret(r, was_np)
+
+    def get_batch_terminal(self, obs, pre_obs=None, action=None, state=None, pre_state=None):
+        _, d, was_np = score(self, self._scoring_params(), obs)
+        return self._ret(d, was_np)

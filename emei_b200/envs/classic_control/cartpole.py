@@ -23,7 +23,6 @@ from .base_control import BaseControlEnv
 
 class BaseCartPoleEnv(BaseControlEnv):
     _variant = None
-    _continuous = False
 
     def __init__(self, freq_rate: int = 1, real_time_scale: float = 0.02, integrator: str = "euler", **kwargs):
         super().__init__(freq_rate=freq_rate, real_time_scale=real_time_scale, integrator=integrator, **kwargs)
@@ -64,20 +63,12 @@ class BaseCartPoleEnv(BaseControlEnv):
         p.x_threshold, p.theta_threshold = float(self.x_threshold), self.theta_threshold_radians
         return p
 
-    def _make_engine(self):
+    def _ensure_engine(self):
         if self._variant is None:
             raise NotImplementedError  # abstract base: reset() raises (test/test_envs/.../test_cartpole.py:4-11)
-        self._engine = CartPoleEngine(self, self._params(), separate_obs=False)
-
-    @property
-    def state(self):
-        return self._engine.state if self._engine is not None else None
-
-    @state.setter
-    def state(self, value):
         if self._engine is None:
-            self._make_engine()
-        self._engine.set_state(value)
+            self._engine = CartPoleEngine(self, self._params(), separate_obs=False)
+        return self._engine
 
     def get_batch_init_state(self, batch_size):
         raise NotImplementedError
@@ -99,14 +90,6 @@ class BaseCartPoleEnv(BaseControlEnv):
         )
         return out
 
-    def get_batch_reward(self, obs, pre_obs=None, action=None, state=None, pre_state=None):
-        r, _, was_np = score(self, self._scoring_params(), obs)
-        return self._ret(r, was_np)
-
-    def get_batch_terminal(self, obs, pre_obs=None, action=None, state=None, pre_state=None):
-        _, d, was_np = score(self, self._scoring_params(), obs)
-        return self._ret(d, was_np)
-
     def get_batch_reward_terminal(self, obs, pre_obs=None, action=None):
         """Additive: both outputs from ONE fused launch."""
         r, d, was_np = score(self, self._scoring_params(), obs)
@@ -115,15 +98,10 @@ class BaseCartPoleEnv(BaseControlEnv):
     def get_batch_next_obs(self, obs, pre_obs=None, action=None, state=None, pre_state=None):
         """core.py:190-193: requires a frozen env; one dynamics step from the given observations."""
         assert self.frozen
-        if self._engine is None:
-            self._make_engine()
+        eng = self._ensure_engine()
         o, was_np = self._to_device(obs, self.dtype)
-        saved, self.num_envs = self.num_envs, o.shape[0]
-        try:
-            a = normalise_action(self, action, self._continuous)
-        finally:
-            self.num_envs = saved
-        return self._ret(self._engine.next_obs_stateless(o, a), was_np)
+        a = normalise_action(self, action, self._continuous, o.shape[0])
+        return self._ret(eng.next_obs_stateless(o, a), was_np)
 
 
 class CartPoleBalancingEnv(BaseCartPoleEnv):

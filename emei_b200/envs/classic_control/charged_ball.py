@@ -8,15 +8,13 @@ observation is ``free`` (:96-97).  Constructor keywords follow the reference: ``
 ``time_step`` (the reference then overwrites time_step with 0.02, :17 -- replicated).
 """
 from ... import _lib, spaces
-from ...engine import ChargedBallEngine, normalise_action, score
+from ...engine import ChargedBallEngine
 from .base_control import BaseControlEnv
 
 import numpy as np
 
 
 class BaseChargedBallEnv(BaseControlEnv):
-    _continuous = False
-
     def __init__(self, freq_rate=1, time_step=0.02, **kwargs):
         BaseControlEnv.__init__(self, freq_rate=freq_rate, **kwargs)
         # the reference intends env_params = (freq_rate, time_step): charged_ball.py:11-12
@@ -78,20 +76,6 @@ class BaseChargedBallEnv(BaseControlEnv):
 
     def transform_obs_to_state(self, batch_obs):
         raise NotImplementedError("the 4-float observation does not determine on_circle (charged_ball.py:99-108)")
-
-    def step(self, action):
-        assert self.state is not None, "Call reset before using step method."
-        a = normalise_action(self, action, self._continuous)
-        obs, reward, terminal = self._engine.step(a, self.copy_outputs)
-        return obs, reward, terminal, False, {}
-
-    def get_batch_reward(self, obs, pre_obs=None, action=None, state=None, pre_state=None):
-        r, _, was_np = score(self, self._scoring_params(), obs)
-        return self._ret(r, was_np)
-
-    def get_batch_terminal(self, obs, pre_obs=None, action=None, state=None, pre_state=None):
-        _, d, was_np = score(self, self._scoring_params(), obs)
-        return self._ret(d, was_np)
 
 
 class ChargedBallCenteringEnv(BaseChargedBallEnv):

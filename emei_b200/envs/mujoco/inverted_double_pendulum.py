@@ -18,13 +18,12 @@ import numpy as np
 import torch
 
 from ... import _lib
-from ...engine import I2PEngine, normalise_action
-from .mujoco_env import EmeiMujocoEnv
+from ...engine import I2PEngine
+from .mujoco_env import AnalyticPendulumEnv, EmeiMujocoEnv
 
 
-class BaseInvertedDoublePendulumEnv(EmeiMujocoEnv):
+class BaseInvertedDoublePendulumEnv(AnalyticPendulumEnv):
     _model = (3, 1, (-1.0, 1.0), [0.0, 0.0, 0.0])  # inverted_double_pendulum.xml:45
-    _family = None
 
     def __init__(self, freq_rate: int = 1, real_time_scale: float = 0.02, integrator="euler",
                  init_noise_params=5e-3, obs_noise_params=0.0, **kwargs):
@@ -53,12 +52,6 @@ class BaseInvertedDoublePendulumEnv(EmeiMujocoEnv):
         self.mass_cart = 1000.0 * (math.pi * 0.1**2 * 0.2 + 4.0 / 3.0 * math.pi * 0.1**3)
         self.mass_pole = 1000.0 * (math.pi * 0.045**2 * 0.6 + 4.0 / 3.0 * math.pi * 0.045**3)
         self.pole_half_length = 0.3
-        self._engine = None
-
-    def _scoring_params(self) -> _lib.ScoringParams:
-        p = EmeiMujocoEnv._scoring_params(self)
-        p.x_left, p.x_right = float(self.jnt_range[0][0]), float(self.jnt_range[0][1])
-        return p
 
     def _params(self) -> _lib.I2PParams:
         p = _lib.I2PParams()
@@ -76,21 +69,8 @@ class BaseInvertedDoublePendulumEnv(EmeiMujocoEnv):
         rp.action_low, rp.action_high = float(self.action_space.low[0]), float(self.action_space.high[0])
         return rp
 
-    def _ensure_engine(self):
-        if self._family is None:
-            raise NotImplementedError("BaseInvertedDoublePendulumEnv is abstract")
-        if self._engine is None:
-            self._engine = I2PEngine(self, self._params())
-        return self._engine
-
-    # (qpos, qvel) state [B,6], angles unwrapped
-    @property
-    def state(self):
-        return self._engine.state if self._engine is not None else None
-
-    @state.setter
-    def state(self, value):
-        self._ensure_engine().set_state(value)
+    def _new_engine(self):
+        return I2PEngine(self, self._params())
 
     @property
     def current_obs(self):
@@ -99,42 +79,10 @@ class BaseInvertedDoublePendulumEnv(EmeiMujocoEnv):
         s[:, 1:3] = torch.remainder(s[:, 1:3] + math.pi, 2) * math.pi - math.pi
         return s
 
-    def reset(self, *, seed=None, options=None):
-        if self.integrator != "euler":
-            raise NotImplementedError("the analytic inverted double pendulum implements integrator='euler' (mujoco_env.py:94-97)")
-        self._reseed(seed)
-        self._noise_step = 0
-        self.state = self._sample_init_obs(self.num_envs)  # reset_model: mujoco_env.py:130-135 (returns qpos||qvel)
-        self._engine.new_episodes(reseed=True)
-        return self.state.clone(), {}
-
-    def step(self, action):
-        assert self.state is not None, "Call reset before using step method."
-        a = normalise_action(self, action, True)
-        obs, reward, terminal = self._engine.step(a, self.copy_outputs, noise=self._next_obs_noise())
-        return obs, reward, terminal, False, {}
-
-    def get_batch_next_obs(self, obs, pre_obs=None, action=None, state=None, pre_state=None):
-        """core.py:190-193 (requires frozen).  The dynamics need the STATE (qpos||qvel): pass it as ``state=``, or as
-        ``obs`` when the rows are unwrapped states (``current_obs`` is not invertible, :56-60)."""
-        assert self.frozen
-        o, was_np = self._to_device(state if state is not None else obs, self.dtype)
-        saved, self.num_envs = self.num_envs, o.shape[0]
-        try:
-            a = normalise_action(self, action, True)
-        finally:
-            self.num_envs = saved
-        return self._ret(self._ensure_engine().next_obs_stateless(o.contiguous(), a), was_np)
-
-    def freeze(self):
-        self.frozen = True  # mujoco_env.py:114-116
-        if self.state is not None:
-            self.frozen_state = self._engine.snapshot()
-
-    def unfreeze(self):
-        self.frozen = False  # mujoco_env.py:118-120
-        if self.frozen_state is not None:
-            self._engine.restore(self.frozen_state)
+    def _next_obs_rows(self, obs, state):
+        """The dynamics need the STATE (qpos||qvel): ``state=`` when given, else ``obs`` holding unwrapped states
+        (``current_obs`` is not invertible, :56-60)."""
+        return state if state is not None else obs
 
 
 class ReboundInvertedDoublePendulumBalancingEnv(BaseInvertedDoublePendulumEnv):

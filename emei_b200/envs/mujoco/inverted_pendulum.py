@@ -17,8 +17,8 @@ import numpy as np
 import torch
 
 from ... import _lib
-from ...engine import CartPoleEngine, normalise_action
-from .mujoco_env import EmeiMujocoEnv
+from ...engine import CartPoleEngine
+from .mujoco_env import AnalyticPendulumEnv, EmeiMujocoEnv
 
 # capsule volume = pi r^2 L + 4/3 pi r^3 at MuJoCo's default density 1000 kg/m^3
 # (inverted_pendulum.xml:15 cart r=0.1 half-length 0.1; :18 pole r=0.049 length 0.6)
@@ -26,9 +26,8 @@ _MASS_CART = 1000.0 * (math.pi * 0.1**2 * 0.2 + 4.0 / 3.0 * math.pi * 0.1**3)
 _MASS_POLE = 1000.0 * (math.pi * 0.049**2 * 0.6 + 4.0 / 3.0 * math.pi * 0.049**3)
 
 
-class BaseInvertedPendulumEnv(EmeiMujocoEnv):
+class BaseInvertedPendulumEnv(AnalyticPendulumEnv):
     _model = (2, 1, (-3.0, 3.0), [0.0, 0.0])  # nq, nu, ctrlrange (:23), init_qpos
-    _family = None
 
     def __init__(self, freq_rate: int = 1, real_time_scale: float = 0.02, integrator="euler",
                  init_noise_params=5e-3, obs_noise_params=0.0, **kwargs):
@@ -46,7 +45,6 @@ class BaseInvertedPendulumEnv(EmeiMujocoEnv):
         self._transition_graph = np.array(
             [[0, 0, 0, 0], [0, 0, 1, 1], [1, 0, 0, 0], [0, 1, 1, 1], [0, 0, 1, 1]]  # x, theta, v, omega, action
         )  # inverted_pendulum.py:39-41
-        self._engine = None
 
     def _update_model(self):
         pass
@@ -65,34 +63,14 @@ class BaseInvertedPendulumEnv(EmeiMujocoEnv):
     def _rollout_params(self) -> _lib.RolloutParams:
         rp = _lib.RolloutParams()
         rp.init_kind, rp.init_pi_column = 1, -1  # reset_model: init_qpos/qvel + N(0, sigma) (mujoco_env.py:130-140)
-        sp, sv = self._noise_sigmas(self.init_noise_params)
-        mean = np.concatenate([self.init_qpos, self.init_qvel])
-        sigma = np.concatenate([sp, sv])
+        mean, sigma = self._init_tables()
         for j in range(4):
             rp.init_mean[j], rp.init_sigma[j] = float(mean[j]), float(sigma[j])
         rp.action_low, rp.action_high = float(self.action_space.low[0]), float(self.action_space.high[0])
         return rp
 
-    def _scoring_params(self) -> _lib.ScoringParams:
-        p = EmeiMujocoEnv._scoring_params(self)
-        p.x_left, p.x_right = float(self.jnt_range[0][0]), float(self.jnt_range[0][1])
-        return p
-
-    def _ensure_engine(self):
-        if self._family is None:
-            raise NotImplementedError("BaseInvertedPendulumEnv is abstract")
-        if self._engine is None:
-            self._engine = CartPoleEngine(self, self._params(), separate_obs=True)
-        return self._engine
-
-    # (qpos, qvel) state, unwrapped theta
-    @property
-    def state(self):
-        return self._engine.state if self._engine is not None else None
-
-    @state.setter
-    def state(self, value):
-        self._ensure_engine().set_state(value)
+    def _new_engine(self):
+        return CartPoleEngine(self, self._params(), separate_obs=True)
 
     @property
     def current_obs(self):
@@ -100,43 +78,6 @@ class BaseInvertedPendulumEnv(EmeiMujocoEnv):
         s = self.state.clone()
         s[:, 1] = torch.remainder(s[:, 1] + math.pi, 2 * math.pi) - math.pi
         return s
-
-    def reset(self, *, seed=None, options=None):
-        if self.integrator != "euler":
-            raise NotImplementedError("the analytic inverted pendulum implements integrator='euler' (mujoco_env.py:94-97)")
-        self._reseed(seed)
-        self._noise_step = 0
-        self.state = self._sample_init_obs(self.num_envs)  # reset_model: mujoco_env.py:130-135
-        self._engine.new_episodes(reseed=True)
-        return self.state.clone(), {}
-
-    def step(self, action):
-        assert self.state is not None, "Call reset before using step method."
-        a = normalise_action(self, action, True)
-        obs, reward, terminal = self._engine.step(a, self.copy_outputs, noise=self._next_obs_noise())
-        return obs, reward, terminal, False, {}
-
-    def get_batch_next_obs(self, obs, pre_obs=None, action=None, state=None, pre_state=None):
-        assert self.frozen
-        o, was_np = self._to_device(obs, self.dtype)
-        saved, self.num_envs = self.num_envs, o.shape[0]
-        try:
-            a = normalise_action(self, action, True)
-        finally:
-            self.num_envs = saved
-        return self._ret(self._ensure_engine().next_obs_stateless(o, a), was_np)
-
-    def freeze(self):
-        # mujoco_env.py:114-116: snapshot (qpos, qvel)
-        self.frozen = True
-        if self.state is not None:
-            self.frozen_state = self._engine.snapshot()
-
-    def unfreeze(self):
-        # mujoco_env.py:118-120
-        self.frozen = False
-        if self.frozen_state is not None:
-            self._engine.restore(self.frozen_state)
 
 
 class ReboundInvertedPendulumBalancingEnv(BaseInvertedPendulumEnv):

@@ -3,8 +3,8 @@
 In scope (SURVEY.md section 2 row 7): constructor keywords, ``dt``, batched Gaussian initial-state
 sampling (:137-140,197-249), ``transform_state_to_obs`` / ``transform_obs_to_state`` (:142-151),
 freeze semantics (:114-120) and the scoring interface.  Out of scope: ``mujoco.mj_step`` rigid-body
-dynamics (third-party C library, un-vendored) -- ``step`` exists only for the inverted pendulum,
-whose acceleration has a closed form in the reference (classic_control/cartpole.py:48-60).
+dynamics (third-party C library, un-vendored) -- ``step`` exists only for the inverted pendulums
+(``AnalyticPendulumEnv``), whose accelerations have a closed form (classic_control/cartpole.py:48-60).
 
 Reference quirks (SURVEY.md appendix A + DESIGN.md):
   * ``additive_gaussian_noise`` slices ROWS where it means columns (:243-244), so the reference
@@ -26,7 +26,7 @@ import torch
 
 from ... import _lib, spaces
 from ...core import EmeiEnv
-from ...engine import score, score_seq
+from ...engine import normalise_action, score, score_seq
 
 
 class EmeiMujocoEnv(EmeiEnv):
@@ -130,9 +130,7 @@ class EmeiMujocoEnv(EmeiEnv):
         return obs[:, : self.nq], obs[:, self.nq :]
 
     def _sample_init_obs(self, batch_size):
-        sp, sv = self._noise_sigmas(self.init_noise_params)
-        mean = np.concatenate([self.init_qpos, self.init_qvel])
-        sigma = np.concatenate([sp, sv])
+        mean, sigma = self._init_tables()
         d = mean.shape[0]
         out = torch.empty((batch_size, d), dtype=self.dtype, device=self.device)
         Arr = ctypes.c_double * d
@@ -203,3 +201,65 @@ class EmeiMujocoEnv(EmeiEnv):
 
     def unfreeze(self):
         self.frozen = False
+
+
+class AnalyticPendulumEnv(EmeiMujocoEnv):
+    """The inverted pendulums, whose accelerations have a closed form: ``reset`` / ``step`` / ``get_batch_next_obs`` /
+    ``freeze`` run on the device through the engine that the subclass's ``_new_engine`` builds (forward Euler,
+    mujoco_env.py:91-97).  State = qpos || qvel, angles unwrapped."""
+
+    def _ensure_engine(self):
+        if self._family is None:
+            raise NotImplementedError(f"{type(self).__name__} is abstract")
+        if self._engine is None:
+            self._engine = self._new_engine()
+        return self._engine
+
+    def _scoring_params(self) -> _lib.ScoringParams:
+        p = EmeiMujocoEnv._scoring_params(self)
+        p.x_left, p.x_right = float(self.jnt_range[0][0]), float(self.jnt_range[0][1])
+        return p
+
+    @property
+    def state(self):
+        return self._engine.state if self._engine is not None else None
+
+    @state.setter
+    def state(self, value):
+        self._ensure_engine().set_state(value)
+
+    def reset(self, *, seed=None, options=None):
+        if self.integrator != "euler":
+            raise NotImplementedError(f"{type(self).__name__}: the analytic dynamics implement integrator='euler' (mujoco_env.py:94-97)")
+        self._reseed(seed)
+        self._noise_step = 0
+        self.state = self._sample_init_obs(self.num_envs)  # reset_model: mujoco_env.py:130-135 (returns qpos||qvel)
+        self._engine.new_episodes(reseed=True)
+        return self.state.clone(), {}
+
+    def step(self, action):
+        assert self.state is not None, "Call reset before using step method."
+        a = normalise_action(self, action, True, self.num_envs)
+        obs, reward, terminal = self._engine.step(a, self.copy_outputs, noise=self._next_obs_noise())
+        return obs, reward, terminal, False, {}
+
+    def _next_obs_rows(self, obs, state):
+        """The rows get_batch_next_obs steps: ``obs`` (``state=`` is not read)."""
+        return obs
+
+    def get_batch_next_obs(self, obs, pre_obs=None, action=None, state=None, pre_state=None):
+        """core.py:190-193: requires a frozen env; one dynamics step from the given rows, the env does not move."""
+        assert self.frozen
+        o, was_np = self._to_device(self._next_obs_rows(obs, state), self.dtype)
+        a = normalise_action(self, action, True, o.shape[0])
+        return self._ret(self._ensure_engine().next_obs_stateless(o, a), was_np)
+
+    def freeze(self):
+        self.frozen = True  # mujoco_env.py:114-116: snapshot (qpos, qvel)
+        if self.state is not None:
+            self.frozen_state = self._engine.snapshot()
+
+    def unfreeze(self):
+        self.frozen = False  # mujoco_env.py:118-120
+        if self.frozen_state is not None:
+            self._engine.restore(self.frozen_state)

@@ -212,6 +212,8 @@ def test_abstract_methods_raise():
         env.get_batch_next_obs(None)  # not frozen
     with pytest.raises(NotImplementedError):
         BaseCartPoleEnv().reset()
+    with pytest.raises(NotImplementedError):
+        E.make("HopperRunning-v0").rollout(3)  # scoring-only env: no fused rollout kernel
 
 
 def test_registry_ids_and_spaces():

@@ -1332,6 +1332,9 @@ def test_i2p_reset_freeze_next_obs_and_graph():
     snap = env.state.clone()
     nxt = env.get_batch_next_obs(env.state, action=a)  # stateless: the env does not move
     assert torch.equal(env.state, snap)
+    # state= takes precedence over obs, any batch size: rows 100..611 step exactly as in the full batch
+    part = env.get_batch_next_obs(env.current_obs[:7], action=a[100:612], state=snap[100:612])
+    assert torch.equal(part, nxt[100:612]) and env.num_envs == 2048
     o1, _, _, _, _ = env.step(a)
     assert torch.equal(o1, nxt)
     env.step(a)

@@ -281,6 +281,7 @@ def test_cartpole_ip_f32_step_matrix(kind, fr):
     env.freeze()
     nxt = env.get_batch_next_obs(torch.from_numpy(st).cuda(), action=action_tensor(act, action_kinds(kind)[0], 0))
     assert np.array_equal(bits(nxt.cpu().numpy()), bits(first[1]))
+    assert env.num_envs == 4
 
 
 def ring_slots(action_bytes):
