@@ -1,0 +1,86 @@
+"""Gradients of the analytic dynamics: ``torch.autograd`` through the step kernels.
+
+The cart-pole family, the analytic inverted pendulum and the analytic inverted double pendulum have closed-form dynamics
+(freq_rate forward-Euler sub-steps), so their step is differentiable almost everywhere.  Two entry points serve them:
+
+* ``transition(env, state, action)`` -> ``(next_state, obs, reward [B,1], done bool [B,1])``: the step kernel run
+  statelessly on caller rows (outputs bit-equal to ``get_batch_next_obs`` / ``step`` from the same rows), recorded in the
+  autograd graph when ``state`` or ``action`` requires grad; its backward is the vector-Jacobian-product kernel
+  (``emei_*_step_vjp_*``), which never materialises the Jacobian.  Chaining it T times is backpropagation through time.
+* ``jacobian(env, state, action)`` -> ``(jac [B,D,D+1], reward_grad [B,D+1])``: the per-sample Jacobian
+  ``d(next_state, reward) / d(state, action)`` (``emei_*_step_jacobian_*``); the last column is the action's.
+
+Semantics (include/emei_b200.h, DESIGN.md "Derivatives"): no state noise; the action gradient passes the control clamp
+where ``ctrl_low <= ctrl <= ctrl_high`` and is 0 for discrete actions; the I2P observation's angles have slope pi (the
+``current_obs`` precedence quirk).  The float64 cart-pole gradient is that of the float64 Euler step (the forward keeps
+the reference's float32-rounded increments).  A continuous action is cast to the env dtype inside the graph, so its
+gradient comes back in the caller's dtype and shape (``[B]`` or ``[B,1]``).
+"""
+import torch
+from torch.autograd.function import once_differentiable
+
+from .engine import normalise_action
+
+
+def _rows(t: torch.Tensor) -> torch.Tensor:
+    """contiguous rows at a 16-byte aligned address (the kernels' row loads)"""
+    t = t.contiguous()
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
+def _inputs(env, state, action):
+    """-> (engine, state rows [B, D] in the env dtype, action [B] in its kernel encoding, came_from_numpy).  Every
+    conversion is an autograd-tracked op, so gradients flow back to the caller's tensors."""
+    eng = env._ensure_engine()
+    s, was_np = env._to_device(state, env.dtype)
+    if s.dim() != 2 or s.shape[1] != eng.obs_dim:
+        raise ValueError(f"state must be [B, {eng.obs_dim}], got {tuple(s.shape)}")
+    continuous = len(env.action_space.shape) > 0
+    a = normalise_action(env, action, continuous, s.shape[0])
+    if continuous:
+        a = a.to(env.dtype)
+    return eng, s, a, was_np
+
+
+class StepTransition(torch.autograd.Function):
+    """forward: ``RowStateEngine.transition_stateless``; backward: ``RowStateEngine.vjp``."""
+
+    @staticmethod
+    def forward(ctx, state, action, engine):
+        rows, act = _rows(state.detach()), action.detach().contiguous()
+        s_out, obs, reward, done = engine.transition_stateless(rows, act)
+        if obs is s_out:  # cart-pole: the observation is the next state; two outputs need two tensors
+            obs = s_out.clone()
+        ctx.engine = engine
+        ctx.save_for_backward(rows, act)
+        ctx.mark_non_differentiable(done)
+        ctx.set_materialize_grads(False)
+        return s_out, obs, reward, done
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_state, g_obs, g_reward, g_done):
+        rows, act = ctx.saved_tensors
+        want_state, want_action = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        if g_state is None and g_obs is None and g_reward is None:
+            return None, None, None
+        g_state = _rows(g_state) if g_state is not None else None
+        g_obs = _rows(g_obs) if g_obs is not None else None
+        g_reward = g_reward.reshape(-1).contiguous() if g_reward is not None else None
+        g_in, g_act = ctx.engine.vjp(rows, act, g_state, g_obs, g_reward, want_action)
+        return (g_in if want_state else None), g_act, None
+
+
+def transition(env, state, action):
+    """``env.get_batch_transition``: see the module docstring."""
+    eng, s, a, was_np = _inputs(env, state, action)
+    out = StepTransition.apply(s, a, eng)
+    return tuple(env._ret(t, was_np) for t in out) if was_np else out
+
+
+def jacobian(env, state, action):
+    """``env.get_batch_jacobian``: see the module docstring."""
+    eng, s, a, was_np = _inputs(env, state, action)
+    with torch.no_grad():
+        jac, reward_grad = eng.jacobian(_rows(s.detach()), a.detach().contiguous())
+    return env._ret(jac, was_np), env._ret(reward_grad, was_np)

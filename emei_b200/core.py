@@ -213,6 +213,17 @@ class EmeiEnv(Freezable):
         assert self.frozen
         raise NotImplementedError
 
+    # ------------------------------------------------------------------ derivatives (autodiff.py)
+    _no_derivatives = "it has no differentiable dynamics kernel"  # why get_batch_transition / get_batch_jacobian raise
+
+    def get_batch_transition(self, state, action):
+        """Differentiable stateless step ``(next_state, obs, reward [B,1], done bool [B,1])``: the analytic families only."""
+        raise NotImplementedError(f"{type(self).__name__}: no gradients, {self._no_derivatives}")
+
+    def get_batch_jacobian(self, state, action):
+        """``(jac [B,D,D+1], reward_grad [B,D+1])`` of the step: the analytic families only."""
+        raise NotImplementedError(f"{type(self).__name__}: no Jacobian, {self._no_derivatives}")
+
     # ------------------------------------------------------------------ fused rollouts
     def rollout(self, horizon: int, actions=None, record: bool = False, auto_reset: bool = True, max_episode_steps=None):
         """``horizon`` steps of every env in ONE kernel launch: the batched counterpart of the reference's

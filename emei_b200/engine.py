@@ -177,6 +177,7 @@ class RowStateEngine(Engine):
         self.obs_dim = width
         self.separate_obs = separate_obs
         self._step_entry, self._noisy_entry = step_entry, noisy_entry
+        self._jacobian_entry, self._vjp_entry = step_entry + "_jacobian", step_entry + "_vjp"
         self._bufs = self._obs = self._out = None
         self._cur = 0
         self.has_state = False
@@ -252,9 +253,10 @@ class RowStateEngine(Engine):
     def flip(self):
         self._cur = 1 - self._cur
 
-    def next_obs_stateless(self, rows: torch.Tensor, action: torch.Tensor):
-        """get_batch_next_obs: one dynamics step from caller-supplied state rows (any batch size); the engine's own
-        state is untouched."""
+    def transition_stateless(self, rows: torch.Tensor, action: torch.Tensor):
+        """One step of the step kernel from caller-supplied state rows [b, width] (any batch size, no state noise, no
+        statistics); the engine's own state is untouched.  -> (state_out, obs, reward [b,1], done bool [b,1]); obs is
+        state_out itself when the family has no separate observation."""
         env = self.env
         b = rows.shape[0]
         out = torch.empty_like(rows)
@@ -262,7 +264,36 @@ class RowStateEngine(Engine):
         reward = torch.empty((b, 1), dtype=env.dtype, device=env.device)
         done = torch.empty((b, 1), dtype=torch.uint8, device=env.device)
         self._launch(0, b, rows, out, obs, action, reward, done, None, None)
-        return obs if obs is not None else out
+        return out, (obs if obs is not None else out), reward, done.view(torch.bool)
+
+    def next_obs_stateless(self, rows: torch.Tensor, action: torch.Tensor):
+        """get_batch_next_obs: the observation of ``transition_stateless``."""
+        return self.transition_stateless(rows, action)[1]
+
+    def jacobian(self, rows: torch.Tensor, action: torch.Tensor):
+        """d(state_out, reward) / d(state_in, action) of ``transition_stateless`` (emei_*_step_jacobian_*):
+        -> (jac [b, width, width + 1], reward_grad [b, width + 1]); the last column is the action's."""
+        env = self.env
+        b, d = rows.shape[0], self.obs_dim
+        jac = torch.empty((b, d, d + 1), dtype=env.dtype, device=env.device)
+        reward_grad = torch.empty((b, d + 1), dtype=env.dtype, device=env.device)
+        self.params.action_kind = _ACTION_KIND[action.dtype]
+        env._call(self._jacobian_entry, rows.data_ptr(), action.data_ptr(), jac.data_ptr(), reward_grad.data_ptr(), b,
+                  ctypes.byref(self.params), env._stream())
+        return jac, reward_grad
+
+    def vjp(self, rows: torch.Tensor, action: torch.Tensor, g_state_out, g_obs, g_reward, want_action: bool):
+        """Backward of ``transition_stateless`` (emei_*_step_vjp_*): the cotangents ``g_state_out`` / ``g_obs`` [b, width]
+        and ``g_reward`` [b] are contiguous tensors or None (zero).  -> (g_state_in [b, width], g_action [b] or None)."""
+        env = self.env
+        b = rows.shape[0]
+        g_in = torch.empty_like(rows)
+        g_act = torch.empty((b,), dtype=env.dtype, device=env.device) if want_action else None
+        self.params.action_kind = _ACTION_KIND[action.dtype]
+        ptr = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
+        env._call(self._vjp_entry, rows.data_ptr(), action.data_ptr(), ptr(g_state_out), ptr(g_obs), ptr(g_reward), g_in.data_ptr(),
+                  ptr(g_act), b, ctypes.byref(self.params), env._stream())
+        return g_in, g_act
 
 
 class CartPoleEngine(RowStateEngine):

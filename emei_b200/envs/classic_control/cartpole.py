@@ -16,7 +16,7 @@ import math
 import numpy as np
 import torch
 
-from ... import _lib, spaces
+from ... import _lib, autodiff, spaces
 from ...engine import CartPoleEngine, normalise_action, score
 from .base_control import BaseControlEnv
 
@@ -102,6 +102,19 @@ class BaseCartPoleEnv(BaseControlEnv):
         o, was_np = self._to_device(obs, self.dtype)
         a = normalise_action(self, action, self._continuous, o.shape[0])
         return self._ret(eng.next_obs_stateless(o, a), was_np)
+
+    def get_batch_transition(self, state, action):
+        """One differentiable step from caller rows ``state`` [B,4] (any B; no freeze needed, the env's state, stats and
+        buffers are untouched) -> ``(next_state, obs, reward [B,1], done bool [B,1])``, bit-equal to
+        ``get_batch_next_obs`` / ``step``.  Records the autograd graph when ``state`` or a continuous ``action`` requires
+        grad (backward: emei_cartpole_step_vjp_*).  float64: the gradient is that of the float64 Euler step; the forward
+        keeps the reference's float32-rounded increments (DESIGN.md "Derivatives")."""
+        return autodiff.transition(self, state, action)
+
+    def get_batch_jacobian(self, state, action):
+        """``(jac [B,4,5], reward_grad [B,5])`` = d(next_state, reward) / d(state, action) of the same step; the action
+        column is 0 for discrete actions."""
+        return autodiff.jacobian(self, state, action)
 
 
 class CartPoleBalancingEnv(BaseCartPoleEnv):

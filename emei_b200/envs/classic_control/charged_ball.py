@@ -15,6 +15,8 @@ import numpy as np
 
 
 class BaseChargedBallEnv(BaseControlEnv):
+    _no_derivatives = "the ball's landing / take-off events (charged_ball.py:62-82) make its step discontinuous"
+
     def __init__(self, freq_rate=1, time_step=0.02, **kwargs):
         BaseControlEnv.__init__(self, freq_rate=freq_rate, **kwargs)
         # the reference intends env_params = (freq_rate, time_step): charged_ball.py:11-12

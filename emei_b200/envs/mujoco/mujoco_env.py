@@ -24,7 +24,7 @@ from typing import Dict, Optional, Tuple, Union
 import numpy as np
 import torch
 
-from ... import _lib, spaces
+from ... import _lib, autodiff, spaces
 from ...core import EmeiEnv
 from ...engine import normalise_action, score, score_seq
 
@@ -35,6 +35,7 @@ class EmeiMujocoEnv(EmeiEnv):
     # subclasses set: (nq, nu, ctrlrange, init_qpos)
     _model = None
     _family = None
+    _no_derivatives = "its dynamics are MuJoCo's mj_step, which is outside the emei_b200 hot path"
 
     def __init__(
         self,
@@ -242,6 +243,18 @@ class AnalyticPendulumEnv(EmeiMujocoEnv):
         a = normalise_action(self, action, True, self.num_envs)
         obs, reward, terminal = self._engine.step(a, self.copy_outputs, noise=self._next_obs_noise())
         return obs, reward, terminal, False, {}
+
+    def get_batch_transition(self, state, action):
+        """One differentiable step from caller rows ``state`` = qpos || qvel, angles unwrapped (as ``state=`` of
+        ``get_batch_next_obs``; any B, no freeze needed, the env's state, stats and buffers are untouched) ->
+        ``(next_state, obs, reward [B,1], done bool [B,1])``, bit-equal to ``get_batch_next_obs`` / ``step``.  Records the
+        autograd graph when ``state`` or ``action`` requires grad (backward: emei_cartpole_step_vjp_* / emei_i2p_step_vjp_*);
+        the action gradient passes the control clamp on [ctrl_low, ctrl_high] only."""
+        return autodiff.transition(self, state, action)
+
+    def get_batch_jacobian(self, state, action):
+        """``(jac [B,D,D+1], reward_grad [B,D+1])`` = d(next_state, reward) / d(state, action) of the same step."""
+        return autodiff.jacobian(self, state, action)
 
     def _next_obs_rows(self, obs, state):
         """The rows get_batch_next_obs steps: ``obs`` (``state=`` is not read)."""

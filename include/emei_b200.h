@@ -168,6 +168,50 @@ int emei_i2p_step_f32(const float* state_in, float* state_out, float* obs_out, c
 int emei_i2p_step_f64(const double* state_in, double* state_out, double* obs_out, const void* action, double* reward,
                       uint8_t* done, double* stats, int64_t n, const emei_i2p_params* p, emei_stream_t stream);
 
+/* ---- derivatives of the analytic steps (Jacobians and vector-Jacobian products) --------------------
+ * What is differentiated: the real-valued model emei_cartpole_step_* / emei_i2p_step_* evaluate -- freq_rate forward-Euler
+ * sub-steps of the analytic acceleration, then the observation, then the variant's reward -- without state noise (the
+ * stateless transition of get_batch_next_obs).
+ *   _f64: plain float64 arithmetic.  The cart-pole family's forward step rounds each Euler increment through float32 (the
+ *         reference's mixed rule); the derivative is that of y + h f(y) in float64, which matches a complex-step derivative
+ *         to ~1e-12.  The forward step is unchanged.
+ *   _f32: float32 through the generic device arithmetic: gradients are a tolerance product, not a bit product.
+ * Action column: cart-pole continuous kinds d/da of force = force_mag * a; IP / I2P force = gear * clamp(ctrl), whose
+ * gradient passes where ctrl_low <= ctrl <= ctrl_high (inclusive, as torch.clamp) and is 0 outside; discrete kinds: 0.
+ * Observation: the IP angle wrap (th + pi) mod 2pi - pi has slope 1; the I2P current_obs quirk ((th + pi) mod 2) * pi - pi
+ * has slope pi on both angles (inverted_double_pendulum.py:56-60, replicated by the forward), and the reward computed on that
+ * observation inherits the factor.  `done` is not differentiable.  Non-finite inputs give non-finite gradients.
+ * Validation as the step entry points (codes, row alignment); variants outside the family: EMEI_ERR_BAD_VARIANT. */
+/* d(state_out, reward) / d(state_in, action) of emei_cartpole_step_* (cart-pole and EMEI_IP_* variants):
+ *   jac [n,4,5]: jac[i][r][c] = d state_out[i][r] / d state_in[i][c] (c < 4); c = 4: d state_out[i][r] / d action[i]
+ *   reward_grad [n,5] nullable: the same row for reward[i] */
+int emei_cartpole_step_jacobian_f32(const float* state_in, const void* action, float* jac, float* reward_grad, int64_t n,
+                                    const emei_cartpole_params* p, emei_stream_t stream);
+int emei_cartpole_step_jacobian_f64(const double* state_in, const void* action, double* jac, double* reward_grad, int64_t n,
+                                    const emei_cartpole_params* p, emei_stream_t stream);
+/* vector-Jacobian product (autograd's backward) of the same step:
+ *   g_state_in[i] = g_state_out[i] . d state_out / d state_in + g_obs[i] . d obs_out / d state_in + g_reward[i] d reward / d state_in
+ *   g_state_out [n,4], g_obs [n,4], g_reward [n]: each nullable (= zero); g_state_in [n,4] written;
+ *   g_action [n] written, nullable; must be NULL for discrete action kinds (else EMEI_ERR_BAD_ACTION_KIND).
+ * The Jacobian is contracted in registers and never stored. */
+int emei_cartpole_step_vjp_f32(const float* state_in, const void* action, const float* g_state_out, const float* g_obs,
+                               const float* g_reward, float* g_state_in, float* g_action, int64_t n, const emei_cartpole_params* p,
+                               emei_stream_t stream);
+int emei_cartpole_step_vjp_f64(const double* state_in, const void* action, const double* g_state_out, const double* g_obs,
+                               const double* g_reward, double* g_state_in, double* g_action, int64_t n, const emei_cartpole_params* p,
+                               emei_stream_t stream);
+/* the same pair for emei_i2p_step_*: rows of 6, jac [n,6,7], reward_grad [n,7], g_state_out / g_obs / g_state_in [n,6] */
+int emei_i2p_step_jacobian_f32(const float* state_in, const void* action, float* jac, float* reward_grad, int64_t n,
+                               const emei_i2p_params* p, emei_stream_t stream);
+int emei_i2p_step_jacobian_f64(const double* state_in, const void* action, double* jac, double* reward_grad, int64_t n,
+                               const emei_i2p_params* p, emei_stream_t stream);
+int emei_i2p_step_vjp_f32(const float* state_in, const void* action, const float* g_state_out, const float* g_obs,
+                          const float* g_reward, float* g_state_in, float* g_action, int64_t n, const emei_i2p_params* p,
+                          emei_stream_t stream);
+int emei_i2p_step_vjp_f64(const double* state_in, const void* action, const double* g_state_out, const double* g_obs,
+                          const double* g_reward, double* g_state_in, double* g_action, int64_t n, const emei_i2p_params* p,
+                          emei_stream_t stream);
+
 /* ---- per-sub-step Gaussian state noise ("obs_noise_params", SURVEY 8f rank 4) -------------------
  * Replaces mujoco_env.py:98-104: after EVERY sub-step the reference overwrites the simulator state with
  * additive_gaussian_noise(qpos, qvel, obs_noise_params) (mujoco_env.py:197-249: one N(0, sigma_pos) /
