@@ -125,17 +125,15 @@ __device__ __forceinline__ float action_to_f_mt(float a, const CartPoleF32Consts
 }
 
 // reward, not-done flag and observation of one env after its step (cartpole.py:124-129,145-151;
-// inverted_pendulum.py:45-49,73-79,103-111,139-146,174-183).  have_cos: cos_in = cos of the reward angle from
-// the integrator (cart-pole: theta; IP: the IP's own theta, i.e. the integrator's value with the flip undone);
-// otherwise (the env was redone with the libm path) it is computed here.
+// inverted_pendulum.py:45-49,73-79,103-111,139-146,174-183).  cy = cos of the reward angle from the integrator
+// (cart-pole: theta; IP: the IP's own theta, i.e. the integrator's value with the flip undone).
 template <bool IP>
-__device__ __forceinline__ void cartpole_outcome(const float4& y, bool have_cos, float cos_in, const CartPoleF32Consts& k,
-                                                 float& rew, bool& notdone, float4& obs) {
+__device__ __forceinline__ void cartpole_outcome(const float4& y, float cy, const CartPoleF32Consts& k, float& rew, bool& notdone,
+                                                 float4& obs) {
   obs = y;
   if constexpr (!IP) {
     if (k.variant == EMEI_CARTPOLE_SWINGUP) {
-      const float cth = have_cos ? cos_in : cosf(y.z);
-      rew = fmaf(cth, 0.5f, 0.5f);     // cartpole.py:149-151
+      rew = fmaf(cy, 0.5f, 0.5f);      // cartpole.py:149-151
       notdone = fabsf(y.x) < k.x_thr;  // cartpole.py:145-147
     } else {
       rew = 1.0f;                                                     // cartpole.py:128-129
@@ -145,7 +143,6 @@ __device__ __forceinline__ void cartpole_outcome(const float4& y, bool have_cos,
     const float th_obs = wrap_pi_f32(y.y);  // observation: theta wrapped to [-pi, pi) (inverted_pendulum.py:45-49)
     obs.y = th_obs;
     const bool finite = isfinite(y.x) && isfinite(th_obs) && isfinite(y.z) && isfinite(y.w);
-    const float cy = have_cos ? cos_in : f32::cos_core(th_obs);  // |th_obs| <= pi (NaN stays NaN)
     const bool in_rail = (k.x_left < y.x) && (y.x < k.x_right);
     switch (k.variant) {
       case EMEI_IP_REBOUND_BALANCING:  // inverted_pendulum.py:73-79
@@ -178,7 +175,7 @@ __device__ __forceinline__ void cartpole_step_one(float4& y, float f_mt, uint32_
   if (!ok) {
     y = integrate_libm<IP, FR>(y0, f_mt, flip, k.k, k.freq_rate, &c);
   }
-  cartpole_outcome<IP>(y, true, IP ? f32::u2f(f32::f2u(c) ^ flip) : c, k, rew, notdone, obs);
+  cartpole_outcome<IP>(y, IP ? f32::u2f(f32::f2u(c) ^ flip) : c, k, rew, notdone, obs);
 }
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }

@@ -15,18 +15,16 @@
 //
 // Chunk c = envs [512 c, 512 c + 512): thread t of a group owns envs 512 c + t and 512 c + 256 + t.
 #pragma once
-#include <cstdlib>
 #include <type_traits>
 #include "cartpole_f32.cuh"
 
 namespace emei {
 
-constexpr int kTmaGroups = 4;                                 // consumer groups per CTA of the shipped shape (template GROUPS)
-constexpr int kTmaThreads = kTmaGroups * kBlock;              // 1024 threads: 8 warps per scheduler at <= 64 registers; thread 0 doubles as the TMA producer
+constexpr int kTmaGroups = 4;                                 // consumer groups of kBlock threads per CTA
+constexpr int kTmaThreads = kTmaGroups * kBlock;              // 1024 threads: 8 warps per scheduler at <= 64 registers
 constexpr uint32_t kChunk = 2 * kBlock;                       // envs per chunk
 constexpr int kTmaSmemBudget = 208 * 1024;                    // ring bytes (of 227 KB per SM)
 constexpr int kTmaMaxSlots = 32;
-constexpr uint32_t kChunkOutBytes = kChunk * 5;               // BULK: staged reward (4 B) + done (1 B) of a chunk
 // The first ring-full (up to 16 chunks x 2 bulk copies, ~1 000 instructions of one thread) is requested by the first
 // thread of the LAST consumer group: with 13.8 chunks per SM the groups own 4, 4, 3, 3 (or 4, 3, 3, 3) chunks, so the
 // last group's warps have a chunk's worth of slack while group 0's are on the critical path of the CTA.
@@ -92,75 +90,30 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 }
 // 1-D bulk copy global -> shared (TMA engine); completes `bytes` on the mbarrier.  16-byte aligned, size % 16 == 0.
 __device__ __forceinline__ void tma_load_1d(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar) {
-#ifdef EMEI_TMA_STREAM_HINTS  // development A/B (tools/kbench): L2 evict-first policy on the streamed inputs
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(smem_u32(smem_dst)),
-               "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)), "l"(pol)
-               : "memory");
-#else
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(smem_dst)),
                "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar))
                : "memory");
-#endif
 }
 
-// 1-D bulk copy shared -> global (TMA engine), bulk-group completion.  16-byte aligned, size % 16 == 0.
-__device__ __forceinline__ void tma_store_1d(void* gmem_dst, uint32_t smem_src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gmem_dst), "r"(smem_src), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void tma_store_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void sts128(uint32_t addr, const float4& v) {
-  asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-}
-__device__ __forceinline__ void sts32(uint32_t addr, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory"); }
-__device__ __forceinline__ void sts8(uint32_t addr, uint32_t v) { asm volatile("st.shared.u8 [%0], %1;" ::"r"(addr), "r"(v) : "memory"); }
-
-#ifdef EMEI_TMA_TRACE
-// development only (tools/kbench -DEMEI_TMA_TRACE): per (CTA, group) timestamps of the chunk pipeline
-__device__ unsigned long long* g_tma_trace = nullptr;  // [gridDim.x][GROUPS][64]
-__device__ __forceinline__ unsigned long long tma_now() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-#define EMEI_TRACE(slot_idx)                                                                                     \
-  if (g_tma_trace != nullptr && t == 0 && (slot_idx) < 64)                                                       \
-  g_tma_trace[(static_cast<size_t>(blockIdx.x) * GROUPS + g) * 64 + (slot_idx)] = tma_now()
-#else
-#define EMEI_TRACE(slot_idx)
-#endif
-
-// GROUPS consumer groups of 256 threads per CTA (4: one CTA fills an SM; 2: half an SM, so that the CTA of the NEXT
-// step kernel -- launched early by programmatic dependent launch -- can already be resident, initialised and
-// parked in griddepcontrol.wait while this one computes).  BULK: a warp stages its 64 envs' outputs in shared memory
-// (next state in place over the staged input rows, reward and done in a per-slot output area) and its lane 0 writes
-// them with three bulk copies shared -> global; only for launches that never recycle a slot (the host decides).
+// kTmaGroups consumer groups of kBlock threads per CTA, one CTA per SM.
 // Chunk c = envs [512 c, 512 c + 512); warp w of a group owns the 64 contiguous envs 512 c + 64 w ..: lane l takes
 // 64 w + l and 64 w + 32 + l.
-template <bool IP, int AK, int FR, bool HAS_OBS, int GROUPS = kTmaGroups, bool BULK = false, int GSZ = kBlock>
-__global__ void __launch_bounds__(GROUPS * GSZ, 1024 / (GROUPS * GSZ))
+template <bool IP, int AK, int FR, bool HAS_OBS>
+__global__ void __launch_bounds__(kTmaThreads, 1)
     cartpole_step_f32_tma_kernel(const float4* state_in, float4* state_out, float4* obs_out,
                                  const void* __restrict__ action, float* __restrict__ reward, uint8_t* __restrict__ done,
                                  double* stats, uint32_t n, int n_slots, int flags, const CartPoleF32Consts k) {
-  // GSZ threads per consumer group, 2 * GSZ envs per chunk (the names below shadow the namespace-level defaults)
-  constexpr int kBlock = GSZ;
-  constexpr uint32_t kChunk = 2 * GSZ;
-  [[maybe_unused]] constexpr uint32_t kChunkOutBytes = kChunk * 5;
   // flags: bit 0 = the action array is 16-byte aligned (staged by TMA); bit 1 = prefetch the first ring-full into L2 before
-  // griddepcontrol.wait; bits 8.. = the consumer group whose first thread requests the first ring-full (kTmaProducerGroup)
+  // griddepcontrol.wait; bits 16.. = how many chunks of it to prefetch (0: all)
   const int action_via_tma = flags & 1;
-  const uint32_t producer_tid = static_cast<uint32_t>((flags >> 8) & 0xff) * kBlock;
+  constexpr uint32_t producer_tid = kTmaProducerGroup * kBlock;
   using f32::f2;
   using ActT = typename ActionStorage<AK>::type;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   // layout: [n_slots] state chunks (8 KB each) | [n_slots] action chunks | full[n_slots] | empty[n_slots] | reduction scratch
   float4* s_state = reinterpret_cast<float4*>(smem_raw);
   ActT* s_act = reinterpret_cast<ActT*>(smem_raw + static_cast<size_t>(n_slots) * kChunk * sizeof(float4));
-  unsigned char* s_out = reinterpret_cast<unsigned char*>(s_act) + static_cast<size_t>(n_slots) * kChunk * sizeof(ActT);  // BULK: [n_slots] x (512 rewards | 512 done bytes)
-  uint64_t* full = reinterpret_cast<uint64_t*>(s_out + (BULK ? static_cast<size_t>(n_slots) * kChunkOutBytes : 0));
+  uint64_t* full = reinterpret_cast<uint64_t*>(reinterpret_cast<unsigned char*>(s_act) + static_cast<size_t>(n_slots) * kChunk * sizeof(ActT));
   uint64_t* empty = full + n_slots;
   const uint32_t tid = threadIdx.x;
   const uint32_t n_chunks = (n + kChunk - 1) / kChunk;
@@ -182,9 +135,9 @@ __global__ void __launch_bounds__(GROUPS * GSZ, 1024 / (GROUPS * GSZ))
   // lines (the same batch stepped again) they are in L2 already and the prefetch is a hit; if they are cold (another batch,
   // a state set from the host) the DRAM reads start while the previous grid's stragglers drain -- the 1-2 us between
   // griddepcontrol.wait and the first chunk's landing (profiles/r02_c2_chunk_pipeline_trace.txt) shrink to an L2 hit.
-  if ((flags & 2) && tid == kBlock * (GROUPS > 1 ? 1 : 0)) {  // a thread that neither initialises barriers nor issues the loads
+  if ((flags & 2) && tid == kBlock) {  // a thread that neither initialises barriers nor issues the loads
     uint32_t first = my_chunks < static_cast<uint32_t>(n_slots) ? my_chunks : static_cast<uint32_t>(n_slots);
-    const uint32_t depth = static_cast<uint32_t>((flags >> 16) & 0xff);  // development knob: 0 = the whole first ring-full
+    const uint32_t depth = static_cast<uint32_t>((flags >> 16) & 0xff);
     if (depth != 0 && depth < first) first = depth;
     for (uint32_t j = 0; j < first; ++j) {
       const uint32_t base = (blockIdx.x + j * gridDim.x) * kChunk;
@@ -202,7 +155,7 @@ __global__ void __launch_bounds__(GROUPS * GSZ, 1024 / (GROUPS * GSZ))
   {
     // ------------------------------------------------------------------ four independent pipelines
     // Group g (256 threads) owns the CTA's local chunks g, g+4, ... and a private ring of n_slots / 4 slots.
-    // Thread 0 requests the first ring-full of every group at t = 0; after that (batches whose share of an SM
+    // The first thread of group kTmaProducerGroup requests the first ring-full of every group at t = 0; after that (batches whose share of an SM
     // exceeds the ring) thread 0 OF EACH GROUP refills, at the top of iteration m, the slot the group
     // read in iteration m - 1 -- by then all 8 warps of the group have long finished reading it, so the wait on
     // the empty barrier never blocks, and the request runs n_slots / 4 - 1 iterations ahead of its use.
@@ -212,21 +165,13 @@ __global__ void __launch_bounds__(GROUPS * GSZ, 1024 / (GROUPS * GSZ))
     // env index and the slot / phase pair.  The body is compiled twice: FULL (every chunk but possibly the last
     // of the batch: no per-lane predicates) and the ragged tail.
     const uint32_t g = tid / kBlock, t = tid % kBlock;
-    EMEI_TRACE(0);  // after griddepcontrol.wait
-#ifdef EMEI_TMA_TRACE
-    if (g_tma_trace != nullptr && t == 0) {
-      unsigned smid;
-      asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-      g_tma_trace[(static_cast<size_t>(blockIdx.x) * GROUPS + g) * 64 + 63] = smid;
-    }
-#endif
     const uint32_t flip = ip_flip(IP, k.variant);
-    const uint32_t spg = static_cast<uint32_t>(n_slots) / GROUPS;                  // slots per group (n_slots % GROUPS == 0)
-    const uint32_t my_g = my_chunks > g ? (my_chunks - g + GROUPS - 1) / GROUPS : 0;  // this group's chunks
+    const uint32_t spg = static_cast<uint32_t>(n_slots) / kTmaGroups;                      // slots per group (n_slots % kTmaGroups == 0)
+    const uint32_t my_g = my_chunks > g ? (my_chunks - g + kTmaGroups - 1) / kTmaGroups : 0;  // this group's chunks
     const bool recycling = my_g > spg;  // group-uniform: the ring is reused
     const uint32_t slot0 = g * spg;
     auto issue = [&](uint32_t gg, uint32_t m, uint32_t sl) {  // chunk m of group gg into slot sl
-      const uint32_t c = blockIdx.x + (gg + m * GROUPS) * gridDim.x;
+      const uint32_t c = blockIdx.x + (gg + m * kTmaGroups) * gridDim.x;
       const uint32_t base = c * kChunk;
       const uint32_t cnt = n - base < kChunk ? n - base : kChunk;
       const bool act_tma = action_via_tma && cnt == kChunk;  // partial tail: consumers read their actions directly
@@ -241,19 +186,17 @@ __global__ void __launch_bounds__(GROUPS * GSZ, 1024 / (GROUPS * GSZ))
     // complete late (10.8 us per step at 2^20 envs instead of 9.7); issued in order, chunk 0 lands first.
     if (tid == producer_tid) {
       const uint32_t first = my_chunks < static_cast<uint32_t>(n_slots) ? my_chunks : static_cast<uint32_t>(n_slots);
-      for (uint32_t j = 0; j < first; ++j) issue(j % GROUPS, j / GROUPS, (j % GROUPS) * spg + j / GROUPS);
+      for (uint32_t j = 0; j < first; ++j) issue(j % kTmaGroups, j / kTmaGroups, (j % kTmaGroups) * spg + j / kTmaGroups);
     }
     // 32-bit shared-window addresses (the generic-pointer forms re-derive the window base per chunk)
     const uint32_t tw = (t >> 5) * 64u + (t & 31u);  // env A of this thread within a chunk; env B = tw + 32
     const uint32_t state_u32 = smem_u32(s_state) + tw * 16u, full_u32 = smem_u32(full), empty_u32 = smem_u32(empty);
     const uint32_t act_u32 = smem_u32(s_act) + tw * static_cast<uint32_t>(sizeof(ActT));
-    [[maybe_unused]] const uint32_t out_u32 = smem_u32(s_out);
-    const uint32_t i_step = GROUPS * gridDim.x * kChunk;
+    const uint32_t i_step = kTmaGroups * gridDim.x * kChunk;
     uint32_t i = (blockIdx.x + g * gridDim.x) * kChunk + tw;  // env A of this thread in the current chunk; env B = i + 32
     uint32_t slot = slot0, phase = 0u;                      // slot / parity of the chunk consumed now
     uint32_t prev_slot = slot0, prev_phase = 0u;            // ... and of the previous iteration (the one to refill)
 
-    [[maybe_unused]] uint32_t trace_m = 0;
     auto body = [&](auto full_tag, auto recycle_tag) {
       constexpr bool FULL = decltype(full_tag)::value;
       constexpr bool RECYCLE = decltype(recycle_tag)::value;
@@ -261,7 +204,6 @@ __global__ void __launch_bounds__(GROUPS * GSZ, 1024 / (GROUPS * GSZ))
       const bool live_a = FULL || i < n, live_b = FULL || i + kB < n;
       const bool act_tma = FULL && action_via_tma;  // partial tail: consumers read their actions directly
       mbar_wait_u32(full_u32 + slot * 8u, phase);
-      EMEI_TRACE(2 + 2 * trace_m);  // this chunk's bytes have landed
       const uint32_t sl = state_u32 + slot * (kChunk * 16u);
       float4 ya = live_a ? lds128(sl) : make_float4(0.f, 0.f, 0.f, 0.f);
       float4 yb = live_b ? lds128(sl + kB * 16u) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -327,73 +269,27 @@ __global__ void __launch_bounds__(GROUPS * GSZ, 1024 / (GROUPS * GSZ))
       float rew_a, rew_b;
       bool nd_a, nd_b;
       float4 oa, ob;
-      cartpole_outcome<IP>(na, true, ca, k, rew_a, nd_a, oa);
-      cartpole_outcome<IP>(nb, true, cb, k, rew_b, nd_b, ob);
-      if constexpr (BULK && FULL) {
-        // stage the outputs: next state over this thread's own input rows, reward / done in the slot's output area;
-        // lane 0 then writes the warp's 64 envs with three bulk copies (1024 + 256 + 64 bytes)
-        const uint32_t ol = out_u32 + slot * kChunkOutBytes;
-        sts128(sl, na);
-        sts128(sl + kB * 16u, nb);
-        sts32(ol + tw * 4u, rew_a);
-        sts32(ol + (tw + kB) * 4u, rew_b);
-        sts8(ol + kChunk * 4u + tw, nd_a ? 0u : 1u);
-        sts8(ol + kChunk * 4u + tw + kB, nd_b ? 0u : 1u);
-        if constexpr (HAS_OBS) {
-          obs_out[i] = oa;
-          obs_out[i + kB] = ob;
-        }
-        fence_proxy_async_smem();
-        __syncwarp();
-        if ((t & 31u) == 0) {
-          const uint32_t w0 = tw;  // first env of this warp within the chunk
-          tma_store_1d(state_out + i, sl, 64u * 16u);
-          tma_store_1d(reward + i, ol + w0 * 4u, 64u * 4u);
-          tma_store_1d(done + i, ol + kChunk * 4u + w0, 64u);
-          tma_store_commit();
-        }
-        r_acc += rew_a + rew_b;
-        d_cnt += (nd_a ? 0u : 1u) + (nd_b ? 0u : 1u);
-      } else {
-        float4* so = state_out + i;
-        float* ro = reward + i;
-        uint8_t* dn = done + i;
-#if defined(EMEI_TMA_STREAM_HINTS) && EMEI_TMA_STREAM_HINTS >= 2  // development A/B: streaming (evict-first) stores
-        if (live_a) {
-          __stcs(so, na);
-          __stcs(ro, rew_a);
-          __stcs(dn, static_cast<uint8_t>(nd_a ? 0 : 1));
-          r_acc += rew_a;
-          d_cnt += nd_a ? 0u : 1u;
-        }
-        if (live_b) {
-          __stcs(so + kB, nb);
-          __stcs(ro + kB, rew_b);
-          __stcs(dn + kB, static_cast<uint8_t>(nd_b ? 0 : 1));
-          r_acc += rew_b;
-          d_cnt += nd_b ? 0u : 1u;
-        }
-        if (false)
-#endif
-        if (live_a) {
-          so[0] = na;
-          if constexpr (HAS_OBS) obs_out[i] = oa;
-          ro[0] = rew_a;
-          dn[0] = nd_a ? 0 : 1;
-          r_acc += rew_a;
-          d_cnt += nd_a ? 0u : 1u;
-        }
-        if (live_b) {
-          so[kB] = nb;
-          if constexpr (HAS_OBS) obs_out[i + kB] = ob;
-          ro[kB] = rew_b;
-          dn[kB] = nd_b ? 0 : 1;
-          r_acc += rew_b;
-          d_cnt += nd_b ? 0u : 1u;
-        }
+      cartpole_outcome<IP>(na, ca, k, rew_a, nd_a, oa);
+      cartpole_outcome<IP>(nb, cb, k, rew_b, nd_b, ob);
+      float4* so = state_out + i;
+      float* ro = reward + i;
+      uint8_t* dn = done + i;
+      if (live_a) {
+        so[0] = na;
+        if constexpr (HAS_OBS) obs_out[i] = oa;
+        ro[0] = rew_a;
+        dn[0] = nd_a ? 0 : 1;
+        r_acc += rew_a;
+        d_cnt += nd_a ? 0u : 1u;
       }
-      EMEI_TRACE(3 + 2 * trace_m);  // this chunk's stores are issued
-      ++trace_m;
+      if (live_b) {
+        so[kB] = nb;
+        if constexpr (HAS_OBS) obs_out[i + kB] = ob;
+        ro[kB] = rew_b;
+        dn[kB] = nd_b ? 0 : 1;
+        r_acc += rew_b;
+        d_cnt += nd_b ? 0u : 1u;
+      }
     };
 
     if (!recycling) {
@@ -427,14 +323,7 @@ __global__ void __launch_bounds__(GROUPS * GSZ, 1024 / (GROUPS * GSZ))
       }
     }
   }
-#ifdef EMEI_TMA_TRACE
-  if (g_tma_trace != nullptr && (tid % kBlock) == 0) g_tma_trace[(static_cast<size_t>(blockIdx.x) * GROUPS + tid / kBlock) * 64 + 1] = tma_now();  // group done
-#endif
-  if constexpr (BULK) {  // the staged outputs must have been read before the CTA's shared memory goes away
-    if ((tid & 31u) == 0) tma_store_wait_read0();
-  }
   // ---- statistics: warp shuffles -> shared -> one atomic pair per CTA
-  constexpr int kTmaThreads = GROUPS * kBlock;
   if (stats != nullptr) {  // uniform across the grid
     double* s_r = reinterpret_cast<double*>(empty + n_slots);
     unsigned* s_d = reinterpret_cast<unsigned*>(s_r + kTmaThreads / 32);
@@ -498,17 +387,16 @@ __global__ void __launch_bounds__(kSmallBlock)
 }
 
 // slots, dynamic shared memory bytes for an action element size
-inline void tma_ring_shape(int action_bytes, int64_t chunks_per_cta, int* n_slots, size_t* smem_bytes, int groups = kTmaGroups,
-                           bool bulk = false, int budget = kTmaSmemBudget, int gsz = kBlock) {
-  const int slot_bytes = 2 * gsz * (16 + action_bytes) + (bulk ? 2 * gsz * 5 : 0);
-  int s = budget / slot_bytes;
+inline void tma_ring_shape(int action_bytes, int64_t chunks_per_cta, int* n_slots, size_t* smem_bytes) {
+  const int slot_bytes = static_cast<int>(kChunk) * (16 + action_bytes);
+  int s = kTmaSmemBudget / slot_bytes;
   if (s > kTmaMaxSlots) s = kTmaMaxSlots;
   if (s > chunks_per_cta) s = static_cast<int>(chunks_per_cta);
-  s = (s + groups - 1) / groups * groups;  // every consumer group owns n_slots / groups slots
-  while (s * slot_bytes > budget) s -= groups;
-  if (s < groups) s = groups;
+  s = (s + kTmaGroups - 1) / kTmaGroups * kTmaGroups;  // every consumer group owns n_slots / kTmaGroups slots
+  while (s * slot_bytes > kTmaSmemBudget) s -= kTmaGroups;
+  if (s < kTmaGroups) s = kTmaGroups;
   *n_slots = s;
-  *smem_bytes = static_cast<size_t>(s) * slot_bytes + 2 * s * sizeof(uint64_t) + (groups * gsz / 32) * (sizeof(double) + sizeof(unsigned)) + 16;
+  *smem_bytes = static_cast<size_t>(s) * slot_bytes + 2 * s * sizeof(uint64_t) + (kTmaThreads / 32) * (sizeof(double) + sizeof(unsigned)) + 16;
 }
 
 // opt in to > 48 KB of dynamic shared memory: the attribute is PER DEVICE, so it is set once per (kernel
@@ -523,22 +411,6 @@ inline cudaError_t tma_allow_smem() {
     done[d] = true;
   }
   return cudaSuccess;
-}
-
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl_smem(void (*kernel)(KArgs...), int grid, int block, size_t smem, cudaStream_t stream, Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(static_cast<unsigned>(grid), 1, 1);
-  cfg.blockDim = dim3(static_cast<unsigned>(block), 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  static const bool no_pdl = getenv("EMEI_NO_PDL") != nullptr;  // development A/B: ordinary stream order (griddepcontrol.* become no-ops)
-  cfg.numAttrs = no_pdl ? 0 : 1;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
 template <bool IP, int FR>
@@ -587,19 +459,19 @@ inline void launch_cartpole_f32_tma(int ak, cudaStream_t s, const float* state_i
     // depth 6-8 is best (32.2 -> 29.9 us), at 2^18 depth 3 (4.70 -> 3.77 us).
     const int64_t per_cta = (chunks + grid - 1) / grid;
     const int depth = static_cast<int>(per_cta / 5 + 1 < 3 ? 3 : (per_cta / 5 + 1 > 8 ? 8 : per_cta / 5 + 1));
-    const int act_tma = ((reinterpret_cast<uintptr_t>(act) & 15u) == 0 ? 1 : 0) | 2 | (kTmaProducerGroup << 8) | (depth << 16);
+    const int act_tma = ((reinterpret_cast<uintptr_t>(act) & 15u) == 0 ? 1 : 0) | 2 | (depth << 16);
     switch (ak) {
-#define EMEI_AK(A)                                                                                                       \
-  case A:                                                                                                                \
-    if (obs4 != nullptr) {                                                                                               \
-      if (tma_allow_smem<cartpole_step_f32_tma_kernel<IP, A, FR, true>>() == cudaSuccess)                                  \
-        launch_pdl_smem(cartpole_step_f32_tma_kernel<IP, A, FR, true>, grid, kTmaThreads, smem, s, in4, out4, obs4, act, \
-                        reward + off, done + off, stats, static_cast<uint32_t>(m), n_slots, act_tma, k);                 \
-    } else {                                                                                                             \
-      if (tma_allow_smem<cartpole_step_f32_tma_kernel<IP, A, FR, false>>() == cudaSuccess)                                 \
-        launch_pdl_smem(cartpole_step_f32_tma_kernel<IP, A, FR, false>, grid, kTmaThreads, smem, s, in4, out4, obs4, act, \
-                        reward + off, done + off, stats, static_cast<uint32_t>(m), n_slots, act_tma, k);                 \
-    }                                                                                                                    \
+#define EMEI_AK(A)                                                                                                  \
+  case A:                                                                                                           \
+    if (obs4 != nullptr) {                                                                                          \
+      if (tma_allow_smem<cartpole_step_f32_tma_kernel<IP, A, FR, true>>() == cudaSuccess)                             \
+        launch_pdl(cartpole_step_f32_tma_kernel<IP, A, FR, true>, grid, kTmaThreads, smem, s, in4, out4, obs4, act, \
+                   reward + off, done + off, stats, static_cast<uint32_t>(m), n_slots, act_tma, k);                 \
+    } else {                                                                                                        \
+      if (tma_allow_smem<cartpole_step_f32_tma_kernel<IP, A, FR, false>>() == cudaSuccess)                            \
+        launch_pdl(cartpole_step_f32_tma_kernel<IP, A, FR, false>, grid, kTmaThreads, smem, s, in4, out4, obs4, act, \
+                   reward + off, done + off, stats, static_cast<uint32_t>(m), n_slots, act_tma, k);                 \
+    }                                                                                                               \
     break;
       EMEI_AK(EMEI_ACTION_DISCRETE_U8)
       EMEI_AK(EMEI_ACTION_DISCRETE_I32)
@@ -611,9 +483,11 @@ inline void launch_cartpole_f32_tma(int ak, cudaStream_t s, const float* state_i
   }
 }
 
-inline void cartpole_step_f32_tma_dispatch(const float* state_in, float* state_out, float* obs_out, const void* action,
-                                           float* reward, uint8_t* done, double* stats, int64_t n,
-                                           const emei_cartpole_params& p, cudaStream_t s) {
+// R = float.  A template, so that the float64 translation unit, which sees this header too, instantiates none of the kernels.
+template <typename R>
+inline void cartpole_step_f32_tma_dispatch(const R* state_in, R* state_out, R* obs_out, const void* action, R* reward,
+                                           uint8_t* done, double* stats, int64_t n, const emei_cartpole_params& p,
+                                           cudaStream_t s) {
   const CartPoleF32Consts k = make_cartpole_f32_consts(p);
   const bool ip = p.variant > EMEI_CARTPOLE_SWINGUP;
   const int ab = action_kind_bytes(p.action_kind);

@@ -10,7 +10,6 @@
 // branches (on the circle: two sincos; free flight: four FMAs) use the lean float32 math of
 // f32math.cuh; only a landing (rare) evaluates asin / fmod / sqrt through libm.
 #pragma once
-#include <cstdlib>
 #include "common.cuh"
 #include "f32math.cuh"
 
@@ -228,38 +227,26 @@ __global__ void __launch_bounds__(kBlock, MINB)
 // (32 registers, 53 KB of loads in flight per SM) 0.687 ms = 0.835 of the copy peak; 2 x 6: 0.635; 2 x 5: 0.618; 4 x 4
 // (64 registers, 106 KB in flight): 0.611 ms = 0.94; shapes that spill (4 x 5, 8 x 3) collapse.  At 2^23 envs (the 8-way
 // strong-scaled shard of BASELINE configs[3]) the two ends measure the same (84 vs 86 us), so small batches keep the shape with
-// the most CTAs.  EMEI_CB_SHAPE overrides the choice (development knob for that A/B).
-inline int cb_shape(int64_t n) {
-  static const int forced = []() {
-    const char* e = getenv("EMEI_CB_SHAPE");
-    return e ? atoi(e) : 0;
-  }();
-  if (forced) return forced;
-  return n >= (int64_t{1} << 24) ? 44 : 18;
-}
-
-inline void charged_ball_step_f32_dispatch(uint8_t* on_circle, float* circle, float* free_state, const void* action,
-                                           float* reward, uint8_t* done, double* stats, int64_t n,
-                                           const emei_charged_ball_params& p, cudaStream_t s) {
+// the most CTAs.
+// R = float.  A template, so that the translation units that see this header without calling it instantiate none of the kernels.
+template <typename R>
+inline void charged_ball_step_f32_dispatch(uint8_t* on_circle, R* circle, R* free_state, const void* action, R* reward,
+                                           uint8_t* done, double* stats, int64_t n, const emei_charged_ball_params& p,
+                                           cudaStream_t s) {
   const ChargedBallF32Consts k = make_cb_f32_consts(p);
   float2* c2 = reinterpret_cast<float2*>(circle);
   float4* f4 = reinterpret_cast<float4*>(free_state);
-  const int shape = cb_shape(n);
+  const bool large = n >= (int64_t{1} << 24);
 #define EMEI_CB_LAUNCH(A, EPT, MINB)                                                                                               \
   launch_pdl(charged_ball_step_f32_kernel<A, EPT, MINB>, persistent_grid((n + EPT - 1) / EPT, kBlock, MINB), kBlock, s, on_circle, c2, f4, \
              action, reward, done, stats, n, k)
   switch (p.action_kind) {
-#define EMEI_AK(A)                                                                                                 \
-  case A:                                                                                                          \
-    if (shape == 26) EMEI_CB_LAUNCH(A, 2, 6);                                                                      \
-    else if (shape == 25) EMEI_CB_LAUNCH(A, 2, 5);                                                                 \
-    else if (shape == 24) EMEI_CB_LAUNCH(A, 2, 4);                                                                 \
-    else if (shape == 44) EMEI_CB_LAUNCH(A, 4, 4);                                                                 \
-    else if (shape == 45) EMEI_CB_LAUNCH(A, 4, 5);                                                                 \
-    else if (shape == 43) EMEI_CB_LAUNCH(A, 4, 3);                                                                 \
-    else if (shape == 83) EMEI_CB_LAUNCH(A, 8, 3);                                                                 \
-    else if (shape == 82) EMEI_CB_LAUNCH(A, 8, 2);                                                                 \
-    else EMEI_CB_LAUNCH(A, 1, 8);                                                                                  \
+#define EMEI_AK(A)              \
+  case A:                       \
+    if (large)                  \
+      EMEI_CB_LAUNCH(A, 4, 4);  \
+    else                        \
+      EMEI_CB_LAUNCH(A, 1, 8);  \
     break;
     EMEI_AK(EMEI_ACTION_DISCRETE_U8)
     EMEI_AK(EMEI_ACTION_DISCRETE_I32)

@@ -39,6 +39,37 @@ inline int launch_status() {
   return e == cudaSuccess ? EMEI_OK : static_cast<int>(e);
 }
 
+// ---------------------------------------------------------------------------------------------
+// parameter checks shared by the entry points of each family, in the order every entry point applies them
+// ---------------------------------------------------------------------------------------------
+inline bool action_kind_valid(int ak) { return ak >= EMEI_ACTION_DISCRETE_U8 && ak <= EMEI_ACTION_CONTINUOUS_F64; }
+inline int check_cartpole_params(const emei_cartpole_params& p) {
+  if (p.variant < EMEI_CARTPOLE_BALANCING || p.variant > EMEI_IP_BOUNDARY_SWINGUP) return EMEI_ERR_BAD_VARIANT;
+  if (!action_kind_valid(p.action_kind)) return EMEI_ERR_BAD_ACTION_KIND;
+  if (p.freq_rate < 1 || !(p.dt > 0.0)) return EMEI_ERR_BAD_PARAM;
+  return EMEI_OK;
+}
+inline int check_i2p_params(const emei_i2p_params& p) {
+  if (p.variant < EMEI_I2P_REBOUND_BALANCING || p.variant > EMEI_I2P_BOUNDARY_SWINGUP) return EMEI_ERR_BAD_VARIANT;
+  if (!action_kind_valid(p.action_kind)) return EMEI_ERR_BAD_ACTION_KIND;
+  if (p.freq_rate < 1 || !(p.dt > 0.0) || !(p.mass_cart > 0.0) || !(p.mass_pole0 > 0.0) || !(p.mass_pole1 > 0.0) ||
+      !(p.length0 > 0.0) || !(p.length1 > 0.0))
+    return EMEI_ERR_BAD_PARAM;
+  return EMEI_OK;
+}
+inline int check_charged_ball_params(const emei_charged_ball_params& p) {
+  if (!action_kind_valid(p.action_kind)) return EMEI_ERR_BAD_ACTION_KIND;
+  if (p.freq_rate < 1 || !(p.time_step > 0.0) || !(p.radius > 0.0) || !(p.mass_ball > 0.0)) return EMEI_ERR_BAD_PARAM;
+  return EMEI_OK;
+}
+// state noise: sigma[0, dim) >= 0 (no noise: EMEI_OK)
+inline int check_noise_params(const emei_noise_params* z, int dim) {
+  if (z != nullptr)
+    for (int j = 0; j < dim; ++j)
+      if (!(z->sigma[j] >= 0.0)) return EMEI_ERR_BAD_PARAM;
+  return EMEI_OK;
+}
+
 inline int grid_for(int64_t n, int per_block) {
   int64_t g = (n + per_block - 1) / per_block;
   return static_cast<int>(g);
@@ -80,12 +111,13 @@ inline int resident_grid(void (*kernel)(KArgs...), int64_t n) {
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
+// smem: dynamic shared memory bytes (the overload without it launches with none)
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, cudaStream_t stream, Args... args) {
+inline cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, size_t smem, cudaStream_t stream, Args... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(static_cast<unsigned>(grid), 1, 1);
   cfg.blockDim = dim3(static_cast<unsigned>(block), 1, 1);
-  cfg.dynamicSmemBytes = 0;
+  cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -94,7 +126,10 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, cud
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
-
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, cudaStream_t stream, Args... args) {
+  return launch_pdl(kernel, grid, block, size_t{0}, stream, args...);
+}
 
 // ---------------------------------------------------------------------------------------------
 // vector types: one env row (4 scalars) per 128-bit (f32) / 2 x 128-bit (f64) access
@@ -170,35 +205,7 @@ __device__ __forceinline__ double warp_sum(double v) {
   return v;
 }
 
-// Must be called by ALL threads of the CTA (no early exit before it).
-__device__ __forceinline__ void block_stats_accumulate(double* stats, double reward_sum, bool done) {
-  if (stats == nullptr) return;  // uniform across the grid
-  __shared__ double s_r[kBlock / 32];
-  __shared__ unsigned s_d[kBlock / 32];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  double r = warp_sum(reward_sum);
-  unsigned d = __popc(__ballot_sync(0xffffffffu, done));
-  if (lane == 0) {
-    s_r[warp] = r;
-    s_d[warp] = d;
-  }
-  __syncthreads();
-  if (warp == 0) {
-    const int nw = blockDim.x >> 5;
-    double rr = lane < nw ? s_r[lane] : 0.0;
-    unsigned dd = lane < nw ? s_d[lane] : 0u;
-    rr = warp_sum(rr);
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) dd += __shfl_xor_sync(0xffffffffu, dd, o);
-    if (lane == 0) {
-      atomicAdd(&stats[0], rr);
-      atomicAdd(&stats[1], static_cast<double>(dd));  // exact: counts << 2^53
-    }
-  }
-}
-
-// Same, for kernels whose threads carry several units: per-thread reward partial + done COUNT.
-// Must be called by ALL threads of the CTA.
+// Per-thread reward partial + done COUNT of the thread's units.  Must be called by ALL threads of the CTA.
 __device__ __forceinline__ void block_stats_accumulate_counts(double* stats, double reward_sum, unsigned done_count) {
   if (stats == nullptr) return;  // uniform across the grid
   __shared__ double s_r2[kBlock / 32];
@@ -330,6 +337,14 @@ struct Philox {
     out[3] = c[3];
   }
 };
+
+// Philox purpose words (the counter's last word): one per random stream of the library
+constexpr uint32_t kPurposeUniform = 1;        // initial states, uniform families
+constexpr uint32_t kPurposeGaussian = 2;       // initial states, Gaussian families
+constexpr uint32_t kPurposeChargedBall = 3;    // initial states, charged ball
+constexpr uint32_t kPurposeRolloutAction = 4;  // the rollouts' random policy
+constexpr uint32_t kPurposeRolloutReset = 5;   // the float32 rollouts' lean uniform reset
+constexpr uint32_t kPurposeObsNoise = 6;       // per-sub-step state noise (bits 8..: the high word of the block index)
 
 // 53-bit uniform in [0,1) from two 32-bit words (same construction as numpy's next_double)
 __host__ __device__ inline double u01_from_bits(uint32_t hi, uint32_t lo) {

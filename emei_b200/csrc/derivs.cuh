@@ -149,9 +149,7 @@ int cartpole_step_derivs(const R* state_in, const void* action, R* jac, R* rewar
                          bool vjp) {
   if (n < 0) return EMEI_ERR_BAD_SIZE;
   EMEI_CHECK_PTR(p);
-  if (p->variant < EMEI_CARTPOLE_BALANCING || p->variant > EMEI_IP_BOUNDARY_SWINGUP) return EMEI_ERR_BAD_VARIANT;
-  if (p->action_kind < EMEI_ACTION_DISCRETE_U8 || p->action_kind > EMEI_ACTION_CONTINUOUS_F64) return EMEI_ERR_BAD_ACTION_KIND;
-  if (p->freq_rate < 1 || !(p->dt > 0.0)) return EMEI_ERR_BAD_PARAM;
+  if (const int e = check_cartpole_params(*p)) return e;
   if (vjp && g_action != nullptr && p->action_kind < EMEI_ACTION_CONTINUOUS_F32) return EMEI_ERR_BAD_ACTION_KIND;
   if (n == 0) return EMEI_OK;
   EMEI_CHECK_PTR(state_in);
@@ -328,11 +326,7 @@ int i2p_step_derivs(const R* state_in, const void* action, R* jac, R* reward_gra
                     const R* g_reward, R* g_state_in, R* g_action, int64_t n, const emei_i2p_params* p, emei_stream_t stream, bool vjp) {
   if (n < 0) return EMEI_ERR_BAD_SIZE;
   EMEI_CHECK_PTR(p);
-  if (p->variant < EMEI_I2P_REBOUND_BALANCING || p->variant > EMEI_I2P_BOUNDARY_SWINGUP) return EMEI_ERR_BAD_VARIANT;
-  if (p->action_kind < EMEI_ACTION_DISCRETE_U8 || p->action_kind > EMEI_ACTION_CONTINUOUS_F64) return EMEI_ERR_BAD_ACTION_KIND;
-  if (p->freq_rate < 1 || !(p->dt > 0.0) || !(p->mass_cart > 0.0) || !(p->mass_pole0 > 0.0) || !(p->mass_pole1 > 0.0) ||
-      !(p->length0 > 0.0) || !(p->length1 > 0.0))
-    return EMEI_ERR_BAD_PARAM;
+  if (const int e = check_i2p_params(*p)) return e;
   if (vjp && g_action != nullptr && p->action_kind < EMEI_ACTION_CONTINUOUS_F32) return EMEI_ERR_BAD_ACTION_KIND;
   if (n == 0) return EMEI_OK;
   EMEI_CHECK_PTR(state_in);

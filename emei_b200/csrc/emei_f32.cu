@@ -1,9 +1,4 @@
 // float32 (tolerance) mode of every entry point.  FMA contraction allowed.
 #define EMEI_REAL float
 #define EMEI_FN(name) name##_f32
-#include "cartpole_f32.cuh"
-#include "cartpole_tma.cuh"
-#include "charged_ball_f32.cuh"
-#define EMEI_HAVE_CARTPOLE_F32 1
-#define EMEI_HAVE_CHARGED_BALL_F32 1
 #include "impl.inc"

@@ -6,7 +6,7 @@ namespace {
 using namespace emei;
 
 // validation + conversion shared by the two entry points; returns EMEI_OK or an error code
-int make_rollout(const emei_rollout_params* r, int max_init_kind, const void* actions, float* rec_observations,
+int make_rollout(const emei_rollout_params* r, const void* actions, float* rec_observations,
                  float* rec_next_observations, void* rec_actions, float* rec_rewards, uint8_t* rec_dones,
                  uint8_t* rec_timeouts, int32_t* ep_step, float* ep_return, int32_t* ep_index, double* stats,
                  RolloutConsts& rc, RolloutIO& io) {
@@ -23,7 +23,6 @@ int make_rollout(const emei_rollout_params* r, int max_init_kind, const void* ac
     EMEI_CHECK_ALIGN16(rec_observations);
     EMEI_CHECK_ALIGN16(rec_next_observations);
   }
-  (void)max_init_kind;
   rc.horizon = r->horizon;
   rc.max_episode_steps = r->max_episode_steps;
   rc.auto_reset = r->auto_reset;
@@ -58,16 +57,14 @@ extern "C" int emei_cartpole_rollout_f32(float* state_io, int32_t* episode_step_
   if (n < 0 || n > kCartPoleMaxLaunch) return EMEI_ERR_BAD_SIZE;
   EMEI_CHECK_PTR(p);
   EMEI_CHECK_PTR(r);
-  if (p->variant < EMEI_CARTPOLE_BALANCING || p->variant > EMEI_IP_BOUNDARY_SWINGUP) return EMEI_ERR_BAD_VARIANT;
-  if (p->action_kind < EMEI_ACTION_DISCRETE_U8 || p->action_kind > EMEI_ACTION_CONTINUOUS_F64)
-    return EMEI_ERR_BAD_ACTION_KIND;
-  if (p->freq_rate < 1 || !(p->dt > 0.0) || r->horizon < 0 || (r->init_kind != 0 && r->init_kind != 1)) return EMEI_ERR_BAD_PARAM;
+  if (const int e = check_cartpole_params(*p)) return e;
+  if (r->horizon < 0 || (r->init_kind != 0 && r->init_kind != 1)) return EMEI_ERR_BAD_PARAM;
   if (n == 0 || r->horizon == 0) return EMEI_OK;
   EMEI_CHECK_PTR(state_io);
   EMEI_CHECK_ALIGN16(state_io);
   RolloutConsts rc;
   RolloutIO io;
-  const int rcode = make_rollout(r, 1, actions, rec_observations, rec_next_observations, rec_actions, rec_rewards, rec_dones,
+  const int rcode = make_rollout(r, actions, rec_observations, rec_next_observations, rec_actions, rec_rewards, rec_dones,
                                  rec_timeouts, episode_step_io, episode_return_io, episode_index_io, stats, rc, io);
   if (rcode != EMEI_OK) return rcode;
   const CartPoleF32Consts k = make_cartpole_f32_consts(*p);
@@ -96,10 +93,8 @@ extern "C" int emei_charged_ball_rollout_f32(uint8_t* on_circle_io, float* circl
   if (n < 0 || n > kCartPoleMaxLaunch) return EMEI_ERR_BAD_SIZE;
   EMEI_CHECK_PTR(p);
   EMEI_CHECK_PTR(r);
-  if (p->action_kind < EMEI_ACTION_DISCRETE_U8 || p->action_kind > EMEI_ACTION_CONTINUOUS_F64)
-    return EMEI_ERR_BAD_ACTION_KIND;
-  if (p->freq_rate < 1 || !(p->time_step > 0.0) || !(p->radius > 0.0) || !(p->mass_ball > 0.0) || r->horizon < 0)
-    return EMEI_ERR_BAD_PARAM;
+  if (const int e = check_charged_ball_params(*p)) return e;
+  if (r->horizon < 0) return EMEI_ERR_BAD_PARAM;
   if (n == 0 || r->horizon == 0) return EMEI_OK;
   EMEI_CHECK_PTR(on_circle_io);
   EMEI_CHECK_PTR(circle_io);
@@ -108,7 +103,7 @@ extern "C" int emei_charged_ball_rollout_f32(uint8_t* on_circle_io, float* circl
   EMEI_CHECK_ALIGN16(free_state_io);
   RolloutConsts rc;
   RolloutIO io;
-  const int rcode = make_rollout(r, 2, actions, rec_observations, rec_next_observations, rec_actions, rec_rewards, rec_dones,
+  const int rcode = make_rollout(r, actions, rec_observations, rec_next_observations, rec_actions, rec_rewards, rec_dones,
                                  rec_timeouts, episode_step_io, episode_return_io, episode_index_io, stats, rc, io);
   if (rcode != EMEI_OK) return rcode;
   rc.init_kind = 2;  // charged_ball.py:84-94 is the only reset sampler of this family

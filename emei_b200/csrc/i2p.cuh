@@ -238,14 +238,8 @@ int i2p_step(const R* state_in, R* state_out, R* obs_out, const void* action, R*
              int64_t n, const emei_i2p_params* p, emei_stream_t stream, const emei_noise_params* noise = nullptr) {
   if (n < 0) return EMEI_ERR_BAD_SIZE;
   EMEI_CHECK_PTR(p);
-  if (p->variant < EMEI_I2P_REBOUND_BALANCING || p->variant > EMEI_I2P_BOUNDARY_SWINGUP) return EMEI_ERR_BAD_VARIANT;
-  if (p->action_kind < EMEI_ACTION_DISCRETE_U8 || p->action_kind > EMEI_ACTION_CONTINUOUS_F64) return EMEI_ERR_BAD_ACTION_KIND;
-  if (p->freq_rate < 1 || !(p->dt > 0.0) || !(p->mass_cart > 0.0) || !(p->mass_pole0 > 0.0) || !(p->mass_pole1 > 0.0) ||
-      !(p->length0 > 0.0) || !(p->length1 > 0.0))
-    return EMEI_ERR_BAD_PARAM;
-  if (noise != nullptr)
-    for (int j = 0; j < 6; ++j)
-      if (!(noise->sigma[j] >= 0.0)) return EMEI_ERR_BAD_PARAM;
+  if (const int e = check_i2p_params(*p)) return e;
+  if (const int e = check_noise_params(noise, 6)) return e;
   if (n == 0) return EMEI_OK;
   EMEI_CHECK_PTR(state_in);
   EMEI_CHECK_PTR(state_out);

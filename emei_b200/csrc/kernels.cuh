@@ -7,6 +7,8 @@
 #pragma once
 #include "common.cuh"
 #include "f32math.cuh"
+#include "cartpole_tma.cuh"
+#include "charged_ball_f32.cuh"
 
 namespace emei {
 
@@ -73,7 +75,20 @@ __device__ __forceinline__ double euler_cp(double y, double d, const CartPoleCon
 // pair of Philox block (g * 4 + pr) keyed by (seed, e) -- same arithmetic as init_gaussian_kernel
 // (mirror: oracle/philox.py obs_noise).  on == 0: no noise, no cost beyond one uniform branch.
 // ---------------------------------------------------------------------------------------------
-constexpr uint32_t kPurposeObsNoise = 6;
+
+// Box-Muller: the standard-normal pair (rad cs, rad sn) of one Philox block (numpy-style 53-bit uniforms, float64
+// arithmetic), returned as its three factors so that a caller forms only the products it stores.  The one normal sampler
+// of the library: state noise, init_gaussian_kernel and the resets of both rollout kernels.
+__device__ __forceinline__ void philox_normal_pair(uint64_t seed, uint64_t env, uint32_t block, uint32_t purpose, double& rad,
+                                                   double& cs, double& sn) {
+  uint32_t w[4];
+  Philox::generate(seed, env, block, purpose, w);
+  const double u1 = 1.0 - u01_from_bits(w[0], w[1]);  // (0,1]
+  const double u2 = u01_from_bits(w[2], w[3]);
+  rad = sqrt(-2.0 * log(u1));
+  sincospi(2.0 * u2, &sn, &cs);
+}
+
 struct NoiseConsts {
   double sigma[6];
   unsigned long long seed, env_offset, substep0;  // substep0 = step * freq_rate: global index of this call's first sub-step
@@ -96,13 +111,8 @@ __device__ __forceinline__ void add_state_noise(R (&y)[DIM], const NoiseConsts& 
 #pragma unroll
   for (int pr = 0; pr < DIM / 2; ++pr) {
     const unsigned long long blk = g * 4ull + static_cast<unsigned long long>(pr);
-    uint32_t w[4];
-    Philox::generate(z.seed, env, static_cast<uint32_t>(blk), kPurposeObsNoise | (static_cast<uint32_t>(blk >> 32) << 8), w);
-    const double u1 = 1.0 - u01_from_bits(w[0], w[1]);
-    const double u2 = u01_from_bits(w[2], w[3]);
-    const double rad = sqrt(-2.0 * log(u1));
-    double sn, cs;
-    sincospi(2.0 * u2, &sn, &cs);
+    double rad, cs, sn;
+    philox_normal_pair(z.seed, env, static_cast<uint32_t>(blk), kPurposeObsNoise | (static_cast<uint32_t>(blk >> 32) << 8), rad, cs, sn);
     y[2 * pr] = static_cast<R>(__dadd_rn(static_cast<double>(y[2 * pr]), __dmul_rn(z.sigma[2 * pr], __dmul_rn(rad, cs))));
     y[2 * pr + 1] = static_cast<R>(__dadd_rn(static_cast<double>(y[2 * pr + 1]), __dmul_rn(z.sigma[2 * pr + 1], __dmul_rn(rad, sn))));
   }
@@ -230,15 +240,10 @@ int cartpole_step(const R* state_in, R* state_out, R* obs_out, const void* actio
                   const emei_noise_params* noise = nullptr) {
   if (n < 0) return EMEI_ERR_BAD_SIZE;
   EMEI_CHECK_PTR(p);
-  if (p->variant < EMEI_CARTPOLE_BALANCING || p->variant > EMEI_IP_BOUNDARY_SWINGUP) return EMEI_ERR_BAD_VARIANT;
-  if (p->action_kind < EMEI_ACTION_DISCRETE_U8 || p->action_kind > EMEI_ACTION_CONTINUOUS_F64)
-    return EMEI_ERR_BAD_ACTION_KIND;
-  if (p->freq_rate < 1 || !(p->dt > 0.0)) return EMEI_ERR_BAD_PARAM;
-  if (noise != nullptr) {  // the noisy step exists for the MuJoCo-shell family only (mujoco_env.py:98-104)
-    if (p->variant < EMEI_IP_REBOUND_BALANCING) return EMEI_ERR_BAD_VARIANT;
-    for (int j = 0; j < 4; ++j)
-      if (!(noise->sigma[j] >= 0.0)) return EMEI_ERR_BAD_PARAM;
-  }
+  if (const int e = check_cartpole_params(*p)) return e;
+  // the noisy step exists for the MuJoCo-shell family only (mujoco_env.py:98-104)
+  if (noise != nullptr && p->variant < EMEI_IP_REBOUND_BALANCING) return EMEI_ERR_BAD_VARIANT;
+  if (const int e = check_noise_params(noise, 4)) return e;
   if (n == 0) return EMEI_OK;
   EMEI_CHECK_PTR(state_in);
   EMEI_CHECK_PTR(state_out);
@@ -249,14 +254,12 @@ int cartpole_step(const R* state_in, R* state_out, R* obs_out, const void* actio
   EMEI_CHECK_ALIGN16(state_out);
   if (obs_out) EMEI_CHECK_ALIGN16(obs_out);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-#ifdef EMEI_HAVE_CARTPOLE_F32
   if constexpr (sizeof(R) == 4) {  // lean float32 kernel: TMA-staged, packed f32x2 (cartpole_tma.cuh)
     if (noise == nullptr) {        // (the noisy step takes the generic kernel below: Philox + double Box-Muller dominate it)
-      cartpole_step_f32_tma_dispatch(state_in, state_out, obs_out, action, reward, done, stats, n, *p, s);
+      cartpole_step_f32_tma_dispatch<R>(state_in, state_out, obs_out, action, reward, done, stats, n, *p, s);
       return launch_status();
     }
   }
-#endif
   const CartPoleConsts<R> k = make_cartpole_consts<R>(*p);
   const NoiseConsts z = make_noise_consts(noise, p->freq_rate);
   if (p->variant <= EMEI_CARTPOLE_SWINGUP)
@@ -409,9 +412,7 @@ int charged_ball_step(uint8_t* on_circle, R* circle, R* free_state, const void* 
                       double* stats, int64_t n, const emei_charged_ball_params* p, emei_stream_t stream) {
   if (n < 0) return EMEI_ERR_BAD_SIZE;
   EMEI_CHECK_PTR(p);
-  if (p->action_kind < EMEI_ACTION_DISCRETE_U8 || p->action_kind > EMEI_ACTION_CONTINUOUS_F64)
-    return EMEI_ERR_BAD_ACTION_KIND;
-  if (p->freq_rate < 1 || !(p->time_step > 0.0) || !(p->radius > 0.0) || !(p->mass_ball > 0.0)) return EMEI_ERR_BAD_PARAM;
+  if (const int e = check_charged_ball_params(*p)) return e;
   if (n == 0) return EMEI_OK;
   EMEI_CHECK_PTR(on_circle);
   EMEI_CHECK_PTR(circle);
@@ -421,22 +422,18 @@ int charged_ball_step(uint8_t* on_circle, R* circle, R* free_state, const void* 
   EMEI_CHECK_PTR(done);
   EMEI_CHECK_ALIGN16(circle);
   EMEI_CHECK_ALIGN16(free_state);
-#ifdef EMEI_HAVE_CHARGED_BALL_F32
-  if constexpr (sizeof(R) == 4) {  // lean float32 kernel (charged_ball_f32.cuh)
-    charged_ball_step_f32_dispatch(on_circle, circle, free_state, action, reward, done, stats, n, *p,
-                                   static_cast<cudaStream_t>(stream));
-    return launch_status();
-  }
-#endif
-  const ChargedBallConsts<R> k = make_cb_consts<R>(*p);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const bool continuous = p->action_kind >= EMEI_ACTION_CONTINUOUS_F32;
-  if (sizeof(R) == 8 && continuous)
-    charged_ball_step_kernel<R, (sizeof(R) == 8)><<<resident_grid(charged_ball_step_kernel<R, (sizeof(R) == 8)>, n), kBlock, 0, s>>>(
-        on_circle, circle, free_state, action, reward, done, stats, n, k);
-  else
-    charged_ball_step_kernel<R, false><<<resident_grid(charged_ball_step_kernel<R, false>, n), kBlock, 0, s>>>(
-        on_circle, circle, free_state, action, reward, done, stats, n, k);
+  if constexpr (sizeof(R) == 4) {  // lean float32 kernel (charged_ball_f32.cuh)
+    charged_ball_step_f32_dispatch<R>(on_circle, circle, free_state, action, reward, done, stats, n, *p, s);
+  } else {
+    const ChargedBallConsts<R> k = make_cb_consts<R>(*p);
+    if (p->action_kind >= EMEI_ACTION_CONTINUOUS_F32)
+      charged_ball_step_kernel<R, true><<<resident_grid(charged_ball_step_kernel<R, true>, n), kBlock, 0, s>>>(
+          on_circle, circle, free_state, action, reward, done, stats, n, k);
+    else
+      charged_ball_step_kernel<R, false><<<resident_grid(charged_ball_step_kernel<R, false>, n), kBlock, 0, s>>>(
+          on_circle, circle, free_state, action, reward, done, stats, n, k);
+  }
   return launch_status();
 }
 
@@ -840,12 +837,38 @@ int sumsq(const R* x, int64_t n_elems, double* out, double* workspace, emei_stre
 // =============================================================================================
 // initial-state sampling (Philox4x32-10; value depends on (seed, env id, column) only)
 // =============================================================================================
-constexpr uint32_t kPurposeUniform = 1, kPurposeGaussian = 2, kPurposeChargedBall = 3;
-
 __host__ __device__ inline double philox_uniform(uint64_t seed, uint64_t env, int col, uint32_t purpose) {
   uint32_t w[4];
   Philox::generate(seed, env, static_cast<uint32_t>(col >> 1), purpose, w);
   return (col & 1) ? u01_from_bits(w[2], w[3]) : u01_from_bits(w[0], w[1]);
+}
+
+// Column col of a uniform initial state (cartpole.py:131-132,153-156): numpy Generator.uniform, low + (high-low)*next_double
+// (no FMA), + pi on pi_column (cartpole.py:155).  init_uniform_kernel and the resets of rollout_ref.cuh.
+__device__ __forceinline__ double uniform_initial_sample(uint64_t seed, uint64_t env, int col, double low, double high, int pi_column) {
+  const double u = philox_uniform(seed, env, col, kPurposeUniform);
+  double v = __dadd_rn(low, __dmul_rn(high - low, u));
+  if (col == pi_column) v = __dadd_rn(v, 3.141592653589793238462643383279502884);
+  return v;
+}
+
+// Charged-ball initial state (charged_ball.py:84-94): on the ring at theta = pi + U(-0.5, 0.5) with omega = U(-0.5, 0.5)
+// (float64 like the reference, then cast to R), f = (x, y, vx, vy) of that ring point.  init_charged_ball_kernel and the
+// resets of both rollout kernels.
+template <typename R>
+__device__ __forceinline__ void charged_ball_initial_sample(uint64_t seed, uint64_t env, R radius, R& th, R& om, R (&f)[4]) {
+  const double theta = __dadd_rn(__dadd_rn(-0.5, philox_uniform(seed, env, 0, kPurposeChargedBall)),
+                                 3.141592653589793238462643383279502884);
+  const double omega = __dadd_rn(-0.5, philox_uniform(seed, env, 1, kPurposeChargedBall));
+  th = static_cast<R>(theta);
+  om = static_cast<R>(omega);
+  R s, c;
+  sincos_r(th, &s, &c);
+  const R x = s * radius, y = c * radius;
+  f[0] = x;
+  f[1] = y;
+  f[2] = om * y;
+  f[3] = -om * x;
 }
 
 template <typename R>
@@ -856,10 +879,7 @@ __global__ void __launch_bounds__(kBlock)
   if (idx >= n * dim) return;
   const int64_t row = idx / dim;
   const int col = static_cast<int>(idx - row * dim);
-  const double u = philox_uniform(seed, env_offset + static_cast<uint64_t>(row), col, kPurposeUniform);
-  double v = __dadd_rn(low, __dmul_rn(high - low, u));  // numpy Generator.uniform: low + (high-low)*next_double (no FMA)
-  if (col == pi_column) v = __dadd_rn(v, 3.141592653589793238462643383279502884);  // cartpole.py:155
-  out[idx] = static_cast<R>(v);
+  out[idx] = static_cast<R>(uniform_initial_sample(seed, env_offset + static_cast<uint64_t>(row), col, low, high, pi_column));
 }
 
 struct GaussianTable {
@@ -877,13 +897,8 @@ __global__ void __launch_bounds__(kBlock)
   if (idx >= n * pairs) return;
   const int64_t row = idx / pairs;
   const int pr = static_cast<int>(idx - row * pairs);
-  uint32_t w[4];
-  Philox::generate(seed, env_offset + static_cast<uint64_t>(row), static_cast<uint32_t>(pr), kPurposeGaussian, w);
-  const double u1 = 1.0 - u01_from_bits(w[0], w[1]);  // (0,1]
-  const double u2 = u01_from_bits(w[2], w[3]);
-  const double rad = sqrt(-2.0 * log(u1));
-  double sn, cs;
-  sincospi(2.0 * u2, &sn, &cs);
+  double rad, cs, sn;
+  philox_normal_pair(seed, env_offset + static_cast<uint64_t>(row), static_cast<uint32_t>(pr), kPurposeGaussian, rad, cs, sn);
   const int c0 = 2 * pr, c1 = 2 * pr + 1;
   out[row * dim + c0] = static_cast<R>(__dadd_rn(t.mean[c0], __dmul_rn(t.sigma[c0], __dmul_rn(rad, cs))));
   if (c1 < dim) out[row * dim + c1] = static_cast<R>(__dadd_rn(t.mean[c1], __dmul_rn(t.sigma[c1], __dmul_rn(rad, sn))));
@@ -895,20 +910,13 @@ __global__ void __launch_bounds__(kBlock)
                              int64_t n, double radius, uint64_t seed, uint64_t env_offset) {
   const int64_t i = static_cast<int64_t>(blockIdx.x) * kBlock + threadIdx.x;
   if (i >= n) return;
-  // charged_ball.py:84-94 (float64 like the reference, then cast to the engine dtype)
-  const uint64_t env = env_offset + static_cast<uint64_t>(i);
-  const double theta = __dadd_rn(__dadd_rn(-0.5, philox_uniform(seed, env, 0, kPurposeChargedBall)),
-                                 3.141592653589793238462643383279502884);
-  const double omega = __dadd_rn(-0.5, philox_uniform(seed, env, 1, kPurposeChargedBall));
-  const R th = static_cast<R>(theta), om = static_cast<R>(omega), r = static_cast<R>(radius);
-  R s, c;
-  sincos_r(th, &s, &c);
-  const R x = s * r, y = c * r;
+  R th, om, f[4];
+  charged_ball_initial_sample<R>(seed, env_offset + static_cast<uint64_t>(i), static_cast<R>(radius), th, om, f);
   on_circle[i] = 1;
   circle[2 * i] = th;
   circle[2 * i + 1] = om;
-  Vec4<R> f = {x, y, om * y, -om * x};
-  f.store(free_state + 4 * i);
+  Vec4<R> v = {f[0], f[1], f[2], f[3]};
+  v.store(free_state + 4 * i);
 }
 
 template <typename R>

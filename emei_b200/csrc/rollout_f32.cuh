@@ -18,12 +18,9 @@
 // The kernel is written once over a `Dyn` policy (the env family): Dyn::Buffers (state arrays), Dyn::Regs
 // (one env in registers), load/store/observation/step/reset.
 #pragma once
-#include "cartpole_f32.cuh"
-#include "charged_ball_f32.cuh"
+#include "kernels.cuh"
 
 namespace emei {
-
-constexpr uint32_t kPurposeRolloutAction = 4;
 
 struct RolloutConsts {
   int horizon, max_episode_steps, auto_reset, random_policy, init_kind /*0 uniform, 1 gaussian, 2 charged ball*/, init_pi_column;
@@ -31,8 +28,6 @@ struct RolloutConsts {
   double init_low, init_high, mean[4], sigma[4];
   float act_low, act_high;
 };
-
-constexpr uint32_t kPurposeRolloutReset = 5;
 
 // In-rollout reset sample of one env row.
 // Uniform family (cartpole.py:131-132,153-156: U(low, high) per coordinate, + pi on the swing-up angle): the lean
@@ -56,13 +51,8 @@ static __device__ __noinline__ float4 rollout_init_state(const RolloutConsts& r,
   } else {
 #pragma unroll
     for (int pr = 0; pr < 2; ++pr) {
-      uint32_t w[4];
-      Philox::generate(seed, env, static_cast<uint32_t>(pr), 2u /*kPurposeGaussian*/, w);
-      const double u1 = 1.0 - u01_from_bits(w[0], w[1]);
-      const double u2 = u01_from_bits(w[2], w[3]);
-      const double rad = sqrt(-2.0 * log(u1));
-      double sn, cs;
-      sincospi(2.0 * u2, &sn, &cs);
+      double rad, cs, sn;
+      philox_normal_pair(seed, env, static_cast<uint32_t>(pr), kPurposeGaussian, rad, cs, sn);
       v[2 * pr] = static_cast<float>(__dadd_rn(r.mean[2 * pr], __dmul_rn(r.sigma[2 * pr], __dmul_rn(rad, cs))));
       v[2 * pr + 1] = static_cast<float>(__dadd_rn(r.mean[2 * pr + 1], __dmul_rn(r.sigma[2 * pr + 1], __dmul_rn(rad, sn))));
     }
@@ -72,18 +62,11 @@ static __device__ __noinline__ float4 rollout_init_state(const RolloutConsts& r,
 
 // same arithmetic as init_charged_ball_kernel<float> (kernels.cuh; charged_ball.py:84-94), one env
 static __device__ __noinline__ CBRegs rollout_init_charged_ball(float radius, unsigned long long env, unsigned long long seed) {
-  uint32_t w[4];
-  Philox::generate(seed, env, 0u, 3u /*kPurposeChargedBall*/, w);
-  const double theta = __dadd_rn(__dadd_rn(-0.5, u01_from_bits(w[0], w[1])), 3.141592653589793238462643383279502884);
-  const double omega = __dadd_rn(-0.5, u01_from_bits(w[2], w[3]));
   CBRegs e;
+  float f[4];
+  charged_ball_initial_sample<float>(seed, env, radius, e.theta, e.omega, f);
   e.on = true;
-  e.theta = static_cast<float>(theta);
-  e.omega = static_cast<float>(omega);
-  float s, c;
-  sincosf(e.theta, &s, &c);  // libm like the init kernel: the sample's bits do not depend on who draws it
-  const float x = s * radius, y = c * radius;
-  e.f = make_float4(x, y, e.omega * y, -e.omega * x);
+  e.f = make_float4(f[0], f[1], f[2], f[3]);
   cb_prepare(e);
   return e;
 }
@@ -177,8 +160,8 @@ struct CartPoleDyn {
       }
     }
     bool nd_a, nd_b;
-    cartpole_outcome<IP>(na, true, ca, k, rew[0], nd_a, next_obs[0]);
-    cartpole_outcome<IP>(nb, true, cb, k, rew[1], nd_b, next_obs[1]);
+    cartpole_outcome<IP>(na, ca, k, rew[0], nd_a, next_obs[0]);
+    cartpole_outcome<IP>(nb, cb, k, rew[1], nd_b, next_obs[1]);
     e[0].y = na;
     e[1].y = nb;
     terminated[0] = !nd_a;

@@ -17,8 +17,6 @@
 
 namespace emei {
 
-constexpr uint32_t kPurposeRefRolloutAction = 4;  // the action streams of rollout_f32.cuh (same bits for the same seed)
-
 struct RefRolloutConsts {
   int horizon, max_episode_steps, auto_reset, random_policy, init_pi_column, action_kind;
   unsigned long long seed_reset, seed_action, env_offset, t0;
@@ -104,14 +102,9 @@ struct RefCartPole {
   }
   __device__ static void reset(Regs& e, const RefRolloutConsts& r, const Consts&, unsigned long long env, unsigned long long seed) {
     R v[4];
-    if constexpr (!IP) {  // init_uniform_kernel (cartpole.py:131-132,153-156)
+    if constexpr (!IP) {  // init_uniform_kernel
 #pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        const double u = philox_uniform(seed, env, c, kPurposeUniform);
-        double x = __dadd_rn(r.init_low, __dmul_rn(r.init_high - r.init_low, u));
-        if (c == r.init_pi_column) x = __dadd_rn(x, 3.141592653589793238462643383279502884);
-        v[c] = static_cast<R>(x);
-      }
+      for (int c = 0; c < 4; ++c) v[c] = static_cast<R>(uniform_initial_sample(seed, env, c, r.init_low, r.init_high, r.init_pi_column));
     } else {  // init_gaussian_kernel (mujoco_env.py:137-140)
 #pragma unroll
       for (int pr = 0; pr < 2; ++pr) gaussian_pair<R>(r, env, seed, pr, v[2 * pr], v[2 * pr + 1]);
@@ -121,13 +114,8 @@ struct RefCartPole {
   template <typename T>
   __device__ __forceinline__ static void gaussian_pair(const RefRolloutConsts& r, unsigned long long env, unsigned long long seed, int pr,
                                                        T& v0, T& v1) {
-    uint32_t w[4];
-    Philox::generate(seed, env, static_cast<uint32_t>(pr), kPurposeGaussian, w);
-    const double u1 = 1.0 - u01_from_bits(w[0], w[1]);
-    const double u2 = u01_from_bits(w[2], w[3]);
-    const double rad = sqrt(-2.0 * log(u1));
-    double sn, cs;
-    sincospi(2.0 * u2, &sn, &cs);
+    double rad, cs, sn;
+    philox_normal_pair(seed, env, static_cast<uint32_t>(pr), kPurposeGaussian, rad, cs, sn);
     v0 = static_cast<T>(__dadd_rn(r.mean[2 * pr], __dmul_rn(r.sigma[2 * pr], __dmul_rn(rad, cs))));
     v1 = static_cast<T>(__dadd_rn(r.mean[2 * pr + 1], __dmul_rn(r.sigma[2 * pr + 1], __dmul_rn(rad, sn))));
   }
@@ -213,17 +201,10 @@ struct RefChargedBall {
     o[0] = e.f.x, o[1] = e.f.y, o[2] = e.f.z, o[3] = e.f.w;
   }
   __device__ static void reset(Regs& e, const RefRolloutConsts&, const Consts& k, unsigned long long env, unsigned long long seed) {
-    // init_charged_ball_kernel (charged_ball.py:84-94)
-    const double theta = __dadd_rn(__dadd_rn(-0.5, philox_uniform(seed, env, 0, kPurposeChargedBall)), 3.141592653589793238462643383279502884);
-    const double omega = __dadd_rn(-0.5, philox_uniform(seed, env, 1, kPurposeChargedBall));
-    const R th = static_cast<R>(theta), om = static_cast<R>(omega);
-    R s, c;
-    sincos_r(th, &s, &c);
-    const R x = s * k.r, y = c * k.r;
+    R f[4];
+    charged_ball_initial_sample<R>(seed, env, k.r, e.theta, e.omega, f);  // init_charged_ball_kernel
     e.on = true;
-    e.theta = th;
-    e.omega = om;
-    e.f = {x, y, om * y, -om * x};
+    e.f = {f[0], f[1], f[2], f[3]};
   }
 };
 
@@ -255,12 +236,12 @@ __global__ void __launch_bounds__(kBlock)
       const unsigned long long tg = r.t0 + static_cast<unsigned long long>(t);
       if (r.random_policy) {
         if (discrete) {
-          if (t == 0 || (tg & 127ull) == 0) Philox::generate(r.seed_action, env, static_cast<uint32_t>(tg >> 7), kPurposeRefRolloutAction, w);
+          if (t == 0 || (tg & 127ull) == 0) Philox::generate(r.seed_action, env, static_cast<uint32_t>(tg >> 7), kPurposeRolloutAction, w);
           const unsigned j = static_cast<unsigned>(tg >> 5) & 3u;
           const uint32_t word = j == 0 ? w[0] : (j == 1 ? w[1] : (j == 2 ? w[2] : w[3]));
           a.value = static_cast<float>((word >> (static_cast<unsigned>(tg) & 31u)) & 1u);
         } else {
-          if (t == 0 || (tg & 3ull) == 0) Philox::generate(r.seed_action, env, static_cast<uint32_t>(tg >> 2), kPurposeRefRolloutAction, w);
+          if (t == 0 || (tg & 3ull) == 0) Philox::generate(r.seed_action, env, static_cast<uint32_t>(tg >> 2), kPurposeRolloutAction, w);
           const unsigned j = static_cast<unsigned>(tg) & 3u;
           const uint32_t word = j == 0 ? w[0] : (j == 1 ? w[1] : (j == 2 ? w[2] : w[3]));
           a.value = fmaf(r.act_high - r.act_low, static_cast<float>(word >> 8) * (1.0f / 16777216.0f), r.act_low);
@@ -383,15 +364,10 @@ int cartpole_rollout_ref(R* state_io, int32_t* ep_step, R* ep_return, int32_t* e
   if (n < 0) return EMEI_ERR_BAD_SIZE;
   EMEI_CHECK_PTR(p);
   EMEI_CHECK_PTR(r);
-  if (p->variant < EMEI_CARTPOLE_BALANCING || p->variant > EMEI_IP_BOUNDARY_SWINGUP) return EMEI_ERR_BAD_VARIANT;
-  if (p->action_kind < EMEI_ACTION_DISCRETE_U8 || p->action_kind > EMEI_ACTION_CONTINUOUS_F64) return EMEI_ERR_BAD_ACTION_KIND;
-  if (p->freq_rate < 1 || !(p->dt > 0.0)) return EMEI_ERR_BAD_PARAM;
+  if (const int e = check_cartpole_params(*p)) return e;
   const bool ip = p->variant > EMEI_CARTPOLE_SWINGUP;
-  if (noise != nullptr) {
-    if (!ip) return EMEI_ERR_BAD_VARIANT;  // the noisy step exists for the MuJoCo-shell family only (mujoco_env.py:98-104)
-    for (int j = 0; j < 4; ++j)
-      if (!(noise->sigma[j] >= 0.0)) return EMEI_ERR_BAD_PARAM;
-  }
+  if (noise != nullptr && !ip) return EMEI_ERR_BAD_VARIANT;  // the noisy step exists for the MuJoCo-shell family only (mujoco_env.py:98-104)
+  if (const int e = check_noise_params(noise, 4)) return e;
   RefRolloutConsts rc;
   RefRolloutIO<R> io;
   const int code = make_ref_rollout<R>(r, p->action_kind, actions, rec_obs, rec_next, rec_act, rec_rew, rec_done, rec_timeout, ep_step, ep_return,
@@ -423,14 +399,8 @@ int i2p_rollout(R* state_io, int32_t* ep_step, R* ep_return, int32_t* ep_index, 
   EMEI_CHECK_PTR(r);
   EMEI_CHECK_PTR(init_mean);
   EMEI_CHECK_PTR(init_sigma);
-  if (p->variant < EMEI_I2P_REBOUND_BALANCING || p->variant > EMEI_I2P_BOUNDARY_SWINGUP) return EMEI_ERR_BAD_VARIANT;
-  if (p->action_kind < EMEI_ACTION_DISCRETE_U8 || p->action_kind > EMEI_ACTION_CONTINUOUS_F64) return EMEI_ERR_BAD_ACTION_KIND;
-  if (p->freq_rate < 1 || !(p->dt > 0.0) || !(p->mass_cart > 0.0) || !(p->mass_pole0 > 0.0) || !(p->mass_pole1 > 0.0) ||
-      !(p->length0 > 0.0) || !(p->length1 > 0.0))
-    return EMEI_ERR_BAD_PARAM;
-  if (noise != nullptr)
-    for (int j = 0; j < 6; ++j)
-      if (!(noise->sigma[j] >= 0.0)) return EMEI_ERR_BAD_PARAM;
+  if (const int e = check_i2p_params(*p)) return e;
+  if (const int e = check_noise_params(noise, 6)) return e;
   RefRolloutConsts rc;
   RefRolloutIO<R> io;
   const int code = make_ref_rollout<R>(r, p->action_kind, actions, rec_obs, rec_next, rec_act, rec_rew, rec_done, rec_timeout, ep_step, ep_return,
@@ -451,8 +421,7 @@ int charged_ball_rollout_ref(uint8_t* on_circle_io, R* circle_io, R* free_state_
   if (n < 0) return EMEI_ERR_BAD_SIZE;
   EMEI_CHECK_PTR(p);
   EMEI_CHECK_PTR(r);
-  if (p->action_kind < EMEI_ACTION_DISCRETE_U8 || p->action_kind > EMEI_ACTION_CONTINUOUS_F64) return EMEI_ERR_BAD_ACTION_KIND;
-  if (p->freq_rate < 1 || !(p->time_step > 0.0) || !(p->radius > 0.0) || !(p->mass_ball > 0.0)) return EMEI_ERR_BAD_PARAM;
+  if (const int e = check_charged_ball_params(*p)) return e;
   RefRolloutConsts rc;
   RefRolloutIO<R> io;
   const int code = make_ref_rollout<R>(r, p->action_kind, actions, rec_obs, rec_next, rec_act, rec_rew, rec_done, rec_timeout, ep_step, ep_return,

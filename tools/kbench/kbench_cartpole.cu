@@ -5,8 +5,6 @@
 #include <cstdio>
 #include <cstdlib>
 #include <vector>
-#include <array>
-#include <algorithm>
 #include "../../emei_b200/csrc/cartpole_tma.cuh"
 
 using namespace emei;
@@ -113,65 +111,6 @@ float time_graph(F launch, int K, cudaStream_t s, int reps = 5) {
   return best * 1e3f / K;  // us per launch
 }
 
-__global__ void spin_kernel(long long cycles) {
-  const long long t0 = clock64();
-  while (clock64() - t0 < cycles) {
-  }
-}
-
-// K plain stream launches queued behind a spinning kernel (no graph): what a caller of step() in a loop gets
-template <typename F>
-float time_stream(F launch, int K, cudaStream_t s, int reps = 5) {
-  for (int i = 0; i < 8; ++i) launch(i);
-  CK(cudaStreamSynchronize(s));
-  cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
-  float best = 1e30f;
-  for (int r = 0; r < reps; ++r) {
-    spin_kernel<<<1, 1, 0, s>>>(400000 + 30000ll * K);
-    CK(cudaEventRecord(e0, s));
-    for (int i = 0; i < K; ++i) launch(i);
-    CK(cudaEventRecord(e1, s)); CK(cudaStreamSynchronize(s));
-    float ms; cudaEventElapsedTime(&ms, e0, e1); if (ms < best) best = ms;
-  }
-  return best * 1e3f / K;
-}
-
-// shape variants of the shipped kernel: GROUPS consumer groups per CTA, BULK stores, CTAs per SM, ring budget
-template <int GROUPS, bool BULK, int GSZ = kBlock>
-void run_tma2(const char* name, Ring& R, uint32_t n, int K, cudaStream_t s, int ctas_per_sm, int budget_kb, int producer_group = 0, int prefetch = 0, int depth = 0) {
-  SKIP(name);
-  emei_cartpole_params p = {};
-  p.gravity = 9.8; p.mass_pole = 0.1; p.total_mass = 1.1; p.length = 0.5; p.pole_mass_length = 0.05; p.force_mag = 10.0;
-  p.x_threshold = 5.0; p.theta_threshold = 0.2; p.dt = 0.02; p.freq_rate = 4; p.variant = EMEI_CARTPOLE_SWINGUP;
-  p.action_kind = EMEI_ACTION_CONTINUOUS_F32;
-  CartPoleF32Consts k = make_cartpole_f32_consts(p);
-  const int64_t chunks = (n + 2 * GSZ - 1) / (2 * GSZ);
-  const int64_t cap = (int64_t)kNumSMs * ctas_per_sm;
-  const int grid = (int)(chunks < cap ? chunks : cap);
-  int n_slots; size_t smem;
-  tma_ring_shape(4, (chunks + grid - 1) / grid, &n_slots, &smem, GROUPS, BULK, budget_kb * 1024, GSZ);
-  const bool recycles = (chunks + grid - 1) / grid > n_slots;
-  if (BULK && recycles) { printf("%-52s skipped: BULK needs a ring that holds the CTA's whole share\n", name); return; }
-  double* stats; CK(cudaMalloc(&stats, 16)); CK(cudaMemset(stats, 0, 16));
-  const int ring = (int)R.in.size();
-  auto kern = cartpole_step_f32_tma_kernel<false, EMEI_ACTION_CONTINUOUS_F32, 4, false, GROUPS, BULK, GSZ>;
-  CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-  auto launch = [&](int i) {
-    int j = i % ring;
-    launch_pdl_smem(kern, grid, GROUPS * GSZ, smem, s, (const float4*)R.in[j], (float4*)R.out[j], (float4*)nullptr, (const void*)R.act[j], R.rew[j], R.done[j], stats, n, n_slots, 1 | (prefetch ? 2 : 0) | (producer_group << 8) | (depth << 16), k);
-  };
-  float us = time_graph(launch, K, s);
-  CK(cudaGetLastError());
-  const int reps20 = getenv("KBENCH_REPS") ? atoi(getenv("KBENCH_REPS")) : 9;  // 1: a single shot, like bench.py's timed region
-  float us20g = time_graph(launch, 20, s, reps20);
-  float us20s = time_stream(launch, 20, s, reps20);
-  CK(cudaGetLastError());
-  int occ = 0; cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, GROUPS * GSZ, smem);
-  printf("%-52s grid=%4d thr=%4d slots=%2d smem=%6zu occ=%d  graph K=%d: %6.2f us  %5.0f GB/s | K=20 graph %6.2f us, K=20 stream launches %6.2f us\n",
-         name, grid, GROUPS * GSZ, n_slots, smem, occ, K, us, 41.0 * n / us * 1e-3, us20g, us20s);
-  cudaFree(stats);
-}
-
 template <int FR>
 void run_tma(const char* name, Ring& R, uint32_t n, int K, cudaStream_t s, int slots_cap = 0) {
   SKIP(name);
@@ -184,6 +123,10 @@ void run_tma(const char* name, Ring& R, uint32_t n, int K, cudaStream_t s, int s
   const int grid = (int)(chunks < kNumSMs ? chunks : kNumSMs);
   int n_slots; size_t smem;
   tma_ring_shape(4, (chunks + grid - 1) / grid, &n_slots, &smem);
+  // the shipped flags (launch_cartpole_f32_tma): actions staged by TMA, L2 prefetch of the first `depth` chunks
+  const int64_t per_cta = (chunks + grid - 1) / grid;
+  const int depth = (int)(per_cta / 5 + 1 < 3 ? 3 : (per_cta / 5 + 1 > 8 ? 8 : per_cta / 5 + 1));
+  const int flags = 1 | 2 | (depth << 16);
   if (slots_cap && n_slots > slots_cap) { n_slots = slots_cap; smem = (size_t)n_slots * kChunk * 20 + 2 * n_slots * 8 + (kTmaThreads / 32) * 12 + 16; }
   double* stats; CK(cudaMalloc(&stats, 16)); CK(cudaMemset(stats, 0, 16));
   const int ring = (int)R.in.size();
@@ -191,7 +134,7 @@ void run_tma(const char* name, Ring& R, uint32_t n, int K, cudaStream_t s, int s
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
   auto launch = [&](int i) {
     int j = i % ring;
-    launch_pdl_smem(kern, grid, kTmaThreads, smem, s, (const float4*)R.in[j], (float4*)R.out[j], (float4*)nullptr, (const void*)R.act[j], R.rew[j], R.done[j], stats, n, n_slots, 1, k);
+    launch_pdl(kern, grid, kTmaThreads, smem, s, (const float4*)R.in[j], (float4*)R.out[j], (float4*)nullptr, (const void*)R.act[j], R.rew[j], R.done[j], stats, n, n_slots, flags, k);
   };
   float us = time_graph(launch, K, s);
   CK(cudaGetLastError());
@@ -242,79 +185,6 @@ void run_stream(const char* name, Ring& R, uint32_t n, int K, cudaStream_t s) {
   printf("%-44s grid=%5d  %7.2f us/launch  %6.1f Genv-steps/s  %6.0f GB/s (41 B/env)\n", name, grid, us, n / us * 1e-3, 41.0 * n / us * 1e-3);
 }
 
-#ifdef EMEI_TMA_TRACE
-// one steady-state launch's chunk pipeline: when each group's chunks landed and when their stores were issued
-void run_trace(Ring& R, uint32_t n, cudaStream_t s) {
-  emei_cartpole_params p = {};
-  p.gravity = 9.8; p.mass_pole = 0.1; p.total_mass = 1.1; p.length = 0.5; p.pole_mass_length = 0.05; p.force_mag = 10.0;
-  p.x_threshold = 5.0; p.theta_threshold = 0.2; p.dt = 0.02; p.freq_rate = 4; p.variant = EMEI_CARTPOLE_SWINGUP;
-  p.action_kind = EMEI_ACTION_CONTINUOUS_F32;
-  CartPoleF32Consts k = make_cartpole_f32_consts(p);
-  const int64_t chunks = (n + kChunk - 1) / kChunk;
-  const int grid = (int)(chunks < kNumSMs ? chunks : kNumSMs);
-  int n_slots; size_t smem;
-  tma_ring_shape(4, (chunks + grid - 1) / grid, &n_slots, &smem);
-  auto kern = cartpole_step_f32_tma_kernel<false, EMEI_ACTION_CONTINUOUS_F32, 4, false>;
-  CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-  double* stats; CK(cudaMalloc(&stats, 16)); CK(cudaMemset(stats, 0, 16));
-  const size_t words = (size_t)grid * 4 * 64;
-  unsigned long long* d_trace; CK(cudaMalloc(&d_trace, words * 8)); CK(cudaMemset(d_trace, 0, words * 8));
-  unsigned long long* null_ptr = nullptr;
-  const int ring = (int)R.in.size();
-  auto launch = [&](int i) {
-    int j = i % ring;
-    launch_pdl_smem(kern, grid, kTmaThreads, smem, s, (const float4*)R.in[j], (float4*)R.out[j], (float4*)nullptr, (const void*)R.act[j], R.rew[j], R.done[j], stats, n, n_slots, 1 | 2 | (kTmaProducerGroup << 8) | (3 << 16), k);
-  };
-  for (int i = 0; i < 40; ++i) launch(i);  // steady state, untraced
-  CK(cudaStreamSynchronize(s));
-  CK(cudaMemcpyToSymbol(g_tma_trace, &d_trace, sizeof(d_trace)));
-  for (int i = 40; i < 40 + (getenv("TRACE_LAUNCHES") ? atoi(getenv("TRACE_LAUNCHES")) : 3); ++i) launch(i);  // back-to-back launches overwrite each other's trace: the LAST one stays
-  CK(cudaStreamSynchronize(s));
-  CK(cudaMemcpyToSymbol(g_tma_trace, &null_ptr, sizeof(null_ptr)));
-  std::vector<unsigned long long> h(words);
-  CK(cudaMemcpy(h.data(), d_trace, words * 8, cudaMemcpyDeviceToHost));
-  unsigned long long t0 = ~0ull;
-  for (size_t i = 0; i < words; i += 64) if (h[i] && h[i] < t0) t0 = h[i];
-  printf("trace of one steady-state launch (ns after the earliest group passed griddepcontrol.wait); per group: start | chunk landed -> stores issued ... | done\n");
-  for (int cta : {0, 1, 73, 74, 123, 124, 146, 147}) {
-    for (int g = 0; g < 4; ++g) {
-      const unsigned long long* e = &h[((size_t)cta * 4 + g) * 64];
-      printf("cta %3d g%d  start %5lld |", cta, g, (long long)(e[0] - t0));
-      for (int m = 0; m < 6 && e[2 + 2 * m]; ++m) printf(" %5lld->%5lld", (long long)(e[2 + 2 * m] - t0), (long long)(e[3 + 2 * m] - t0));
-      printf(" | done %5lld\n", (long long)(e[1] - t0));
-    }
-  }
-  // distribution over all CTAs: when the first / last chunk landed, when the group finished
-  double first_land = 0, last_land = 0, done = 0; long long max_done = 0; int cnt = 0;
-  for (int cta = 0; cta < grid; ++cta) for (int g = 0; g < 4; ++g) {
-    const unsigned long long* e = &h[((size_t)cta * 4 + g) * 64];
-    if (!e[2]) continue;
-    int m = 0; while (m < 6 && e[2 + 2 * (m + 1)]) ++m;
-    first_land += (double)(e[2] - t0); last_land += (double)(e[2 + 2 * m] - t0); done += (double)(e[1] - t0);
-    if ((long long)(e[1] - t0) > max_done) max_done = (long long)(e[1] - t0);
-    ++cnt;
-  }
-  printf("mean over %d groups: first chunk landed %.0f ns, last chunk landed %.0f ns, group done %.0f ns; latest group done %lld ns\n", cnt, first_land / cnt, last_land / cnt, done / cnt, max_done);
-  // per CTA: SM id, chunks, first landing, last landing, done (max over groups), sorted by done
-  std::vector<std::array<long long, 6>> rows;
-  for (int cta = 0; cta < grid; ++cta) {
-    long long fl = 1LL << 60, ll = 0, dn = 0; int nch = 0;
-    for (int g = 0; g < 4; ++g) {
-      const unsigned long long* e = &h[((size_t)cta * 4 + g) * 64];
-      for (int m = 0; m < 6 && e[2 + 2 * m]; ++m) { long long v = (long long)(e[2 + 2 * m] - t0); if (v < fl) fl = v; if (v > ll) ll = v; ++nch; }
-      if ((long long)(e[1] - t0) > dn) dn = (long long)(e[1] - t0);
-    }
-    rows.push_back({dn, (long long)cta, (long long)h[((size_t)cta * 4) * 64 + 63], (long long)nch, fl, ll});
-  }
-  std::sort(rows.begin(), rows.end());
-  printf("per CTA sorted by completion: done_ns cta smid chunks first_landed last_landed\n");
-  for (size_t i = 0; i < rows.size(); ++i)
-    if (i < 6 || i + 24 >= rows.size() || i % 16 == 0)
-      printf("  %6lld  cta %3lld  sm %3lld  chunks %2lld  first %5lld  last %5lld\n", rows[i][0], rows[i][1], rows[i][2], rows[i][3], rows[i][4], rows[i][5]);
-  cudaFree(stats); cudaFree(d_trace);
-}
-#endif
-
 int main(int argc, char** argv) {
   const uint32_t n = argc > 1 ? (uint32_t)atol(argv[1]) : (1u << 20);
   const int ring = argc > 2 ? atoi(argv[2]) : 8;
@@ -335,10 +205,6 @@ int main(int argc, char** argv) {
     R.in.push_back(a); R.out.push_back(b); R.act.push_back(c); R.rew.push_back(d); R.done.push_back(e);
   }
   printf("n=%u ring=%d K=%d\n", n, ring, K);
-#ifdef EMEI_TMA_TRACE
-  run_trace(R, n, s);
-  return 0;
-#endif
   run_stream<8, true>("stream minb8 pdl", R, n, K, s);
   run_compute<4, 4, true>("compute-only scalar fr4 minb4 sincos/sub-step", R, n, K, s);
   run_compute<4, 4, false>("compute-only scalar fr4 minb4 angle-addition", R, n, K, s);
@@ -346,43 +212,6 @@ int main(int argc, char** argv) {
   run_compute2<4, 4, false>("compute-only packed fr4 minb4 angle-addition", R, n, K, s);
   run_tma<4>("TMA packed fr4 (shipped)", R, n, K, s);
   run_tma<4>("TMA packed fr4 slots<=8", R, n, K, s, 8);
-  // ---- round 2: shape variants (GROUPS per CTA, bulk stores, CTAs per SM, ring budget in KB)
-  run_tma2<4, false>("r2 G4 direct stores, producer = group 0", R, n, K, s, 1, 208, 0);
-  run_tma2<4, false>("r2 G4 direct stores, producer = group 1", R, n, K, s, 1, 208, 1);
-  run_tma2<4, false>("r2 G4 direct stores, producer = group 2", R, n, K, s, 1, 208, 2);
-  run_tma2<4, false>("r2 G4 direct stores, producer = group 3", R, n, K, s, 1, 208, 3);
-  run_tma2<4, false>("r2 G4 producer 3 + L2 prefetch before the grid dependency (shipped)", R, n, K, s, 1, 208, 3, 1);
-  run_tma2<2, false>("r2 G2 half-SM 10 slots + L2 prefetch", R, n, K, s, 1, 104, 1, 1);
-  run_tma2<2, false>("r2 G2 2 CTAs/SM 7 slots + L2 prefetch", R, n, K, s, 2, 104, 1, 1);
-  run_tma2<2, false>("r3 G2 2 CTAs/SM 8 slots + L2 prefetch, producer g0", R, n, K, s, 2, 104, 0, 1);
-  run_tma2<2, false>("r3 G2 2 CTAs/SM + L2 prefetch depth 2", R, n, K, s, 2, 104, 1, 1, 2);
-  run_tma2<2, false>("r3 G2 2 CTAs/SM + L2 prefetch depth 4", R, n, K, s, 2, 104, 1, 1, 4);
-  run_tma2<1, false>("r3 G1 4 CTAs/SM 4 slots + L2 prefetch", R, n, K, s, 4, 48, 0, 1);
-  run_tma2<1, false>("r3 G1 4 CTAs/SM 4 slots, no prefetch", R, n, K, s, 4, 48, 0, 0);
-  run_tma2<1, false>("r3 G1 3 CTAs/SM 5 slots + L2 prefetch", R, n, K, s, 3, 64, 0, 1);
-  run_tma2<8, false, 128>("r5 G8 x 128 threads, 256-env chunks, prefetch depth 6", R, n, K, s, 1, 208, 7, 1, 6);
-  run_tma2<8, false, 128>("r5 G8 x 128 threads, 256-env chunks, prefetch depth 8", R, n, K, s, 1, 208, 7, 1, 8);
-  run_tma2<8, false, 128>("r5 G8 x 128 threads, 256-env chunks, prefetch depth 4", R, n, K, s, 1, 208, 7, 1, 4);
-  run_tma2<8, false, 128>("r5 G8 x 128 threads, 256-env chunks, no prefetch", R, n, K, s, 1, 208, 7, 0, 0);
-  run_tma2<4, false>("r5 G4 + L2 prefetch depth 3 (shipped)", R, n, K, s, 1, 208, 3, 1, 3);
-  run_tma2<4, false>("r4 G4 + L2 prefetch depth 1", R, n, K, s, 1, 208, 3, 1, 1);
-  run_tma2<4, false>("r4 G4 + L2 prefetch depth 3", R, n, K, s, 1, 208, 3, 1, 3);
-  run_tma2<4, false>("r4 G4 + L2 prefetch depth 4", R, n, K, s, 1, 208, 3, 1, 4);
-  run_tma2<4, false>("r4 G4 + L2 prefetch depth 5", R, n, K, s, 1, 208, 3, 1, 5);
-  run_tma2<4, false>("r4 G4 + L2 prefetch depth 6", R, n, K, s, 1, 208, 3, 1, 6);
-  run_tma2<4, false>("r4 G4 + L2 prefetch depth 8", R, n, K, s, 1, 208, 3, 1, 8);
-  run_tma2<4, false>("r4 G4 no prefetch", R, n, K, s, 1, 208, 3, 0, 0);
-  run_tma2<2, false>("r4 G2 2 CTAs/SM + L2 prefetch depth 1", R, n, K, s, 2, 104, 1, 1, 1);
-  run_tma2<2, false>("r4 G2 2 CTAs/SM + L2 prefetch depth 2", R, n, K, s, 2, 104, 1, 1, 2);
-  run_tma2<2, false>("r4 G2 2 CTAs/SM + L2 prefetch depth 3", R, n, K, s, 2, 104, 1, 1, 3);
-  run_tma2<2, false>("r4 G2 2 CTAs/SM no prefetch", R, n, K, s, 2, 104, 1, 0, 0);
-  run_tma2<4, false>("r3 G4 + L2 prefetch depth 2", R, n, K, s, 1, 208, 3, 1, 2);
-  run_tma2<4, false>("r3 G4 + L2 prefetch depth 4", R, n, K, s, 1, 208, 3, 1, 4);
-  run_tma2<4, true>("r2 G4 BULK stores", R, n, K, s, 1, 216);
-  run_tma2<2, false>("r2 G2 half-SM, 1 CTA/SM/kernel, 10 slots", R, n, K, s, 1, 104);
-  run_tma2<2, false>("r2 G2 half-SM, 1 CTA/SM/kernel, 8 slots", R, n, K, s, 1, 84);
-  run_tma2<2, false>("r2 G2 2 CTAs/SM, 7 slots each", R, n, K, s, 2, 104);
-  run_tma2<2, true>("r2 G2 2 CTAs/SM, 7 slots each, BULK", R, n, K, s, 2, 108);
   run_tma<0>("TMA packed fr-runtime", R, n, K, s);
   run_tma<1>("TMA packed fr1", R, n, K, s);
   return 0;
