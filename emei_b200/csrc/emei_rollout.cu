@@ -1,52 +1,7 @@
 // extern "C" entry points of the fused float32 rollouts (rollout_f32.cuh).
 #include "rollout_f32.cuh"
 
-namespace {
-
 using namespace emei;
-
-// validation + conversion shared by the two entry points; returns EMEI_OK or an error code
-int make_rollout(const emei_rollout_params* r, const void* actions, float* rec_observations,
-                 float* rec_next_observations, void* rec_actions, float* rec_rewards, uint8_t* rec_dones,
-                 uint8_t* rec_timeouts, int32_t* ep_step, float* ep_return, int32_t* ep_index, double* stats,
-                 RolloutConsts& rc, RolloutIO& io) {
-  EMEI_CHECK_PTR(ep_step);
-  EMEI_CHECK_PTR(ep_return);
-  EMEI_CHECK_PTR(ep_index);
-  if (!r->random_policy) EMEI_CHECK_PTR(actions);
-  if (rec_observations != nullptr) {  // records are all-or-nothing
-    EMEI_CHECK_PTR(rec_next_observations);
-    EMEI_CHECK_PTR(rec_actions);
-    EMEI_CHECK_PTR(rec_rewards);
-    EMEI_CHECK_PTR(rec_dones);
-    EMEI_CHECK_PTR(rec_timeouts);
-    EMEI_CHECK_ALIGN16(rec_observations);
-    EMEI_CHECK_ALIGN16(rec_next_observations);
-  }
-  rc.horizon = r->horizon;
-  rc.max_episode_steps = r->max_episode_steps;
-  rc.auto_reset = r->auto_reset;
-  rc.random_policy = r->random_policy;
-  rc.init_kind = r->init_kind;
-  rc.init_pi_column = r->init_pi_column;
-  rc.seed_reset = r->seed_reset;
-  rc.seed_action = r->seed_action;
-  rc.env_offset = r->env_offset;
-  rc.t0 = r->t0;
-  rc.init_low = r->init_low;
-  rc.init_high = r->init_high;
-  for (int j = 0; j < 4; ++j) {
-    rc.mean[j] = r->init_mean[j];
-    rc.sigma[j] = r->init_sigma[j];
-  }
-  rc.act_low = static_cast<float>(r->action_low);
-  rc.act_high = static_cast<float>(r->action_high);
-  io = {ep_step, ep_return, ep_index, actions, reinterpret_cast<float4*>(rec_observations),
-        reinterpret_cast<float4*>(rec_next_observations), rec_actions, rec_rewards, rec_dones, rec_timeouts, stats};
-  return EMEI_OK;
-}
-
-}  // namespace
 
 extern "C" int emei_cartpole_rollout_f32(float* state_io, int32_t* episode_step_io, float* episode_return_io,
                                          int32_t* episode_index_io, const void* actions, float* rec_observations,
@@ -62,11 +17,10 @@ extern "C" int emei_cartpole_rollout_f32(float* state_io, int32_t* episode_step_
   if (n == 0 || r->horizon == 0) return EMEI_OK;
   EMEI_CHECK_PTR(state_io);
   EMEI_CHECK_ALIGN16(state_io);
-  RolloutConsts rc;
-  RolloutIO io;
-  const int rcode = make_rollout(r, actions, rec_observations, rec_next_observations, rec_actions, rec_rewards, rec_dones,
-                                 rec_timeouts, episode_step_io, episode_return_io, episode_index_io, stats, rc, io);
-  if (rcode != EMEI_OK) return rcode;
+  const RolloutIO<float> io = {episode_step_io, episode_return_io, episode_index_io, actions, rec_observations, rec_next_observations,
+                               rec_actions, rec_rewards, rec_dones, rec_timeouts, stats};
+  RolloutConsts<4> rc;
+  if (const int e = make_rollout(r, io, true, nullptr, nullptr, rc)) return e;
   const CartPoleF32Consts k = make_cartpole_f32_consts(*p);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const bool ip = p->variant > EMEI_CARTPOLE_SWINGUP;
@@ -101,11 +55,10 @@ extern "C" int emei_charged_ball_rollout_f32(uint8_t* on_circle_io, float* circl
   EMEI_CHECK_PTR(free_state_io);
   EMEI_CHECK_ALIGN16(circle_io);
   EMEI_CHECK_ALIGN16(free_state_io);
-  RolloutConsts rc;
-  RolloutIO io;
-  const int rcode = make_rollout(r, actions, rec_observations, rec_next_observations, rec_actions, rec_rewards, rec_dones,
-                                 rec_timeouts, episode_step_io, episode_return_io, episode_index_io, stats, rc, io);
-  if (rcode != EMEI_OK) return rcode;
+  const RolloutIO<float> io = {episode_step_io, episode_return_io, episode_index_io, actions, rec_observations, rec_next_observations,
+                               rec_actions, rec_rewards, rec_dones, rec_timeouts, stats};
+  RolloutConsts<4> rc;
+  if (const int e = make_rollout(r, io, true, nullptr, nullptr, rc)) return e;
   rc.init_kind = 2;  // charged_ball.py:84-94 is the only reset sampler of this family
   launch_charged_ball_rollout(p->action_kind, on_circle_io, circle_io, free_state_io, io, n, make_cb_f32_consts(*p), rc,
                               static_cast<cudaStream_t>(stream));

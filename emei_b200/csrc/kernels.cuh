@@ -89,6 +89,17 @@ __device__ __forceinline__ void philox_normal_pair(uint64_t seed, uint64_t env, 
   sincospi(2.0 * u2, &sn, &cs);
 }
 
+// Columns 2 pr, 2 pr + 1 of a Gaussian initial state (mujoco_env.py:137-140): mean + sigma * N(0,1), the arithmetic of
+// init_gaussian_kernel.  The resets of both rollout kernels.
+template <typename T>
+__device__ __forceinline__ void gaussian_initial_pair(const double* mean, const double* sigma, uint64_t seed, uint64_t env, int pr, T& v0,
+                                                      T& v1) {
+  double rad, cs, sn;
+  philox_normal_pair(seed, env, static_cast<uint32_t>(pr), kPurposeGaussian, rad, cs, sn);
+  v0 = static_cast<T>(__dadd_rn(mean[2 * pr], __dmul_rn(sigma[2 * pr], __dmul_rn(rad, cs))));
+  v1 = static_cast<T>(__dadd_rn(mean[2 * pr + 1], __dmul_rn(sigma[2 * pr + 1], __dmul_rn(rad, sn))));
+}
+
 struct NoiseConsts {
   double sigma[6];
   unsigned long long seed, env_offset, substep0;  // substep0 = step * freq_rate: global index of this call's first sub-step

@@ -18,16 +18,9 @@
 // The kernel is written once over a `Dyn` policy (the env family): Dyn::Buffers (state arrays), Dyn::Regs
 // (one env in registers), load/store/observation/step/reset.
 #pragma once
-#include "kernels.cuh"
+#include "rollout.cuh"
 
 namespace emei {
-
-struct RolloutConsts {
-  int horizon, max_episode_steps, auto_reset, random_policy, init_kind /*0 uniform, 1 gaussian, 2 charged ball*/, init_pi_column;
-  unsigned long long seed_reset, seed_action, env_offset, t0;
-  double init_low, init_high, mean[4], sigma[4];
-  float act_low, act_high;
-};
 
 // In-rollout reset sample of one env row.
 // Uniform family (cartpole.py:131-132,153-156: U(low, high) per coordinate, + pi on the swing-up angle): the lean
@@ -37,7 +30,7 @@ struct RolloutConsts {
 // (two blocks, four double conversions) cost ~360 warp instructions per event, this one ~110
 // (mirror: oracle/rollout_oracle.py reset_sample_uniform).
 // Gaussian family (mujoco_env.py:137-140): the arithmetic of init_gaussian_kernel (kernels.cuh).
-static __device__ __noinline__ float4 rollout_init_state(const RolloutConsts& r, unsigned long long env, unsigned long long seed) {
+static __device__ __noinline__ float4 rollout_init_state(const RolloutConsts<4>& r, unsigned long long env, unsigned long long seed) {
   float v[4];
   if (r.init_kind == 0) {
     uint32_t w[4];
@@ -50,12 +43,7 @@ static __device__ __noinline__ float4 rollout_init_state(const RolloutConsts& r,
     }
   } else {
 #pragma unroll
-    for (int pr = 0; pr < 2; ++pr) {
-      double rad, cs, sn;
-      philox_normal_pair(seed, env, static_cast<uint32_t>(pr), kPurposeGaussian, rad, cs, sn);
-      v[2 * pr] = static_cast<float>(__dadd_rn(r.mean[2 * pr], __dmul_rn(r.sigma[2 * pr], __dmul_rn(rad, cs))));
-      v[2 * pr + 1] = static_cast<float>(__dadd_rn(r.mean[2 * pr + 1], __dmul_rn(r.sigma[2 * pr + 1], __dmul_rn(rad, sn))));
-    }
+    for (int pr = 0; pr < 2; ++pr) gaussian_initial_pair<float>(r.mean, r.sigma, seed, env, pr, v[2 * pr], v[2 * pr + 1]);
   }
   return make_float4(v[0], v[1], v[2], v[3]);
 }
@@ -167,7 +155,7 @@ struct CartPoleDyn {
     terminated[0] = !nd_a;
     terminated[1] = !nd_b;
   }
-  __device__ __forceinline__ static void reset(Regs& e, const RolloutConsts& r, const Consts&, unsigned long long env, unsigned long long seed) {
+  __device__ __forceinline__ static void reset(Regs& e, const RolloutConsts<4>& r, const Consts&, unsigned long long env, unsigned long long seed) {
     e.y = rollout_init_state(r, env, seed);
   }
   __device__ __forceinline__ static float4 pack(const Regs& e) { return e.y; }
@@ -212,7 +200,7 @@ struct ChargedBallDyn {
     terminated[0] = false;  // charged_ball.py:110-111
     next_obs[0] = e[0].f;
   }
-  __device__ __forceinline__ static void reset(Regs& e, const RolloutConsts&, const Consts& k, unsigned long long env, unsigned long long seed) {
+  __device__ __forceinline__ static void reset(Regs& e, const RolloutConsts<4>&, const Consts& k, unsigned long long env, unsigned long long seed) {
     e = rollout_init_charged_ball(k.r, env, seed);
   }
   __device__ __forceinline__ static float4 pack(const Regs& e) { return e.f; }  // unused (kSpareReset = false)
@@ -222,26 +210,12 @@ struct ChargedBallDyn {
 // ------------------------------------------------------------------------------------------------
 // the kernel
 // ------------------------------------------------------------------------------------------------
-struct RolloutIO {  // everything that is not the env family's own state
-  int32_t* ep_step;
-  float* ep_return;
-  int32_t* ep_index;
-  const void* actions;
-  float4* rec_obs;
-  float4* rec_next;
-  void* rec_act;
-  float* rec_rew;
-  uint8_t* rec_done;
-  uint8_t* rec_timeout;
-  double* stats;
-};
-
 // One thread owns E = Dyn::kEnvsPerThread envs for the whole horizon: envs i0 + e * kBlock of its CTA's block of
 // E * kBlock envs (every access stays coalesced per e).
 template <class Dyn, bool RECORD>
 __global__ void __launch_bounds__(kBlock, Dyn::kMinBlocks)
-    rollout_f32_kernel(const typename Dyn::Buffers b, const RolloutIO io, uint32_t n, const typename Dyn::Consts k,
-                       const RolloutConsts r) {
+    rollout_f32_kernel(const typename Dyn::Buffers b, const RolloutIO<float> io, uint32_t n, const typename Dyn::Consts k,
+                       const RolloutConsts<4> r) {
   using ActT = typename Dyn::ActT;
   constexpr int E = Dyn::kEnvsPerThread;
   const uint32_t i0 = blockIdx.x * (kBlock * E) + threadIdx.x;
@@ -302,8 +276,7 @@ __global__ void __launch_bounds__(kBlock, Dyn::kMinBlocks)
           for (int e = 0; e < E; ++e) {
             if (live[e] && !have_spare[e]) {
               typename Dyn::Regs nxt = ev[e];
-              Dyn::reset(nxt, r, k, r.env_offset + idx[e],
-                         r.seed_reset + static_cast<unsigned long long>(ep_idx[e] + 1) * 0xD1B54A32D192ED03ull);
+              Dyn::reset(nxt, r, k, r.env_offset + idx[e], reset_seed(r.seed_reset, ep_idx[e] + 1));
               s_spare[e][threadIdx.x] = Dyn::pack(nxt);
               have_spare[e] = true;
             }
@@ -318,7 +291,7 @@ __global__ void __launch_bounds__(kBlock, Dyn::kMinBlocks)
           // block lasts 128 steps: block tg >> 7, word (tg >> 5) & 3, bit tg & 31), Box one 32-bit word per step
           // (block tg >> 2, word tg & 3, top 24 bits -> [low, high)).  The refresh tests depend on the step number
           // only, so they are uniform branches; between refreshes a Discrete step costs a mask and a shift of the
-          // current word.
+          // current word.  rollout_ref_kernel keeps its own copy of this stream (DESIGN.md 4.6).
           if constexpr (Dyn::kDiscrete) {
             if (t == 0 || (tl & 31u) == 0) {
               if (t == 0 || (tl & 127u) == 0)
@@ -342,7 +315,7 @@ __global__ void __launch_bounds__(kBlock, Dyn::kMinBlocks)
         if constexpr (RECORD) {
           if (live[e]) {
             const size_t rec = static_cast<size_t>(t) * n + idx[e];
-            io.rec_obs[rec] = Dyn::observation(ev[e]);
+            reinterpret_cast<float4*>(io.rec_obs)[rec] = Dyn::observation(ev[e]);
             act_out[rec] = static_cast<ActT>(a[e]);
           }
         }
@@ -362,7 +335,7 @@ __global__ void __launch_bounds__(kBlock, Dyn::kMinBlocks)
         const bool done = terminated[e] || truncated;
         if constexpr (RECORD) {
           const size_t rec = static_cast<size_t>(t) * n + idx[e];
-          io.rec_next[rec] = next_obs[e];
+          reinterpret_cast<float4*>(io.rec_next)[rec] = next_obs[e];
           io.rec_rew[rec] = rew[e];
           io.rec_done[rec] = done ? 1 : 0;
           io.rec_timeout[rec] = truncated ? 1 : 0;
@@ -380,7 +353,7 @@ __global__ void __launch_bounds__(kBlock, Dyn::kMinBlocks)
               Dyn::unpack(ev[e], s_spare[e][threadIdx.x]);
               have_spare[e] = false;
             } else {
-              Dyn::reset(ev[e], r, k, r.env_offset + idx[e], r.seed_reset + static_cast<unsigned long long>(ep_idx[e]) * 0xD1B54A32D192ED03ull);
+              Dyn::reset(ev[e], r, k, r.env_offset + idx[e], reset_seed(r.seed_reset, ep_idx[e]));
             }
             ep_step[e] = 0;
             ep_ret[e] = 0.f;
@@ -410,8 +383,8 @@ __global__ void __launch_bounds__(kBlock, Dyn::kMinBlocks)
 }
 
 template <class Dyn>
-inline void launch_rollout(const typename Dyn::Buffers& b, const RolloutIO& io, int64_t n, const typename Dyn::Consts& k,
-                           const RolloutConsts& r, cudaStream_t s) {
+inline void launch_rollout(const typename Dyn::Buffers& b, const RolloutIO<float>& io, int64_t n, const typename Dyn::Consts& k,
+                           const RolloutConsts<4>& r, cudaStream_t s) {
   const int grid = grid_for(n, kBlock * Dyn::kEnvsPerThread);
   if (io.rec_obs != nullptr)
     launch_pdl(rollout_f32_kernel<Dyn, true>, grid, kBlock, s, b, io, static_cast<uint32_t>(n), k, r);
@@ -420,8 +393,8 @@ inline void launch_rollout(const typename Dyn::Buffers& b, const RolloutIO& io, 
 }
 
 template <bool IP, int FR>
-inline void launch_cartpole_rollout(int ak, float* state, const RolloutIO& io, int64_t n, const CartPoleF32Consts& k,
-                                    const RolloutConsts& r, cudaStream_t s) {
+inline void launch_cartpole_rollout(int ak, float* state, const RolloutIO<float>& io, int64_t n, const CartPoleF32Consts& k,
+                                    const RolloutConsts<4>& r, cudaStream_t s) {
   float4* st = reinterpret_cast<float4*>(state);
   switch (ak) {
 #define EMEI_AK(A)                                                           \
@@ -438,8 +411,8 @@ inline void launch_cartpole_rollout(int ak, float* state, const RolloutIO& io, i
   }
 }
 
-inline void launch_charged_ball_rollout(int ak, uint8_t* on_circle, float* circle, float* free_state, const RolloutIO& io,
-                                        int64_t n, const ChargedBallF32Consts& k, const RolloutConsts& r, cudaStream_t s) {
+inline void launch_charged_ball_rollout(int ak, uint8_t* on_circle, float* circle, float* free_state, const RolloutIO<float>& io,
+                                        int64_t n, const ChargedBallF32Consts& k, const RolloutConsts<4>& r, cudaStream_t s) {
   switch (ak) {
 #define EMEI_AK(A)                                                                                                       \
   case A: {                                                                                                              \

@@ -13,31 +13,9 @@
 // `horizon` step calls bit for bit.  In-kernel resets use the arithmetic of the emei_init_* kernels in this precision,
 // keyed by (seed_reset + episode_index * 0xD1B54A32D192ED03, global env id): host mirror = oracle/philox.py init_*.
 #pragma once
-#include "kernels.cuh"
+#include "rollout.cuh"
 
 namespace emei {
-
-struct RefRolloutConsts {
-  int horizon, max_episode_steps, auto_reset, random_policy, init_pi_column, action_kind;
-  unsigned long long seed_reset, seed_action, env_offset, t0;
-  double init_low, init_high, mean[6], sigma[6];
-  float act_low, act_high;
-};
-
-template <typename R>
-struct RefRolloutIO {
-  int32_t* ep_step;
-  R* ep_return;
-  int32_t* ep_index;
-  const void* actions;
-  R* rec_obs;
-  R* rec_next;
-  void* rec_act;
-  R* rec_rew;
-  uint8_t* rec_done;
-  uint8_t* rec_timeout;
-  double* stats;
-};
 
 // action value of env i at step t: teacher-forced array [T, n] in `kind`, or the counter-based random policy of
 // rollout_f32.cuh (Discrete(2): one bit per step; Box: 24 bits -> [low, high), a float32 like action_space.sample())
@@ -100,24 +78,16 @@ struct RefCartPole {
     terminated = !notdone;
     o[0] = obs.x, o[1] = obs.y, o[2] = obs.z, o[3] = obs.w;
   }
-  __device__ static void reset(Regs& e, const RefRolloutConsts& r, const Consts&, unsigned long long env, unsigned long long seed) {
+  __device__ static void reset(Regs& e, const RolloutConsts<6>& r, const Consts&, unsigned long long env, unsigned long long seed) {
     R v[4];
     if constexpr (!IP) {  // init_uniform_kernel
 #pragma unroll
       for (int c = 0; c < 4; ++c) v[c] = static_cast<R>(uniform_initial_sample(seed, env, c, r.init_low, r.init_high, r.init_pi_column));
-    } else {  // init_gaussian_kernel (mujoco_env.py:137-140)
+    } else {  // init_gaussian_kernel
 #pragma unroll
-      for (int pr = 0; pr < 2; ++pr) gaussian_pair<R>(r, env, seed, pr, v[2 * pr], v[2 * pr + 1]);
+      for (int pr = 0; pr < 2; ++pr) gaussian_initial_pair<R>(r.mean, r.sigma, seed, env, pr, v[2 * pr], v[2 * pr + 1]);
     }
     e.y = {v[0], v[1], v[2], v[3]};
-  }
-  template <typename T>
-  __device__ __forceinline__ static void gaussian_pair(const RefRolloutConsts& r, unsigned long long env, unsigned long long seed, int pr,
-                                                       T& v0, T& v1) {
-    double rad, cs, sn;
-    philox_normal_pair(seed, env, static_cast<uint32_t>(pr), kPurposeGaussian, rad, cs, sn);
-    v0 = static_cast<T>(__dadd_rn(r.mean[2 * pr], __dmul_rn(r.sigma[2 * pr], __dmul_rn(rad, cs))));
-    v1 = static_cast<T>(__dadd_rn(r.mean[2 * pr + 1], __dmul_rn(r.sigma[2 * pr + 1], __dmul_rn(rad, sn))));
   }
 };
 
@@ -149,9 +119,9 @@ struct RefI2P {
     i2p_env_step<R>(e.y, drv, k, z, env, substep0, o, rew, notdone);
     terminated = !notdone;
   }
-  __device__ static void reset(Regs& e, const RefRolloutConsts& r, const Consts&, unsigned long long env, unsigned long long seed) {
+  __device__ static void reset(Regs& e, const RolloutConsts<6>& r, const Consts&, unsigned long long env, unsigned long long seed) {
 #pragma unroll
-    for (int pr = 0; pr < 3; ++pr) RefCartPole<R, true>::template gaussian_pair<R>(r, env, seed, pr, e.y[2 * pr], e.y[2 * pr + 1]);
+    for (int pr = 0; pr < 3; ++pr) gaussian_initial_pair<R>(r.mean, r.sigma, seed, env, pr, e.y[2 * pr], e.y[2 * pr + 1]);
   }
 };
 
@@ -200,7 +170,7 @@ struct RefChargedBall {
     terminated = false;  // charged_ball.py:110-111
     o[0] = e.f.x, o[1] = e.f.y, o[2] = e.f.z, o[3] = e.f.w;
   }
-  __device__ static void reset(Regs& e, const RefRolloutConsts&, const Consts& k, unsigned long long env, unsigned long long seed) {
+  __device__ static void reset(Regs& e, const RolloutConsts<6>&, const Consts& k, unsigned long long env, unsigned long long seed) {
     R f[4];
     charged_ball_initial_sample<R>(seed, env, k.r, e.theta, e.omega, f);  // init_charged_ball_kernel
     e.on = true;
@@ -213,8 +183,8 @@ struct RefChargedBall {
 // ------------------------------------------------------------------------------------------------
 template <class Fam>
 __global__ void __launch_bounds__(kBlock)
-    rollout_ref_kernel(const typename Fam::Buffers b, const RefRolloutIO<typename Fam::Real> io, int64_t n, const typename Fam::Consts k,
-                       const RefRolloutConsts r, const NoiseConsts z, int freq_rate) {
+    rollout_ref_kernel(const typename Fam::Buffers b, const RolloutIO<typename Fam::Real> io, int64_t n, const typename Fam::Consts k,
+                       const RolloutConsts<6> r, const NoiseConsts z, int freq_rate) {
   using R = typename Fam::Real;
   constexpr int D = Fam::kObs;
   const int64_t i = static_cast<int64_t>(blockIdx.x) * kBlock + threadIdx.x;
@@ -226,7 +196,7 @@ __global__ void __launch_bounds__(kBlock)
     int ep_step = io.ep_step[i], ep_idx = io.ep_index[i];
     R ep_ret = io.ep_return[i];
     const unsigned long long env = r.env_offset + static_cast<unsigned long long>(i);
-    const bool discrete = r.action_kind <= EMEI_ACTION_DISCRETE_I64;
+    const bool discrete = k.action_kind <= EMEI_ACTION_DISCRETE_I64;
     uint32_t w[4] = {0u, 0u, 0u, 0u};
     for (int t = 0; t < r.horizon; ++t) {
       // ---- policy
@@ -234,7 +204,7 @@ __global__ void __launch_bounds__(kBlock)
       a.value = 0.f;
       a.index = -1;
       const unsigned long long tg = r.t0 + static_cast<unsigned long long>(t);
-      if (r.random_policy) {
+      if (r.random_policy) {  // the stream of rollout_f32_kernel; a copy of its own (DESIGN.md 4.6)
         if (discrete) {
           if (t == 0 || (tg & 127ull) == 0) Philox::generate(r.seed_action, env, static_cast<uint32_t>(tg >> 7), kPurposeRolloutAction, w);
           const unsigned j = static_cast<unsigned>(tg >> 5) & 3u;
@@ -255,13 +225,13 @@ __global__ void __launch_bounds__(kBlock)
         Fam::observation(e, k, o);
 #pragma unroll
         for (int c = 0; c < D; ++c) io.rec_obs[rec * D + c] = o[c];
-        ref_store_action(io.rec_act, rec, r.action_kind, io.actions, a.index, a.value);
+        ref_store_action(io.rec_act, rec, k.action_kind, io.actions, a.index, a.value);
       }
       // ---- dynamics + reward + terminal: the step entry point's device function
       R rew, o[D];
       bool terminated;
       // noise: z.substep0 holds the env-step counter of this call's first step (emei_noise_params.step)
-      Fam::step(e, Fam::drive(k, io.actions, a, r.action_kind), k, z, env,
+      Fam::step(e, Fam::drive(k, io.actions, a, k.action_kind), k, z, env,
                 (z.substep0 + static_cast<unsigned long long>(t)) * static_cast<unsigned long long>(freq_rate), rew, terminated, o);
       // ---- TimeLimit + bookkeeping (zoo/util.py:58-73; gym TimeLimit: truncated = elapsed >= max)
       ep_step += 1;
@@ -283,7 +253,7 @@ __global__ void __launch_bounds__(kBlock)
         fin_ret += static_cast<double>(ep_ret);
         fin_len += static_cast<unsigned>(ep_step);
         ep_idx += 1;
-        Fam::reset(e, r, k, env, r.seed_reset + static_cast<unsigned long long>(ep_idx) * 0xD1B54A32D192ED03ull);
+        Fam::reset(e, r, k, env, reset_seed(r.seed_reset, ep_idx));
         ep_step = 0;
         ep_ret = R(0);
       }
@@ -310,50 +280,9 @@ __global__ void __launch_bounds__(kBlock)
   }
 }
 
-// validation + conversion shared by the entry points
-template <typename R>
-inline int make_ref_rollout(const emei_rollout_params* r, int action_kind, const void* actions, R* rec_observations, R* rec_next_observations,
-                            void* rec_actions, R* rec_rewards, uint8_t* rec_dones, uint8_t* rec_timeouts, int32_t* ep_step, R* ep_return,
-                            int32_t* ep_index, double* stats, const double* mean, const double* sigma, int dim, RefRolloutConsts& rc,
-                            RefRolloutIO<R>& io) {
-  EMEI_CHECK_PTR(r);
-  EMEI_CHECK_PTR(ep_step);
-  EMEI_CHECK_PTR(ep_return);
-  EMEI_CHECK_PTR(ep_index);
-  if (r->horizon < 0) return EMEI_ERR_BAD_PARAM;
-  if (!r->random_policy) EMEI_CHECK_PTR(actions);
-  if (rec_observations != nullptr) {  // records are all-or-nothing
-    EMEI_CHECK_PTR(rec_next_observations);
-    EMEI_CHECK_PTR(rec_actions);
-    EMEI_CHECK_PTR(rec_rewards);
-    EMEI_CHECK_PTR(rec_dones);
-    EMEI_CHECK_PTR(rec_timeouts);
-  }
-  rc.horizon = r->horizon;
-  rc.max_episode_steps = r->max_episode_steps;
-  rc.auto_reset = r->auto_reset;
-  rc.random_policy = r->random_policy;
-  rc.init_pi_column = r->init_pi_column;
-  rc.action_kind = action_kind;
-  rc.seed_reset = r->seed_reset;
-  rc.seed_action = r->seed_action;
-  rc.env_offset = r->env_offset;
-  rc.t0 = r->t0;
-  rc.init_low = r->init_low;
-  rc.init_high = r->init_high;
-  for (int j = 0; j < 6; ++j) {
-    rc.mean[j] = j < dim ? (mean != nullptr ? mean[j] : (j < 4 ? r->init_mean[j] : 0.0)) : 0.0;
-    rc.sigma[j] = j < dim ? (sigma != nullptr ? sigma[j] : (j < 4 ? r->init_sigma[j] : 0.0)) : 0.0;
-  }
-  rc.act_low = static_cast<float>(r->action_low);
-  rc.act_high = static_cast<float>(r->action_high);
-  io = {ep_step, ep_return, ep_index, actions, rec_observations, rec_next_observations, rec_actions, rec_rewards, rec_dones, rec_timeouts, stats};
-  return EMEI_OK;
-}
-
 template <class Fam>
-inline void launch_ref_rollout(const typename Fam::Buffers& b, const RefRolloutIO<typename Fam::Real>& io, int64_t n, const typename Fam::Consts& k,
-                               const RefRolloutConsts& rc, const NoiseConsts& z, int freq_rate, cudaStream_t s) {
+inline void launch_ref_rollout(const typename Fam::Buffers& b, const RolloutIO<typename Fam::Real>& io, int64_t n, const typename Fam::Consts& k,
+                               const RolloutConsts<6>& rc, const NoiseConsts& z, int freq_rate, cudaStream_t s) {
   rollout_ref_kernel<Fam><<<grid_for(n, kBlock), kBlock, 0, s>>>(b, io, n, k, rc, z, freq_rate);
 }
 
@@ -368,11 +297,9 @@ int cartpole_rollout_ref(R* state_io, int32_t* ep_step, R* ep_return, int32_t* e
   const bool ip = p->variant > EMEI_CARTPOLE_SWINGUP;
   if (noise != nullptr && !ip) return EMEI_ERR_BAD_VARIANT;  // the noisy step exists for the MuJoCo-shell family only (mujoco_env.py:98-104)
   if (const int e = check_noise_params(noise, 4)) return e;
-  RefRolloutConsts rc;
-  RefRolloutIO<R> io;
-  const int code = make_ref_rollout<R>(r, p->action_kind, actions, rec_obs, rec_next, rec_act, rec_rew, rec_done, rec_timeout, ep_step, ep_return,
-                                       ep_index, stats, nullptr, nullptr, 4, rc, io);
-  if (code != EMEI_OK) return code;
+  const RolloutIO<R> io = {ep_step, ep_return, ep_index, actions, rec_obs, rec_next, rec_act, rec_rew, rec_done, rec_timeout, stats};
+  RolloutConsts<6> rc;
+  if (const int e = make_rollout(r, io, false, nullptr, nullptr, rc)) return e;
   if (n == 0 || r->horizon == 0) return EMEI_OK;
   EMEI_CHECK_PTR(state_io);
   EMEI_CHECK_ALIGN16(state_io);
@@ -401,11 +328,9 @@ int i2p_rollout(R* state_io, int32_t* ep_step, R* ep_return, int32_t* ep_index, 
   EMEI_CHECK_PTR(init_sigma);
   if (const int e = check_i2p_params(*p)) return e;
   if (const int e = check_noise_params(noise, 6)) return e;
-  RefRolloutConsts rc;
-  RefRolloutIO<R> io;
-  const int code = make_ref_rollout<R>(r, p->action_kind, actions, rec_obs, rec_next, rec_act, rec_rew, rec_done, rec_timeout, ep_step, ep_return,
-                                       ep_index, stats, init_mean, init_sigma, 6, rc, io);
-  if (code != EMEI_OK) return code;
+  const RolloutIO<R> io = {ep_step, ep_return, ep_index, actions, rec_obs, rec_next, rec_act, rec_rew, rec_done, rec_timeout, stats};
+  RolloutConsts<6> rc;
+  if (const int e = make_rollout(r, io, false, init_mean, init_sigma, rc)) return e;
   if (n == 0 || r->horizon == 0) return EMEI_OK;
   EMEI_CHECK_PTR(state_io);
   EMEI_CHECK_ALIGN16(state_io);
@@ -422,11 +347,9 @@ int charged_ball_rollout_ref(uint8_t* on_circle_io, R* circle_io, R* free_state_
   EMEI_CHECK_PTR(p);
   EMEI_CHECK_PTR(r);
   if (const int e = check_charged_ball_params(*p)) return e;
-  RefRolloutConsts rc;
-  RefRolloutIO<R> io;
-  const int code = make_ref_rollout<R>(r, p->action_kind, actions, rec_obs, rec_next, rec_act, rec_rew, rec_done, rec_timeout, ep_step, ep_return,
-                                       ep_index, stats, nullptr, nullptr, 4, rc, io);
-  if (code != EMEI_OK) return code;
+  const RolloutIO<R> io = {ep_step, ep_return, ep_index, actions, rec_obs, rec_next, rec_act, rec_rew, rec_done, rec_timeout, stats};
+  RolloutConsts<6> rc;
+  if (const int e = make_rollout(r, io, false, nullptr, nullptr, rc)) return e;
   if (n == 0 || r->horizon == 0) return EMEI_OK;
   EMEI_CHECK_PTR(on_circle_io);
   EMEI_CHECK_PTR(circle_io);

@@ -79,7 +79,7 @@ class Engine:
     float32 without state noise: the packed kernels (emei_cartpole_rollout_f32 / emei_charged_ball_rollout_f32).
     float64 (reference-exact), the inverted double pendulum and obs_noise_params: the reference-arithmetic kernels
     (emei_cartpole_rollout_ref_* / emei_i2p_rollout_* / emei_charged_ball_rollout_ref_f64), one env per thread, the
-    step entry points' own device functions -- records, rewards and episode returns then have the engine dtype."""
+    step entry points' own device functions.  Records, rewards and episode returns have the engine dtype."""
 
     ep_step = ep_return = ep_index = None
     t_global = 0
@@ -89,7 +89,7 @@ class Engine:
         if self.ep_step is None:
             dev = self.env.device
             self.ep_step = torch.zeros(self.n, dtype=torch.int32, device=dev)
-            self.ep_return = torch.zeros(self.n, dtype=torch.float32, device=dev)
+            self.ep_return = torch.zeros(self.n, dtype=self.env.dtype, device=dev)
             self.ep_index = torch.zeros(self.n, dtype=torch.int32, device=dev)
             self.t_global = 0
 
@@ -102,18 +102,11 @@ class Engine:
                 self.ep_index.zero_()
                 self.t_global = 0
 
-    def _rollout(self, entry: str, state_ptrs, rp: _lib.RolloutParams, actions, record: bool, rollout_stats: torch.Tensor,
-                 ref: bool = False, extra=()):
-        """entry: C-ABI symbol (with the precision suffix); ref: a reference-arithmetic entry point (records, rewards
-        and episode returns in the engine dtype); extra: its trailing arguments before the stream (noise / init tables)."""
+    def _rollout(self, entry: str, state_ptrs, rp: _lib.RolloutParams, actions, record: bool, rollout_stats: torch.Tensor, extra=()):
+        """entry: C-ABI symbol (with the precision suffix); extra: its trailing arguments before the stream (noise / init tables)."""
         env = self.env
-        if env.dtype != torch.float32 and not ref:
-            raise NotImplementedError("the packed rollout kernels are float32")
         self._alloc_episode()
-        rdt = env.dtype if ref else torch.float32
-        if self.ep_return.dtype != rdt:  # the running return follows the kernel's real type
-            self.ep_return = self.ep_return.to(rdt)
-        T, n, dev, D = int(rp.horizon), self.n, env.device, self.obs_dim
+        T, n, dev, D, rdt = int(rp.horizon), self.n, env.device, self.obs_dim, env.dtype
         rp.t0 = self.t_global
         rec = {}
         if actions is not None:
@@ -310,7 +303,7 @@ class CartPoleEngine(RowStateEngine):
         # float64 reference-exact mode / obs_noise_params: the step entry points' own arithmetic, one env per thread
         z = ctypes.byref(noise) if noise is not None else None
         return self._rollout("emei_cartpole_rollout_ref" + self.env._suffix, [state.data_ptr()], rp, actions, record, rollout_stats,
-                             ref=True, extra=(z,))
+                             extra=(z,))
 
 
 class I2PEngine(RowStateEngine):
@@ -328,7 +321,7 @@ class I2PEngine(RowStateEngine):
         Arr = ctypes.c_double * 6
         z = ctypes.byref(noise) if noise is not None else None
         return self._rollout("emei_i2p_rollout" + self.env._suffix, [state.data_ptr()], rp, actions, record, rollout_stats,
-                             ref=True, extra=(Arr(*mean), Arr(*sigma), z))
+                             extra=(Arr(*mean), Arr(*sigma), z))
 
 
 class ChargedBallEngine(Engine):
@@ -339,10 +332,9 @@ class ChargedBallEngine(Engine):
     zero_copy_ok = False
 
     def rollout(self, rp: _lib.RolloutParams, actions, record: bool, rollout_stats: torch.Tensor, noise=None):
-        ptrs = [self.on_circle.data_ptr(), self.circle.data_ptr(), self.free.data_ptr()]
-        if self.env.dtype == torch.float32:
-            return self._rollout("emei_charged_ball_rollout_f32", ptrs, rp, actions, record, rollout_stats)
-        return self._rollout("emei_charged_ball_rollout_ref_f64", ptrs, rp, actions, record, rollout_stats, ref=True)
+        entry = "emei_charged_ball_rollout_f32" if self.env.dtype == torch.float32 else "emei_charged_ball_rollout_ref_f64"
+        return self._rollout(entry, [self.on_circle.data_ptr(), self.circle.data_ptr(), self.free.data_ptr()], rp, actions, record,
+                             rollout_stats)
 
     def __init__(self, env, params: _lib.ChargedBallParams):
         self.env = env

@@ -101,6 +101,62 @@ def test_argument_validation_codes():
     assert [lib.emei_family_action_dim(k) for k in (_lib.HOPPER, _lib.HALFCHEETAH, _lib.CARTPOLE_SWINGUP)] == [3, 6, 1]
 
 
+# Malformed inputs x every rollout entry point: the code each one returns.  The packed entries (float32) check the batch,
+# parameters and horizon, return early for empty work, then check state, episode buffers, actions and records (with the
+# 16-byte alignment of the observation records); the reference-arithmetic entries check the episode buffers, horizon,
+# actions and records (no alignment) before the early return and the state.  Every row is rejected before any launch:
+# the reference entries always get a null state, the packed ones an aligned host state only where a later check fails.
+# Columns: packed cart-pole, packed charged ball, reference cart-pole, I2P, reference charged ball (both precisions).
+_ROLLOUT_ROWS = [
+    # name,                     n,  horizon, init_kind, episode buffers, records,      packed state, codes
+    ("empty batch",             0,  8,       0,         False,           None,         False, (0, 0, -1, -1, -1)),
+    ("negative horizon",        16, -1,      0,         False,           None,         False, (-6, -6, -1, -1, -1)),
+    ("negative horizon, bufs",  16, -1,      0,         True,            None,         False, (-6, -6, -6, -6, -6)),
+    ("partial records",         16, 8,       0,         True,            "partial",    True, (-1, -1, -1, -1, -1)),
+    ("misaligned obs records",  16, 8,       0,         True,            "misaligned", True, (-5, -5, -1, -1, -1)),
+    ("bad init_kind",           16, 8,       5,         True,            None,         False, (-6, -1, -1, -1, -1)),
+]
+
+
+def _check_rollout_validation_table():
+    lib = _lib.lib
+    buf = (ctypes.c_char * 4096)()
+    base = (ctypes.addressof(buf) + 15) & ~15
+    aligned = [base + 256 * j for j in range(14)]  # distinct 16-byte-aligned host addresses (never dereferenced)
+    p = _lib.CartPoleParams()
+    p.freq_rate, p.dt, p.variant, p.action_kind = 1, 0.02, _lib.CARTPOLE_SWINGUP, _lib.ACTION_CONTINUOUS_F32
+    q = _lib.I2PParams()
+    q.gravity, q.mass_cart, q.mass_pole0, q.mass_pole1, q.length0, q.length1, q.dt = 9.81, 10.0, 4.0, 4.0, 0.3, 0.3, 0.02
+    q.freq_rate, q.variant, q.action_kind = 1, _lib.I2P_BOUNDARY_SWINGUP, _lib.ACTION_CONTINUOUS_F32
+    c = _lib.ChargedBallParams()
+    c.gravity_acc, c.mass_ball, c.radius, c.charge, c.time_step, c.freq_rate, c.action_kind = 9.8, 1.0, 1.0, 10.0, 0.02, 1, 0
+    table = (ctypes.c_double * 6)()
+    for name, n, horizon, init_kind, bufs, records, packed_state, codes in _ROLLOUT_ROWS:
+        r = _lib.RolloutParams()
+        r.horizon, r.random_policy, r.init_kind = horizon, 1, init_kind
+        episode = aligned[3:6] if bufs else [None] * 3
+        rec = [None] * 6
+        if records == "partial":
+            rec[0] = aligned[6]
+        elif records == "misaligned":
+            rec = [aligned[6] + 4] + aligned[7:12]
+        tail = [None] + rec + [None]  # actions (random policy), records, stats
+        entries = [
+            (0, lib.emei_cartpole_rollout_f32, 1, (ctypes.byref(p), ctypes.byref(r))),
+            (1, lib.emei_charged_ball_rollout_f32, 3, (ctypes.byref(c), ctypes.byref(r))),
+        ]
+        for sfx in ("_f32", "_f64"):
+            entries += [
+                (2, getattr(lib, "emei_cartpole_rollout_ref" + sfx), 1, (ctypes.byref(p), ctypes.byref(r), None)),
+                (3, getattr(lib, "emei_i2p_rollout" + sfx), 1, (ctypes.byref(q), ctypes.byref(r), table, table, None)),
+                (4, getattr(lib, "emei_charged_ball_rollout_ref" + sfx), 3, (ctypes.byref(c), ctypes.byref(r))),
+            ]
+        for col, f, n_state, params in entries:
+            state = aligned[:n_state] if (packed_state and col < 2) else [None] * n_state
+            got = f(*state, *episode, *tail, n, *params, None)
+            assert got == codes[col], f"{name}: {f.__name__} returned {got}, expected {codes[col]}"
+
+
 def test_rollout_and_transpose_validation_codes():
     lib = _lib.lib
     assert ctypes.sizeof(_lib.RolloutParams) == 6 * 4 + 4 * 8 + 2 * 8 + 8 * 8 + 2 * 8
@@ -135,6 +191,7 @@ def test_rollout_and_transpose_validation_codes():
     assert h(None, None, None, None, None, None, None, 4, ctypes.byref(q), None) == -2
     q.variant, q.length1 = _lib.I2P_REBOUND_BALANCING, 0.0
     assert h(None, None, None, None, None, None, None, 4, ctypes.byref(q), None) == -6
+    _check_rollout_validation_table()
     t = lib.emei_records_transpose
     assert t(None, None, 4, -1, 4, None) == -4
     assert t(None, None, 4, 8, 3, None) == -6          # element sizes: 1, 4, 8, 16
