@@ -134,6 +134,10 @@ _PROTOTYPES = {
     "emei_cartpole_step_vjp": (c_int, [_P] * 7 + [c_int64, POINTER(CartPoleParams), _P]),
     "emei_i2p_step_jacobian": (c_int, [_P, _P, _P, _P, c_int64, POINTER(I2PParams), _P]),
     "emei_i2p_step_vjp": (c_int, [_P] * 7 + [c_int64, POINTER(I2PParams), _P]),
+    "emei_cartpole_trajectory": (c_int, [_P] * 6 + [c_int64, c_int64, POINTER(CartPoleParams), _P]),
+    "emei_cartpole_trajectory_vjp": (c_int, [_P] * 7 + [c_int64, c_int64, POINTER(CartPoleParams), _P]),
+    "emei_i2p_trajectory": (c_int, [_P] * 6 + [c_int64, c_int64, POINTER(I2PParams), _P]),
+    "emei_i2p_trajectory_vjp": (c_int, [_P] * 7 + [c_int64, c_int64, POINTER(I2PParams), _P]),
     "emei_ip_step_noisy": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64, POINTER(CartPoleParams), POINTER(NoiseParams), _P]),
     "emei_i2p_step_noisy": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64, POINTER(I2PParams), POINTER(NoiseParams), _P]),
     "emei_cartpole_rollout_ref": (c_int, [_P] * 12 + [c_int64, POINTER(CartPoleParams), POINTER(RolloutParams), POINTER(NoiseParams), _P]),

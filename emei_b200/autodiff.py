@@ -9,6 +9,10 @@ The cart-pole family, the analytic inverted pendulum and the analytic inverted d
   (``emei_*_step_vjp_*``), which never materialises the Jacobian.  Chaining it T times is backpropagation through time.
 * ``jacobian(env, state, action)`` -> ``(jac [B,D,D+1], reward_grad [B,D+1])``: the per-sample Jacobian
   ``d(next_state, reward) / d(state, action)`` (``emei_*_step_jacobian_*``); the last column is the action's.
+* ``trajectory(env, state, actions)`` -> ``(states [T+1,B,D], obs [T,B,D], rewards [T,B], dones bool [T,B])``: T open-loop
+  steps under actions [T,B] (or [T,B,1]) in one launch (``emei_*_trajectory_*``), bit-equal to T chained ``transition``
+  calls; its backward is one reverse-sweep launch (``emei_*_trajectory_vjp_*``) that carries the state cotangent in
+  registers.  The shooting / open-loop MPC primitive; a closed-loop policy stays on the chained path.
 
 Semantics (include/emei_b200.h, DESIGN.md "Derivatives"): no state noise; the action gradient passes the control clamp
 where ``ctrl_low <= ctrl <= ctrl_high`` and is 0 for discrete actions; the I2P observation's angles have slope pi (the
@@ -16,6 +20,7 @@ where ``ctrl_low <= ctrl <= ctrl_high`` and is 0 for discrete actions; the I2P o
 the reference's float32-rounded increments).  A continuous action is cast to the env dtype inside the graph, so its
 gradient comes back in the caller's dtype and shape (``[B]`` or ``[B,1]``).
 """
+import numpy as np
 import torch
 from torch.autograd.function import once_differentiable
 
@@ -28,15 +33,15 @@ def _rows(t: torch.Tensor) -> torch.Tensor:
     return t if t.data_ptr() % 16 == 0 else t.clone()
 
 
-def _inputs(env, state, action):
-    """-> (engine, state rows [B, D] in the env dtype, action [B] in its kernel encoding, came_from_numpy).  Every
+def _inputs(env, state, action, steps=1):
+    """-> (engine, state rows [B, D] in the env dtype, action [steps * B] in its kernel encoding, came_from_numpy).  Every
     conversion is an autograd-tracked op, so gradients flow back to the caller's tensors."""
     eng = env._ensure_engine()
     s, was_np = env._to_device(state, env.dtype)
     if s.dim() != 2 or s.shape[1] != eng.obs_dim:
         raise ValueError(f"state must be [B, {eng.obs_dim}], got {tuple(s.shape)}")
     continuous = len(env.action_space.shape) > 0
-    a = normalise_action(env, action, continuous, s.shape[0])
+    a = normalise_action(env, action, continuous, steps * s.shape[0])
     if continuous:
         a = a.to(env.dtype)
     return eng, s, a, was_np
@@ -84,3 +89,45 @@ def jacobian(env, state, action):
     with torch.no_grad():
         jac, reward_grad = eng.jacobian(_rows(s.detach()), a.detach().contiguous())
     return env._ret(jac, was_np), env._ret(reward_grad, was_np)
+
+
+class StepTrajectory(torch.autograd.Function):
+    """forward: ``RowStateEngine.trajectory``; backward: ``RowStateEngine.trajectory_vjp``.  ``obs`` is None for the
+    cart-pole envs, whose observation is the next state (``trajectory`` returns ``states[1:]`` for it)."""
+
+    @staticmethod
+    def forward(ctx, state, actions, engine):
+        rows, act = _rows(state.detach()), actions.detach().contiguous()
+        states, obs, rewards, dones = engine.trajectory(rows, act)
+        ctx.engine = engine
+        ctx.save_for_backward(states, act)
+        ctx.mark_non_differentiable(dones)
+        ctx.set_materialize_grads(False)
+        return states, obs, rewards, dones
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_states, g_obs, g_rewards, g_dones):
+        states, act = ctx.saved_tensors
+        want_state, want_action = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        if g_states is None and g_obs is None and g_rewards is None:
+            return None, None, None
+        g_states = _rows(g_states) if g_states is not None else None
+        g_obs = _rows(g_obs) if g_obs is not None else None
+        g_rewards = g_rewards.contiguous() if g_rewards is not None else None
+        g0, g_act = ctx.engine.trajectory_vjp(states, act, g_states, g_obs, g_rewards, want_action)
+        return (g0 if want_state else None), g_act, None
+
+
+def trajectory(env, state, actions):
+    """``env.get_batch_trajectory``: see the module docstring."""
+    shape = tuple(actions.shape) if isinstance(actions, torch.Tensor) else np.shape(actions)
+    B = len(state)
+    if len(shape) not in (2, 3) or shape[1:] not in ((B,), (B, 1)):
+        raise ValueError(f"actions must be [T, B={B}] or [T, B, 1], got shape {shape}")
+    eng, s, a, was_np = _inputs(env, state, actions, steps=shape[0])
+    states, obs, rewards, dones = StepTrajectory.apply(s, a.reshape(shape[0], B), eng)
+    if obs is None:  # cart-pole: the observation is the next state; autograd routes its gradient into states
+        obs = states[1:]
+    out = (states, obs, rewards, dones)
+    return tuple(env._ret(t, was_np) for t in out) if was_np else out

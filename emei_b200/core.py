@@ -224,6 +224,11 @@ class EmeiEnv(Freezable):
         """``(jac [B,D,D+1], reward_grad [B,D+1])`` of the step: the analytic families only."""
         raise NotImplementedError(f"{type(self).__name__}: no Jacobian, {self._no_derivatives}")
 
+    def get_batch_trajectory(self, state, actions):
+        """Differentiable open-loop trajectory ``(states [T+1,B,D], obs [T,B,D], rewards [T,B], dones bool [T,B])`` of
+        actions [T,B]: the analytic families only."""
+        raise NotImplementedError(f"{type(self).__name__}: no gradients, {self._no_derivatives}")
+
     # ------------------------------------------------------------------ fused rollouts
     def rollout(self, horizon: int, actions=None, record: bool = False, auto_reset: bool = True, max_episode_steps=None):
         """``horizon`` steps of every env in ONE kernel launch: the batched counterpart of the reference's

@@ -248,6 +248,16 @@ __device__ __forceinline__ void i2p_tangent(R (&y)[6], R (&T)[6][7], R F, R dF, 
   }
 }
 
+// primal control -> force gear * clamp(ctrl) and d force / d ctrl (the step's mj_step clamp, inclusive)
+template <typename R>
+__device__ __forceinline__ void i2p_force_and_slope(const void* action, int64_t i, const I2PConsts<R>& k, R& F, R& dF) {
+  const bool continuous = k.action_kind >= EMEI_ACTION_CONTINUOUS_F32;
+  const R ctrl = load_ctrl<R>(action, i, k.action_kind);
+  const R cc = ctrl < k.ctrl_low ? k.ctrl_low : (ctrl > k.ctrl_high ? k.ctrl_high : ctrl);
+  F = k.gear * cc;
+  dF = (continuous && ctrl >= k.ctrl_low && ctrl <= k.ctrl_high) ? k.gear : R(0);
+}
+
 // d reward / d y_out of the variant, through the observation (slope pi on both angles: the current_obs quirk)
 template <typename R>
 __device__ __forceinline__ void i2p_reward_slope(const R (&y)[6], const I2PConsts<R>& k, R (&wr)[6]) {
@@ -271,14 +281,11 @@ __global__ void __launch_bounds__(kBlock)
                      const R* __restrict__ g_state_out, const R* __restrict__ g_obs, const R* __restrict__ g_reward,
                      R* __restrict__ g_state_in, R* __restrict__ g_action, int64_t n, bool vec2, const I2PConsts<R> k) {
   const int64_t stride = static_cast<int64_t>(gridDim.x) * kBlock;
-  const bool continuous = k.action_kind >= EMEI_ACTION_CONTINUOUS_F32;
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * kBlock + threadIdx.x; i < n; i += stride) {
-    R y[6], T[6][7], wr[6];
+    R y[6], T[6][7], wr[6], F, dF;
     i2p_load_row<R>(state_in, i, vec2, y);
-    const R ctrl = load_ctrl<R>(action, i, k.action_kind);
-    const R cc = ctrl < k.ctrl_low ? k.ctrl_low : (ctrl > k.ctrl_high ? k.ctrl_high : ctrl);
-    const R dF = (continuous && ctrl >= k.ctrl_low && ctrl <= k.ctrl_high) ? k.gear : R(0);
-    i2p_tangent<R>(y, T, k.gear * cc, dF, k);
+    i2p_force_and_slope<R>(action, i, k, F, dF);
+    i2p_tangent<R>(y, T, F, dF, k);
     i2p_reward_slope<R>(y, k, wr);
     if constexpr (!VJP) {
       R* J = jac + 42 * i;

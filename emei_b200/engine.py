@@ -171,6 +171,8 @@ class RowStateEngine(Engine):
         self.separate_obs = separate_obs
         self._step_entry, self._noisy_entry = step_entry, noisy_entry
         self._jacobian_entry, self._vjp_entry = step_entry + "_jacobian", step_entry + "_vjp"
+        self._trajectory_entry = step_entry[: -len("_step")] + "_trajectory"
+        self._trajectory_vjp_entry = self._trajectory_entry + "_vjp"
         self._bufs = self._obs = self._out = None
         self._cur = 0
         self.has_state = False
@@ -287,6 +289,44 @@ class RowStateEngine(Engine):
         env._call(self._vjp_entry, rows.data_ptr(), action.data_ptr(), ptr(g_state_out), ptr(g_obs), ptr(g_reward), g_in.data_ptr(),
                   ptr(g_act), b, ctypes.byref(self.params), env._stream())
         return g_in, g_act
+
+    def trajectory(self, rows: torch.Tensor, actions: torch.Tensor):
+        """``T`` open-loop steps of ``transition_stateless`` from rows [b, width] under actions [T, b] in one launch
+        (emei_*_trajectory_*) -> (states [T+1, b, width], obs [T, b, width] or None when the family has no separate
+        observation, rewards [T, b], dones bool [T, b]); states[0] = rows.  The engine's own state is untouched."""
+        env = self.env
+        T, b, d = actions.shape[0], rows.shape[0], self.obs_dim
+        states = torch.empty((T + 1, b, d), dtype=env.dtype, device=env.device)
+        obs = torch.empty((T, b, d), dtype=env.dtype, device=env.device) if self.separate_obs else None
+        rewards = torch.empty((T, b), dtype=env.dtype, device=env.device)
+        dones = torch.empty((T, b), dtype=torch.uint8, device=env.device)
+        if T == 0 or b == 0:
+            states.copy_(rows.reshape(1, b, d))
+        else:
+            self.params.action_kind = _ACTION_KIND[actions.dtype]
+            env._call(self._trajectory_entry, rows.data_ptr(), actions.data_ptr(), states.data_ptr(),
+                      obs.data_ptr() if obs is not None else None, rewards.data_ptr(), dones.data_ptr(), b, T,
+                      ctypes.byref(self.params), env._stream())
+        return states, obs, rewards, dones.view(torch.bool)
+
+    def trajectory_vjp(self, states: torch.Tensor, actions: torch.Tensor, g_states, g_obs, g_rewards, want_action: bool):
+        """Reverse sweep of ``trajectory`` (emei_*_trajectory_vjp_*): the cotangents ``g_states`` [T+1, b, width],
+        ``g_obs`` [T, b, width] and ``g_rewards`` [T, b] are contiguous tensors or None (zero).
+        -> (g_state0 [b, width], g_actions [T, b] or None)."""
+        env = self.env
+        T, b = actions.shape[0], states.shape[1]
+        g0 = torch.empty_like(states[0])
+        g_act = torch.empty((T, b), dtype=env.dtype, device=env.device) if want_action else None
+        if T == 0 or b == 0:
+            g0.copy_(g_states[0]) if g_states is not None else g0.zero_()
+            if g_act is not None:
+                g_act.zero_()
+            return g0, g_act
+        self.params.action_kind = _ACTION_KIND[actions.dtype]
+        ptr = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
+        env._call(self._trajectory_vjp_entry, states.data_ptr(), actions.data_ptr(), ptr(g_states), ptr(g_obs), ptr(g_rewards),
+                  g0.data_ptr(), ptr(g_act), b, T, ctypes.byref(self.params), env._stream())
+        return g0, g_act
 
 
 class CartPoleEngine(RowStateEngine):

@@ -116,6 +116,14 @@ class BaseCartPoleEnv(BaseControlEnv):
         column is 0 for discrete actions."""
         return autodiff.jacobian(self, state, action)
 
+    def get_batch_trajectory(self, state, actions):
+        """T open-loop steps from caller rows ``state`` [B,4] under ``actions`` [T,B] (or [T,B,1]) in one launch ->
+        ``(states [T+1,B,4], obs [T,B,4], rewards [T,B], dones bool [T,B])``; states[0] = state, obs = states[1:], and
+        step t equals the t-th of T chained ``get_batch_transition`` calls bit for bit.  No resets, noise or statistics: an
+        env whose done flag is set keeps being integrated, so mask with ``dones``.  Differentiable w.r.t. ``state`` and a
+        continuous ``actions``; the backward is one reverse-sweep launch (emei_cartpole_trajectory_vjp_*)."""
+        return autodiff.trajectory(self, state, actions)
+
 
 class CartPoleBalancingEnv(BaseCartPoleEnv):
     _variant = _lib.CARTPOLE_BALANCING

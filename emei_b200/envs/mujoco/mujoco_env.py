@@ -256,6 +256,14 @@ class AnalyticPendulumEnv(EmeiMujocoEnv):
         """``(jac [B,D,D+1], reward_grad [B,D+1])`` = d(next_state, reward) / d(state, action) of the same step."""
         return autodiff.jacobian(self, state, action)
 
+    def get_batch_trajectory(self, state, actions):
+        """T open-loop steps from rows ``state`` = qpos || qvel (angles unwrapped) under ``actions`` [T,B] (or [T,B,1]) in
+        one launch -> ``(states [T+1,B,D], obs [T,B,D], rewards [T,B], dones bool [T,B])``; states[0] = state, and step t
+        equals the t-th of T chained ``get_batch_transition`` calls bit for bit.  No resets, noise or statistics: an env
+        whose done flag is set keeps being integrated, so mask with ``dones``.  Differentiable w.r.t. ``state`` and
+        ``actions``; the backward is one reverse-sweep launch (emei_cartpole_trajectory_vjp_* / emei_i2p_trajectory_vjp_*)."""
+        return autodiff.trajectory(self, state, actions)
+
     def _next_obs_rows(self, obs, state):
         """The rows get_batch_next_obs steps: ``obs`` (``state=`` is not read)."""
         return obs

@@ -212,6 +212,44 @@ int emei_i2p_step_vjp_f64(const double* state_in, const void* action, const doub
                           const double* g_reward, double* g_state_in, double* g_action, int64_t n, const emei_i2p_params* p,
                           emei_stream_t stream);
 
+/* ---- differentiable open-loop trajectories (T steps in one launch, their VJP in one reverse sweep) -------
+ * The open-loop composition of `horizon` stateless steps of emei_cartpole_step_* (cart-pole and EMEI_IP_* variants) /
+ * emei_i2p_step_* from caller rows: no state noise, no resets, no statistics, and an env whose done flag is set keeps
+ * being integrated.  Every array is time-major; D = 4 (cart-pole family) or 6 (I2P):
+ *   state0 [n,D] ; actions [horizon,n] (EMEI_ACTION_* encoding) ; states [horizon+1,n,D] ; obs [horizon,n,D] ;
+ *   rewards, dones [horizon,n] ; g_state0 [n,D] ; g_states [horizon+1,n,D] ; g_obs [horizon,n,D] ; g_rewards, g_actions [horizon,n].
+ * Forward: states[0] = state0; states[t+1], obs[t], rewards[t], dones[t] are bit-equal to the t-th of `horizon` chained
+ * step calls (the step's own device functions; float32 cart-pole / IP: the lean arithmetic of the step kernel).  obs and
+ * dones are nullable (not written); the cart-pole envs' observation is the next state, so they pass obs NULL.
+ * VJP: the reverse sweep of the same composition under the derivative model above (float64 cart-pole: the float64 Euler
+ * step; clamp inclusive; I2P observation angles slope pi):
+ *   g_state0 = d L / d state0 and g_actions[t] = d L / d actions[t] for L = <g_states, states> + <g_obs, obs> + <g_rewards, rewards>.
+ *   g_states, g_obs, g_rewards each nullable (= zero); g_actions nullable, and must be NULL for discrete action kinds (else
+ *   EMEI_ERR_BAD_ACTION_KIND).  The cotangent is carried in registers from step to step; only g_actions and g_state0 are written.
+ * Validation: n < 0 or horizon < 0 -> EMEI_ERR_BAD_SIZE, then the step / VJP entry points' checks in their order; n == 0 or
+ * horizon == 0 returns EMEI_OK with nothing launched or written.  Cart-pole row arrays are 16-byte aligned (EMEI_ERR_MISALIGNED). */
+int emei_cartpole_trajectory_f32(const float* state0, const void* actions, float* states, float* obs, float* rewards, uint8_t* dones,
+                                 int64_t n, int64_t horizon, const emei_cartpole_params* p, emei_stream_t stream);
+int emei_cartpole_trajectory_f64(const double* state0, const void* actions, double* states, double* obs, double* rewards,
+                                 uint8_t* dones, int64_t n, int64_t horizon, const emei_cartpole_params* p, emei_stream_t stream);
+int emei_cartpole_trajectory_vjp_f32(const float* states, const void* actions, const float* g_states, const float* g_obs,
+                                     const float* g_rewards, float* g_state0, float* g_actions, int64_t n, int64_t horizon,
+                                     const emei_cartpole_params* p, emei_stream_t stream);
+int emei_cartpole_trajectory_vjp_f64(const double* states, const void* actions, const double* g_states, const double* g_obs,
+                                     const double* g_rewards, double* g_state0, double* g_actions, int64_t n, int64_t horizon,
+                                     const emei_cartpole_params* p, emei_stream_t stream);
+/* the same pair for emei_i2p_step_*: rows of 6 */
+int emei_i2p_trajectory_f32(const float* state0, const void* actions, float* states, float* obs, float* rewards, uint8_t* dones,
+                            int64_t n, int64_t horizon, const emei_i2p_params* p, emei_stream_t stream);
+int emei_i2p_trajectory_f64(const double* state0, const void* actions, double* states, double* obs, double* rewards, uint8_t* dones,
+                            int64_t n, int64_t horizon, const emei_i2p_params* p, emei_stream_t stream);
+int emei_i2p_trajectory_vjp_f32(const float* states, const void* actions, const float* g_states, const float* g_obs,
+                                const float* g_rewards, float* g_state0, float* g_actions, int64_t n, int64_t horizon,
+                                const emei_i2p_params* p, emei_stream_t stream);
+int emei_i2p_trajectory_vjp_f64(const double* states, const void* actions, const double* g_states, const double* g_obs,
+                                const double* g_rewards, double* g_state0, double* g_actions, int64_t n, int64_t horizon,
+                                const emei_i2p_params* p, emei_stream_t stream);
+
 /* ---- per-sub-step Gaussian state noise ("obs_noise_params", SURVEY 8f rank 4) -------------------
  * Replaces mujoco_env.py:98-104: after EVERY sub-step the reference overwrites the simulator state with
  * additive_gaussian_noise(qpos, qvel, obs_noise_params) (mujoco_env.py:197-249: one N(0, sigma_pos) /
