@@ -147,6 +147,9 @@ _PROTOTYPES = {
     "emei_reward_terminal": (c_int, [_P, _P, _P, _P, _P, _P, c_int64, POINTER(ScoringParams), _P]),
     "emei_reward_terminal_seq": (c_int, [_P, _P, _P, _P, _P, c_int64, c_int64, POINTER(ScoringParams), _P]),
     "emei_sumsq": (c_int, [_P, c_int64, _P, _P, _P]),
+    "emei_sum": (c_int, [_P, c_int64, _P, _P, _P]),
+    "emei_reward_vjp": (c_int, [_P] * 7 + [c_int64, POINTER(ScoringParams), _P]),
+    "emei_reward_seq_vjp": (c_int, [_P] * 6 + [c_int64, c_int64, POINTER(ScoringParams), _P]),
     "emei_init_uniform": (c_int, [_P, c_int64, c_int32, c_double, c_double, c_int32, c_uint64, c_uint64, _P]),
     "emei_init_gaussian": (c_int, [_P, c_int64, c_int32, POINTER(c_double), POINTER(c_double), c_uint64, c_uint64, _P]),
     "emei_init_charged_ball": (c_int, [_P, _P, _P, c_int64, c_double, c_uint64, c_uint64, _P]),

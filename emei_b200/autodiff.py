@@ -14,17 +14,29 @@ The cart-pole family, the analytic inverted pendulum and the analytic inverted d
   calls; its backward is one reverse-sweep launch (``emei_*_trajectory_vjp_*``) that carries the state cotangent in
   registers.  The shooting / open-loop MPC primitive; a closed-loop policy stays on the chained path.
 
-Semantics (include/emei_b200.h, DESIGN.md "Derivatives"): no state noise; the action gradient passes the control clamp
+* Scoring: ``get_batch_reward`` / ``get_batch_reward_terminal`` / ``get_batch_reward_terminal_seq`` of every env record
+  their reward in the autograd graph when grad mode is on and ``obs``, ``pre_obs`` or ``action`` requires grad
+  (``RewardScore`` / ``RewardScoreSeq``: the scoring kernels forward, ``emei_reward_vjp_*`` / ``emei_reward_seq_vjp_*``
+  backward).  Hopper / HalfCheetah's control cost is summed over the whole batch, so every action's gradient is
+  ``-2 ctrl_w a`` times the sum G of ALL reward cotangents (``emei_sum_*``); with ``ctrl_cost_scope="global"`` and
+  torch.distributed initialised the backward all-reduces G, so every rank must backpropagate through its call (a
+  collective, as with DDP).  ``done`` is not differentiable.  Otherwise the call takes the plain path: same launches,
+  same bits, no ``grad_fn``.
+
+Semantics of the dynamics (include/emei_b200.h, DESIGN.md "Derivatives"): no state noise; the action gradient passes the control clamp
 where ``ctrl_low <= ctrl <= ctrl_high`` and is 0 for discrete actions; the I2P observation's angles have slope pi (the
 ``current_obs`` precedence quirk).  The float64 cart-pole gradient is that of the float64 Euler step (the forward keeps
 the reference's float32-rounded increments).  A continuous action is cast to the env dtype inside the graph, so its
 gradient comes back in the caller's dtype and shape (``[B]`` or ``[B,1]``).
 """
+import ctypes
+
 import numpy as np
 import torch
 from torch.autograd.function import once_differentiable
 
-from .engine import normalise_action
+from . import _lib
+from .engine import _aligned16, _sumsq, normalise_action, score_rows, score_seq_rows
 
 
 def _rows(t: torch.Tensor) -> torch.Tensor:
@@ -131,3 +143,96 @@ def trajectory(env, state, actions):
         obs = states[1:]
     out = (states, obs, rewards, dones)
     return tuple(env._ret(t, was_np) for t in out) if was_np else out
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# scoring
+# ---------------------------------------------------------------------------------------------------------------------
+_MUJOCO = (_lib.HOPPER, _lib.HALFCHEETAH)
+
+
+def _ptr(t):
+    return t.data_ptr() if t is not None else None
+
+
+def _grad_inputs(env, params, obs, action, want_action, rows, group):
+    """-> (obs pointer source or None, action rows or None, G or None): the obs rows only where the family's derivative
+    reads them (not Hopper / HalfCheetah's), and G = the all-reduced sum of the reward cotangents ``rows`` when the
+    action gradient is wanted (one 8-byte all-reduce with ``ctrl_cost_scope="global"``, as the forward's sum of squares)."""
+    mj = params.family in _MUJOCO
+    g_sum = _sumsq(env, rows, group, entry="emei_sum") if want_action else None
+    return (None if mj else _aligned16(obs)), (_aligned16(action) if want_action else None), g_sum
+
+
+def _check_action_width(params, a, rows: int):
+    if params.family in _MUJOCO and a is not None:
+        width = _lib.lib.emei_family_action_dim(params.family)
+        if a.numel() != rows * width:
+            raise ValueError(f"a differentiable reward needs actions of width {width}, got shape {tuple(a.shape)}")
+
+
+class RewardScore(torch.autograd.Function):
+    """forward: ``engine.score_rows`` (the scoring kernels of ``engine.score``); backward: ``emei_reward_vjp_*``."""
+
+    @staticmethod
+    def forward(ctx, obs, pre_obs, action, env, params, group):
+        _check_action_width(params, action, obs.shape[0])
+        reward, done = score_rows(env, params, obs, pre_obs, action, group)
+        ctx.env, ctx.params, ctx.group = env, params, group
+        ctx.save_for_backward(obs, action)
+        ctx.mark_non_differentiable(done)
+        ctx.set_materialize_grads(False)
+        return reward, done
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_reward, g_done):
+        if g_reward is None:
+            return None, None, None, None, None, None
+        env, params = ctx.env, ctx.params
+        obs, action = ctx.saved_tensors
+        want_o, want_p, want_a = ctx.needs_input_grad[:3]
+        b = obs.shape[0]
+        g = _aligned16(g_reward.reshape(b).contiguous())
+        o, a, g_sum = _grad_inputs(env, params, obs, action, want_a, g, ctx.group)
+        g_obs = torch.empty_like(obs) if want_o else None
+        g_pre = torch.empty_like(obs) if want_p else None
+        g_act = torch.empty_like(action) if want_a else None
+        launches = int(want_o or want_p) + int(want_a)
+        env._call("emei_reward_vjp", _ptr(o), _ptr(a), g.data_ptr(), _ptr(g_sum), _ptr(g_obs), _ptr(g_pre), _ptr(g_act), b,
+                  ctypes.byref(params), env._stream(), launches=launches)
+        return g_obs, g_pre, g_act, None, None, None
+
+
+class RewardScoreSeq(torch.autograd.Function):
+    """forward: ``engine.score_seq_rows`` (emei_reward_terminal_seq_*); backward: ``emei_reward_seq_vjp_*``, which writes
+    every row of d/d obs_seq once (row t: transition t-1's obs term + transition t's pre_obs term)."""
+
+    @staticmethod
+    def forward(ctx, obs_seq, action, env, params, group):
+        T, n = obs_seq.shape[0] - 1, obs_seq.shape[1]
+        _check_action_width(params, action, T * n)
+        reward, done = score_seq_rows(env, params, obs_seq, action, group)
+        ctx.env, ctx.params, ctx.group = env, params, group
+        ctx.save_for_backward(obs_seq, action)
+        ctx.mark_non_differentiable(done)
+        ctx.set_materialize_grads(False)
+        return reward, done
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_reward, g_done):
+        if g_reward is None:
+            return None, None, None, None, None
+        env, params = ctx.env, ctx.params
+        obs_seq, action = ctx.saved_tensors
+        want_s, want_a = ctx.needs_input_grad[:2]
+        T, n = obs_seq.shape[0] - 1, obs_seq.shape[1]
+        g = _aligned16(g_reward.reshape(T, n).contiguous())
+        s, a, g_sum = _grad_inputs(env, params, obs_seq, action, want_a, g, ctx.group)
+        # every row is written by the kernel; an empty trajectory launches nothing, so its one row is zero-filled here
+        g_seq = (torch.empty_like if T and n else torch.zeros_like)(obs_seq)
+        g_act = torch.empty_like(action) if want_a else None
+        env._call("emei_reward_seq_vjp", _ptr(s), _ptr(a), g.data_ptr(), _ptr(g_sum), g_seq.data_ptr(), _ptr(g_act), n, T,
+                  ctypes.byref(params), env._stream(), launches=1 + int(want_a))
+        return (g_seq if want_s else None), g_act, None, None, None

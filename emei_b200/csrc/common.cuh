@@ -297,6 +297,8 @@ __device__ __forceinline__ void sincos_r(float a, float* s, float* c) { sincosf(
 __device__ __forceinline__ void sincos_r(double a, double* s, double* c) { sincos(a, s, c); }
 __device__ __forceinline__ float cos_r(float a) { return cosf(a); }
 __device__ __forceinline__ double cos_r(double a) { return cos(a); }
+__device__ __forceinline__ float sin_r(float a) { return sinf(a); }
+__device__ __forceinline__ double sin_r(double a) { return sin(a); }
 __device__ __forceinline__ float sqrt_r(float a) { return sqrtf(a); }
 __device__ __forceinline__ double sqrt_r(double a) { return sqrt(a); }
 __device__ __forceinline__ float asin_r(float a) { return asinf(a); }

@@ -582,6 +582,51 @@ __device__ __forceinline__ void score_row(const R (&o)[D], R p0, R ctrl_cost, co
   }
 }
 
+// 1 / x rounded to nearest, without the division subroutine (whose call made the float64 trajectory VJP spill)
+__device__ __forceinline__ float rcp_rn(float x) { return __frcp_rn(x); }
+__device__ __forceinline__ double rcp_rn(double x) { return __drcp_rn(x); }
+
+// Does the reward gradient of the family read the observation row?  Constant rewards do not, nor do Hopper / HalfCheetah,
+// whose reward is affine in obs[:, 0] and pre_obs[:, 0].
+template <int FAMILY>
+__host__ __device__ constexpr bool score_grad_reads_obs() {
+  return FAMILY == EMEI_CARTPOLE_SWINGUP || FAMILY == EMEI_IP_REBOUND_SWINGUP || FAMILY == EMEI_IP_BOUNDARY_SWINGUP ||
+         FAMILY == EMEI_I2P_REBOUND_SWINGUP || FAMILY == EMEI_I2P_BOUNDARY_SWINGUP || FAMILY == EMEI_CHARGED_BALL;
+}
+
+// The derivative of score_row's reward, the one place it is written (the row and the trajectory VJP kernels call it, so the
+// two layouts give the same bits): go = g * d rew / d o (every column written), gp0 = g * d rew / d p0.  The batch-wide
+// control cost's derivative is the action's (ctrl_cost_vjp_kernel); `notdone` and the healthy term are piecewise constant.
+template <typename R, int FAMILY, int D>
+__device__ __forceinline__ void score_row_grad(const R (&o)[D], R g, const ScoringConsts<R>& k, R (&go)[D], R& gp0) {
+#pragma unroll
+  for (int c = 0; c < D; ++c) go[c] = R(0);
+  gp0 = R(0);
+  if constexpr (FAMILY == EMEI_CARTPOLE_SWINGUP) {  // (cos o2 + 1) / 2
+    go[2] = -sin_r(o[2]) / R(2) * g;
+  } else if constexpr (FAMILY == EMEI_IP_REBOUND_SWINGUP || FAMILY == EMEI_IP_BOUNDARY_SWINGUP) {  // (1 - cos o1) / 2
+    go[1] = sin_r(o[1]) / R(2) * g;
+  } else if constexpr (FAMILY == EMEI_I2P_REBOUND_SWINGUP || FAMILY == EMEI_I2P_BOUNDARY_SWINGUP) {
+    // (2 - cos o1 - cos(o1 + o2)) / 4 [- 5e-3 o4^2 - 1e-4 o5^2]
+    const R s12 = sin_r(o[1] + o[2]) / R(4);
+    go[1] = (sin_r(o[1]) / R(4) + s12) * g;
+    go[2] = s12 * g;
+    if constexpr (FAMILY == EMEI_I2P_BOUNDARY_SWINGUP) {
+      go[4] = R(-1e-2) * o[4] * g;
+      go[5] = R(-2e-4) * o[5] * g;
+    }
+  } else if constexpr (FAMILY == EMEI_HOPPER || FAMILY == EMEI_HALFCHEETAH) {  // fwd_w (o0 - p0) / dt
+    const R v = k.fwd_w * rcp_rn(k.dt) * g;
+    go[0] = v;
+    gp0 = -v;
+  } else if constexpr (FAMILY == EMEI_CHARGED_BALL) {  // 1 - rho / radius; 0 at rho = 0
+    const R rho = sqrt_r(o[0] * o[0] + o[1] * o[1]);
+    const R s = rho == R(0) ? R(0) : -g / (k.radius * rho);
+    go[0] = s * o[0];
+    go[1] = s * o[1];
+  }
+}
+
 template <typename R, int FAMILY>
 __global__ void __launch_bounds__(kBlock)
     reward_terminal_kernel(const R* __restrict__ obs, const R* __restrict__ pre_obs, R* __restrict__ reward,
@@ -761,10 +806,13 @@ constexpr int kSumsqMaxBlocks = kNumSMs * 8;
 // to workspace[1 + blockIdx]; the last CTA to arrive (ticket counter in workspace[0], left at zero
 // again for the next call) adds the partials in index order.  No floating-point atomics: the result
 // does not depend on CTA scheduling, so get_batch_reward and get_batch_reward_terminal agree bitwise.
-template <typename R>
-__global__ void __launch_bounds__(kBlock) sumsq_kernel(const R* __restrict__ x, int64_t n, double* out, double* workspace) {
+// SQUARE: the sum of squares (sumsq_kernel) or the plain sum (sum_kernel: the batch-wide sum of the reward cotangents that the
+// control cost's derivative needs).
+template <typename R, bool SQUARE>
+__device__ __forceinline__ void batch_sum(const R* __restrict__ x, int64_t n, double* out, double* workspace) {
   // grid-stride, 128-bit loads on the aligned body; double accumulation
   constexpr int V = 16 / sizeof(R);
+  auto term = [](double t) { return SQUARE ? t * t : t; };
   const int64_t nvec = n / V;
   double acc = 0.0;
   const int64_t stride = static_cast<int64_t>(gridDim.x) * kBlock;
@@ -779,18 +827,17 @@ __global__ void __launch_bounds__(kBlock) sumsq_kernel(const R* __restrict__ x, 
     for (int u = 0; u < 4; ++u) {
       const R* v = reinterpret_cast<const R*>(&q[u]);
 #pragma unroll
-      for (int e = 0; e < V; ++e) acc += static_cast<double>(v[e]) * static_cast<double>(v[e]);
+      for (int e = 0; e < V; ++e) acc += term(static_cast<double>(v[e]));
     }
   }
   for (; j < nvec; j += stride) {
     const uint4 q = __ldg(reinterpret_cast<const uint4*>(x) + j);
     const R* v = reinterpret_cast<const R*>(&q);
 #pragma unroll
-    for (int e = 0; e < V; ++e) acc += static_cast<double>(v[e]) * static_cast<double>(v[e]);
+    for (int e = 0; e < V; ++e) acc += term(static_cast<double>(v[e]));
   }
   if (blockIdx.x == 0 && threadIdx.x < n - nvec * V) {
-    const double t = static_cast<double>(x[nvec * V + threadIdx.x]);
-    acc += t * t;
+    acc += term(static_cast<double>(x[nvec * V + threadIdx.x]));
   }
   __shared__ double s_acc[kBlock / 32];
   __shared__ bool s_last;
@@ -827,7 +874,17 @@ __global__ void __launch_bounds__(kBlock) sumsq_kernel(const R* __restrict__ x, 
 }
 
 template <typename R>
-int sumsq(const R* x, int64_t n_elems, double* out, double* workspace, emei_stream_t stream) {
+__global__ void __launch_bounds__(kBlock) sumsq_kernel(const R* __restrict__ x, int64_t n, double* out, double* workspace) {
+  batch_sum<R, true>(x, n, out, workspace);
+}
+
+template <typename R>
+__global__ void __launch_bounds__(kBlock) sum_kernel(const R* __restrict__ x, int64_t n, double* out, double* workspace) {
+  batch_sum<R, false>(x, n, out, workspace);
+}
+
+template <typename R, bool SQUARE>
+int batch_sum_launch(const R* x, int64_t n_elems, double* out, double* workspace, emei_stream_t stream) {
   if (n_elems < 0) return EMEI_ERR_BAD_SIZE;
   EMEI_CHECK_PTR(out);
   EMEI_CHECK_PTR(workspace);
@@ -841,9 +898,276 @@ int sumsq(const R* x, int64_t n_elems, double* out, double* workspace, emei_stre
   constexpr int V = 16 / sizeof(R);
   int64_t want = (n_elems / V + kBlock - 1) / kBlock;
   int grid = static_cast<int>(want < 1 ? 1 : (want > kSumsqMaxBlocks ? kSumsqMaxBlocks : want));
-  sumsq_kernel<R><<<grid, kBlock, 0, s>>>(x, n_elems, out, workspace);
+  if constexpr (SQUARE)
+    sumsq_kernel<R><<<grid, kBlock, 0, s>>>(x, n_elems, out, workspace);
+  else
+    sum_kernel<R><<<grid, kBlock, 0, s>>>(x, n_elems, out, workspace);
   return launch_status();
 }
+
+template <typename R>
+int sumsq(const R* x, int64_t n_elems, double* out, double* workspace, emei_stream_t stream) {
+  return batch_sum_launch<R, true>(x, n_elems, out, workspace, stream);
+}
+
+template <typename R>
+int sum(const R* x, int64_t n_elems, double* out, double* workspace, emei_stream_t stream) {
+  return batch_sum_launch<R, false>(x, n_elems, out, workspace, stream);
+}
+
+// =============================================================================================
+// scoring VJP: d reward / d (obs, pre_obs, action) contracted with the reward cotangent g
+// =============================================================================================
+// row store: the widest vector access the row stride allows (the mirror of load_row)
+template <typename R, int D>
+__device__ __forceinline__ void store_row(R* __restrict__ base, int64_t row, const R (&v)[D]) {
+  constexpr int kBytes = D * sizeof(R);
+  char* p = reinterpret_cast<char*>(base) + row * kBytes;
+  if constexpr (kBytes % 16 == 0) {
+#pragma unroll
+    for (int j = 0; j < kBytes / 16; ++j) reinterpret_cast<uint4*>(p)[j] = reinterpret_cast<const uint4*>(v)[j];
+  } else {
+    static_assert(kBytes % 8 == 0, "row stride must be a multiple of 8 bytes");
+#pragma unroll
+    for (int j = 0; j < kBytes / 8; ++j) reinterpret_cast<uint2*>(p)[j] = reinterpret_cast<const uint2*>(v)[j];
+  }
+}
+
+// Gradient row store of the VJP kernels.  Hopper / HalfCheetah rows are 48-144 bytes: one row per lane spreads each of a warp's
+// store instructions over 3-9x the sectors of one contiguous access, and measured 0.21-0.84 of the copy peak.  STAGE: a full
+// warp's 32 consecutive rows (one contiguous run, 16-byte aligned) go through the warp's slice of shared memory and leave as
+// 16-byte stores at consecutive addresses.  `warp_full` must be uniform across the warp; other warps store row by row.
+template <typename R, int D, bool STAGE>
+__device__ __forceinline__ void store_grad_row(R* __restrict__ base, int64_t row, const R (&v)[D], R* __restrict__ s_warp,
+                                               bool warp_full) {
+  if (!STAGE || !warp_full) {
+    store_row<R, D>(base, row, v);
+    return;
+  }
+  const int lane = threadIdx.x & 31;
+  __syncwarp();  // the previous row's chunks have left s_warp
+  store_row<R, D>(s_warp, lane, v);
+  __syncwarp();
+  constexpr int kChunks = 2 * D * static_cast<int>(sizeof(R));  // 32 rows of D * sizeof(R) bytes in 16-byte chunks
+  const uint4* src = reinterpret_cast<const uint4*>(s_warp);
+  uint4* dst = reinterpret_cast<uint4*>(base + (row - lane) * D);
+#pragma unroll
+  for (int q = 0; q < (kChunks + 31) / 32; ++q) {
+    const int c = q * 32 + lane;
+    if (c < kChunks) dst[c] = src[c];
+  }
+}
+
+template <int FAMILY>
+__host__ __device__ constexpr bool score_grad_stages_rows() {
+  return FAMILY == EMEI_HOPPER || FAMILY == EMEI_HALFCHEETAH;
+}
+
+// one transition row per thread: g_obs[i] = g[i] d rew / d obs[i], g_pre_obs[i] = g[i] d rew / d pre_obs[i] (dense rows,
+// each nullable); the obs row is loaded only where the family's derivative reads it
+template <typename R, int FAMILY>
+__global__ void __launch_bounds__(kBlock)
+    reward_vjp_kernel(const R* __restrict__ obs, const R* __restrict__ g_reward, R* __restrict__ g_obs, R* __restrict__ g_pre_obs,
+                      int64_t n, const ScoringConsts<R> k) {
+  constexpr int D = FamilyDim<R, FAMILY>::value;
+  constexpr bool kStage = score_grad_stages_rows<FAMILY>();
+  __shared__ alignas(16) R s_stage[kStage ? kBlock * D : 1];
+  R* s_warp = s_stage + (kStage ? (threadIdx.x >> 5) * 32 * D : 0);
+  const int64_t i = static_cast<int64_t>(blockIdx.x) * kBlock + threadIdx.x;
+  const bool warp_full = static_cast<int64_t>(blockIdx.x) * kBlock + (threadIdx.x | 31) < n;
+  if (i >= n) return;  // in the last, partial warp only
+  alignas(16) R o[D] = {};
+  if constexpr (score_grad_reads_obs<FAMILY>()) load_row<R, D>(obs, i, o);
+  alignas(16) R go[D];
+  R gp0;
+  score_row_grad<R, FAMILY, D>(o, __ldg(g_reward + i), k, go, gp0);
+  if (g_obs != nullptr) store_grad_row<R, D, kStage>(g_obs, i, go, s_warp, warp_full);
+  if (g_pre_obs != nullptr) {
+    alignas(16) R gp[D] = {};
+    gp[0] = gp0;
+    store_grad_row<R, D, kStage>(g_pre_obs, i, gp, s_warp, warp_full);
+  }
+}
+
+// Trajectory layout: g_obs_seq[r] = g[r-1] d rew_{r-1} / d obs + g[r] d rew_r / d pre_obs for the T + 1 rows r of obs_seq
+// (the first term exists for r >= 1, the second for r < T).  One thread per env column walks a segment of rows (grid.y =
+// segments) and carries g[r] to the next row as its g[r-1]: every g_obs_seq row is written once, every cotangent read once,
+// plus one boundary neighbour per segment; the next row's loads are issued before the current row's math.
+template <typename R, int FAMILY>
+__global__ void __launch_bounds__(kBlock)
+    reward_seq_vjp_kernel(const R* __restrict__ obs_seq, const R* __restrict__ g_reward, R* __restrict__ g_obs_seq, int64_t n_envs,
+                          int64_t horizon, int64_t seg_len, const ScoringConsts<R> k) {
+  constexpr int D = FamilyDim<R, FAMILY>::value;
+  constexpr bool kReadsObs = score_grad_reads_obs<FAMILY>();
+  constexpr bool kStage = score_grad_stages_rows<FAMILY>();
+  __shared__ alignas(16) R s_stage[kStage ? kBlock * D : 1];
+  R* s_warp = s_stage + (kStage ? (threadIdx.x >> 5) * 32 * D : 0);
+  const int64_t j = static_cast<int64_t>(blockIdx.x) * kBlock + threadIdx.x;  // env column
+  const int64_t r0 = static_cast<int64_t>(blockIdx.y) * seg_len;
+  // a full warp's 32 columns are 32 consecutive rows at every r, and its lanes walk the same rows
+  const bool warp_full = static_cast<int64_t>(blockIdx.x) * kBlock + (threadIdx.x | 31) < n_envs;
+  if (j >= n_envs || r0 > horizon) return;
+  const int64_t r1 = r0 + seg_len < horizon + 1 ? r0 + seg_len : horizon + 1;
+  R g_prev = r0 > 0 ? __ldg(g_reward + (r0 - 1) * n_envs + j) : R(0);
+  R g_cur = r0 < horizon ? __ldg(g_reward + r0 * n_envs + j) : R(0);
+  alignas(16) R o[D] = {}, nx[D] = {};
+  if constexpr (kReadsObs) load_row<R, D>(obs_seq, r0 * n_envs + j, o);
+  for (int64_t r = r0; r < r1; ++r) {
+    const bool more = r + 1 < r1;
+    R g_next = R(0);
+    if (more) {
+      if constexpr (kReadsObs) load_row<R, D>(obs_seq, (r + 1) * n_envs + j, nx);
+      if (r + 1 < horizon) g_next = __ldg(g_reward + (r + 1) * n_envs + j);
+    }
+    alignas(16) R go[D], unused[D];
+    R gp0, unused0;
+    score_row_grad<R, FAMILY, D>(o, g_prev, k, go, unused0);  // transition r - 1, whose obs is this row
+    if (r == 0) {
+#pragma unroll
+      for (int c = 0; c < D; ++c) go[c] = R(0);
+    }
+    if (r < horizon) {
+      score_row_grad<R, FAMILY, D>(o, g_cur, k, unused, gp0);  // transition r, whose pre_obs is this row
+      // one rounded add of the two rounded terms (no FMA contraction): the bits of the one-shot layout's two rows summed
+      if constexpr (sizeof(R) == 4)
+        go[0] = __fadd_rn(go[0], gp0);
+      else
+        go[0] = __dadd_rn(go[0], gp0);
+    }
+    store_grad_row<R, D, kStage>(g_obs_seq, r * n_envs + j, go, s_warp, warp_full);
+    g_prev = g_cur;
+    g_cur = g_next;
+#pragma unroll
+    for (int c = 0; c < D; ++c) o[c] = nx[c];
+  }
+}
+
+// g_action = -2 ctrl_w G action, G = the batch-wide sum of the reward cotangents: one scalar times the whole action tensor,
+// streamed flat with 128-bit accesses whatever the row width (12 / 24-byte float32 action rows)
+template <typename R>
+__global__ void __launch_bounds__(kBlock)
+    ctrl_cost_vjp_kernel(const R* __restrict__ action, const double* __restrict__ g_sum, R* __restrict__ g_action, int64_t n_elems,
+                         double ctrl_w) {
+  constexpr int V = 16 / sizeof(R);
+  const R c = static_cast<R>(-2.0 * ctrl_w * *g_sum);
+  const int64_t nvec = n_elems / V;
+  const int64_t j = static_cast<int64_t>(blockIdx.x) * kBlock + threadIdx.x;
+  if (j < nvec) {
+    uint4 q = __ldg(reinterpret_cast<const uint4*>(action) + j);
+    R* v = reinterpret_cast<R*>(&q);
+#pragma unroll
+    for (int e = 0; e < V; ++e) v[e] = c * v[e];
+    reinterpret_cast<uint4*>(g_action)[j] = q;
+  }
+  if (blockIdx.x == 0 && threadIdx.x < n_elems - nvec * V) {
+    const int64_t t = nvec * V + threadIdx.x;
+    g_action[t] = c * action[t];
+  }
+}
+
+// argument checks shared by both VJP entry points (after the size checks): the order and codes of reward_terminal
+template <typename R>
+int check_reward_vjp(const R* obs, const R* action, const R* g_reward, const double* g_reward_sum, const R* g_action,
+                     const emei_scoring_params* p) {
+  const bool mj = p->family == EMEI_HOPPER || p->family == EMEI_HALFCHEETAH;
+  const bool reads_obs = !mj && p->family != EMEI_CARTPOLE_BALANCING && p->family != EMEI_IP_REBOUND_BALANCING &&
+                         p->family != EMEI_IP_BOUNDARY_BALANCING && p->family != EMEI_I2P_REBOUND_BALANCING &&
+                         p->family != EMEI_I2P_BOUNDARY_BALANCING;
+  if (reads_obs) EMEI_CHECK_PTR(obs);
+  EMEI_CHECK_PTR(g_reward);
+  if (g_action != nullptr) {
+    if (!mj) return EMEI_ERR_BAD_PARAM;  // no other family's reward reads the action
+    EMEI_CHECK_PTR(action);
+    EMEI_CHECK_PTR(g_reward_sum);
+  }
+  if (reads_obs) EMEI_CHECK_ALIGN16(obs);
+  if (g_action != nullptr) {
+    EMEI_CHECK_ALIGN16(action);
+    EMEI_CHECK_ALIGN16(g_action);
+  }
+  return EMEI_OK;
+}
+
+template <typename R>
+void launch_ctrl_cost_vjp(const R* action, const double* g_reward_sum, R* g_action, int64_t n_elems, const ScoringConsts<R>& k,
+                          cudaStream_t s) {
+  constexpr int V = 16 / sizeof(R);
+  const int64_t nvec = n_elems / V;
+  const int grid = nvec > 0 ? grid_for(nvec, kBlock) : 1;
+  ctrl_cost_vjp_kernel<R><<<grid, kBlock, 0, s>>>(action, g_reward_sum, g_action, n_elems, static_cast<double>(k.ctrl_w));
+}
+
+#define EMEI_SCORING_FAMILIES(X)                                                                                          \
+  X(EMEI_CARTPOLE_BALANCING) X(EMEI_CARTPOLE_SWINGUP) X(EMEI_IP_REBOUND_BALANCING) X(EMEI_IP_BOUNDARY_BALANCING)         \
+  X(EMEI_IP_REBOUND_SWINGUP) X(EMEI_IP_BOUNDARY_SWINGUP) X(EMEI_I2P_REBOUND_BALANCING) X(EMEI_I2P_BOUNDARY_BALANCING)    \
+  X(EMEI_I2P_REBOUND_SWINGUP) X(EMEI_I2P_BOUNDARY_SWINGUP) X(EMEI_HOPPER) X(EMEI_HALFCHEETAH) X(EMEI_CHARGED_BALL)
+
+template <typename R>
+int reward_vjp(const R* obs, const R* action, const R* g_reward, const double* g_reward_sum, R* g_obs, R* g_pre_obs, R* g_action,
+               int64_t n, const emei_scoring_params* p, emei_stream_t stream) {
+  if (n < 0) return EMEI_ERR_BAD_SIZE;
+  EMEI_CHECK_PTR(p);
+  if (p->family < 0 || p->family >= EMEI_NUM_FAMILIES) return EMEI_ERR_BAD_VARIANT;
+  if ((p->family == EMEI_HOPPER || p->family == EMEI_HALFCHEETAH) && !(p->dt > 0.0)) return EMEI_ERR_BAD_PARAM;
+  if (n == 0) return EMEI_OK;
+  if (const int e = check_reward_vjp<R>(obs, action, g_reward, g_reward_sum, g_action, p)) return e;
+  if (g_obs != nullptr) EMEI_CHECK_ALIGN16(g_obs);
+  if (g_pre_obs != nullptr) EMEI_CHECK_ALIGN16(g_pre_obs);
+  const ScoringConsts<R> k = make_scoring_consts<R>(*p);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (g_obs != nullptr || g_pre_obs != nullptr) {
+    switch (p->family) {
+#define EMEI_CASE(F)                                                                                            \
+  case F:                                                                                                       \
+    reward_vjp_kernel<R, F><<<grid_for(n, kBlock), kBlock, 0, s>>>(obs, g_reward, g_obs, g_pre_obs, n, k); \
+    break;
+      EMEI_SCORING_FAMILIES(EMEI_CASE)
+#undef EMEI_CASE
+    }
+  }
+  if (g_action != nullptr) launch_ctrl_cost_vjp<R>(action, g_reward_sum, g_action, n * emei_family_action_dim(p->family), k, s);
+  return launch_status();
+}
+
+template <typename R>
+int reward_seq_vjp(const R* obs_seq, const R* action, const R* g_reward, const double* g_reward_sum, R* g_obs_seq, R* g_action,
+                   int64_t n_envs, int64_t horizon, const emei_scoring_params* p, emei_stream_t stream) {
+  if (n_envs < 0 || horizon < 0) return EMEI_ERR_BAD_SIZE;
+  EMEI_CHECK_PTR(p);
+  if (p->family < 0 || p->family >= EMEI_NUM_FAMILIES) return EMEI_ERR_BAD_VARIANT;
+  if ((p->family == EMEI_HOPPER || p->family == EMEI_HALFCHEETAH) && !(p->dt > 0.0)) return EMEI_ERR_BAD_PARAM;
+  if (n_envs == 0 || horizon == 0) return EMEI_OK;
+  EMEI_CHECK_PTR(g_obs_seq);
+  if (const int e = check_reward_vjp<R>(obs_seq, action, g_reward, g_reward_sum, g_action, p)) return e;
+  const int dim = emei_family_obs_dim(p->family);
+  // the rows of t >= 1 must keep the 16-byte alignment of the row accesses (as emei_reward_terminal_seq_*)
+  if ((static_cast<uint64_t>(n_envs) * dim * sizeof(R)) % 16 != 0) return EMEI_ERR_MISALIGNED;
+  EMEI_CHECK_ALIGN16(g_obs_seq);
+  const ScoringConsts<R> k = make_scoring_consts<R>(*p);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  // segments as the forward's walk: ~2^20 threads in flight, at least 8 rows each
+  const int64_t rows = horizon + 1;
+  int64_t segs = ((int64_t{1} << 20) + n_envs - 1) / n_envs;
+  const int64_t max_segs = (rows + 7) / 8;
+  if (segs > max_segs) segs = max_segs;
+  if (segs < 1) segs = 1;
+  if (segs > 65535) segs = 65535;
+  const int64_t seg_len = (rows + segs - 1) / segs;
+  segs = (rows + seg_len - 1) / seg_len;
+  const dim3 grid(static_cast<unsigned>(grid_for(n_envs, kBlock)), static_cast<unsigned>(segs), 1);
+  switch (p->family) {
+#define EMEI_CASE(F)                                                                                                      \
+  case F:                                                                                                                 \
+    reward_seq_vjp_kernel<R, F><<<grid, kBlock, 0, s>>>(obs_seq, g_reward, g_obs_seq, n_envs, horizon, seg_len, k); \
+    break;
+    EMEI_SCORING_FAMILIES(EMEI_CASE)
+#undef EMEI_CASE
+  }
+  if (g_action != nullptr)
+    launch_ctrl_cost_vjp<R>(action, g_reward_sum, g_action, horizon * n_envs * emei_family_action_dim(p->family), k, s);
+  return launch_status();
+}
+#undef EMEI_SCORING_FAMILIES
 
 // =============================================================================================
 // initial-state sampling (Philox4x32-10; value depends on (seed, env id, column) only)

@@ -450,13 +450,14 @@ def _aligned16(t: torch.Tensor) -> torch.Tensor:
     return t if t.data_ptr() % 16 == 0 else t.clone()
 
 
-def _sumsq(env, a: torch.Tensor, group):
-    """batch-wide sum of squared actions (hopper.py:98 / half_cheetah.py:61), all-reduced when the batch is sharded."""
+def _sumsq(env, a: torch.Tensor, group, entry="emei_sumsq"):
+    """batch-wide sum of squared actions (hopper.py:98 / half_cheetah.py:61), all-reduced when the batch is sharded.
+    ``entry="emei_sum"``: the plain sum (of the reward cotangents, for the control cost's derivative), same exchange."""
     sumsq = torch.empty(1, dtype=torch.float64, device=env.device)
     ws = getattr(env, "_sumsq_ws", None)
     if ws is None:  # zero-filled once; the kernel leaves its ticket counter at zero
         ws = env._sumsq_ws = torch.zeros(_lib.SUMSQ_WORKSPACE_BYTES // 8, dtype=torch.float64, device=env.device)
-    env._call("emei_sumsq", a.data_ptr(), a.numel(), sumsq.data_ptr(), ws.data_ptr(), env._stream())
+    env._call(entry, a.data_ptr(), a.numel(), sumsq.data_ptr(), ws.data_ptr(), env._stream())
     if getattr(env, "ctrl_cost_scope", "global") == "global":
         from .dist import all_reduce_sum_
 
@@ -472,48 +473,16 @@ def _score_cache_key(env, params, tensors, group):
     return (ident, bytes(params), env._stream(), id(group))
 
 
-def score(env, params: _lib.ScoringParams, obs, pre_obs=None, action=None, want="both", group=None):
-    """Fused get_batch_reward + get_batch_terminal through emei_reward_terminal_* for any batch size.
+def needs_grad(*tensors) -> bool:
+    """Does a scoring call on these tensors need a differentiable reward (grad mode on, an input requires grad)?"""
+    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors)
 
-    Hopper/HalfCheetah: pass 1 = emei_sumsq_* over the action batch (the reference sums the control
-    cost over the WHOLE batch, hopper.py:98 / half_cheetah.py:61), optional all-reduce of that one
-    double across ranks when the batch is sharded, pass 2 = the fused row kernel.  When ``pre_obs`` and
-    ``obs`` are the two shifted views of one trajectory tensor (``seq[:-1]`` / ``seq[1:]``) the C side
-    walks the trajectory and reads every observation row once (include/emei_b200.h).
 
-    The reference's API has two calls (get_batch_reward, get_batch_terminal: mujoco_env.py:163-169 callers);
-    a caller that makes them back to back on the SAME device tensors gets the second answer from the first
-    call's fused pass (one row pass instead of two).
-    Returns (reward [B,1] or None, done bool[B,1] or None, came_from_numpy)."""
-    family = params.family
-    o, was_np = env._to_device(obs, env.dtype)
-    if o.dim() != 2 or o.shape[1] != _lib.lib.emei_family_obs_dim(family):
-        raise ValueError(f"obs must be [B,{_lib.lib.emei_family_obs_dim(family)}], got {tuple(o.shape)}")
+def score_rows(env, params: _lib.ScoringParams, o: torch.Tensor, p, a, group):
+    """The kernels of one ``score`` pass on device rows: pass 1 (Hopper / HalfCheetah: emei_sumsq_*) and the fused row
+    kernel -> (reward [B,1], done bool [B,1]).  ``p`` / ``a`` None for Hopper / HalfCheetah: terminal only."""
     b = o.shape[0]
-    needs_pre = family in (_lib.HOPPER, _lib.HALFCHEETAH)
-    p = a = None
-    if needs_pre and (want != "terminal" or (pre_obs is not None and action is not None)):
-        if pre_obs is None or action is None:
-            raise TypeError("get_batch_reward of this env needs obs, pre_obs and action")
-        p, _ = env._to_device(pre_obs, env.dtype)
-        a, _ = env._to_device(action, env.dtype)
-        if tuple(p.shape) != tuple(o.shape) or a.shape[0] != b:
-            raise ValueError("obs / pre_obs / action batch shapes disagree")
-    # ---- the other half of a reward / terminal pair asked for on the same tensors: reuse the fused pass
-    # Only the COMPLEMENTARY half is ever served (reward after terminal, terminal after reward), once: repeating the
-    # same call, or get_batch_reward_terminal, always runs the kernels.
-    key = key_obs = None
-    if not was_np and want in ("reward", "terminal"):
-        key_obs = _score_cache_key(env, params, (o,), group)
-        if not needs_pre or p is not None:
-            key = _score_cache_key(env, params, (o, p, a), group)
-        hit = getattr(env, "_score_cache", None)
-        env._score_cache = None
-        if hit is not None and hit[2] == _lib.launch_count and hit[5] != want:
-            if key is not None and hit[0] == key:
-                return hit[3], hit[4], was_np
-            if key is None and want == "terminal" and hit[1] == key_obs:  # terminal with obs alone: the flags depend on obs only
-                return None, hit[4], was_np
+    needs_pre = params.family in (_lib.HOPPER, _lib.HALFCHEETAH)
     sumsq = None
     if needs_pre and p is not None:
         sumsq = _sumsq(env, _aligned16(a), group)
@@ -532,7 +501,59 @@ def score(env, params: _lib.ScoringParams, obs, pre_obs=None, action=None, want=
         env.stats.data_ptr() if getattr(env, "accumulate_scoring_stats", False) else None,
         sumsq.data_ptr() if sumsq is not None else None, b, ctypes.byref(params), env._stream(),
     )
-    done = done.view(torch.bool)
+    return reward, done.view(torch.bool)
+
+
+def score(env, params: _lib.ScoringParams, obs, pre_obs=None, action=None, want="both", group=None):
+    """Fused get_batch_reward + get_batch_terminal through emei_reward_terminal_* for any batch size.
+
+    Hopper/HalfCheetah: pass 1 = emei_sumsq_* over the action batch (the reference sums the control
+    cost over the WHOLE batch, hopper.py:98 / half_cheetah.py:61), optional all-reduce of that one
+    double across ranks when the batch is sharded, pass 2 = the fused row kernel.  When ``pre_obs`` and
+    ``obs`` are the two shifted views of one trajectory tensor (``seq[:-1]`` / ``seq[1:]``) the C side
+    walks the trajectory and reads every observation row once (include/emei_b200.h).
+
+    The reference's API has two calls (get_batch_reward, get_batch_terminal: mujoco_env.py:163-169 callers);
+    a caller that makes them back to back on the SAME device tensors gets the second answer from the first
+    call's fused pass (one row pass instead of two).
+    With grad mode on and ``obs``, ``pre_obs`` or ``action`` requiring grad, the reward is recorded in the autograd graph
+    (``autodiff.RewardScore``: same kernels forward, emei_reward_vjp_* backward) and never served from that cache.
+    Returns (reward [B,1] or None, done bool[B,1] or None, came_from_numpy)."""
+    family = params.family
+    o, was_np = env._to_device(obs, env.dtype)
+    if o.dim() != 2 or o.shape[1] != _lib.lib.emei_family_obs_dim(family):
+        raise ValueError(f"obs must be [B,{_lib.lib.emei_family_obs_dim(family)}], got {tuple(o.shape)}")
+    b = o.shape[0]
+    needs_pre = family in (_lib.HOPPER, _lib.HALFCHEETAH)
+    p = a = None
+    if needs_pre and (want != "terminal" or (pre_obs is not None and action is not None)):
+        if pre_obs is None or action is None:
+            raise TypeError("get_batch_reward of this env needs obs, pre_obs and action")
+        p, _ = env._to_device(pre_obs, env.dtype)
+        a, _ = env._to_device(action, env.dtype)
+        if tuple(p.shape) != tuple(o.shape) or a.shape[0] != b:
+            raise ValueError("obs / pre_obs / action batch shapes disagree")
+    if want != "terminal" and needs_grad(o, p, a):  # a differentiable reward: never served from the cache below
+        from .autodiff import RewardScore
+
+        reward, done = RewardScore.apply(o, p, a, env, params, group)
+        return reward, done, was_np
+    # ---- the other half of a reward / terminal pair asked for on the same tensors: reuse the fused pass
+    # Only the COMPLEMENTARY half is ever served (reward after terminal, terminal after reward), once: repeating the
+    # same call, or get_batch_reward_terminal, always runs the kernels.
+    key = key_obs = None
+    if not was_np and want in ("reward", "terminal"):
+        key_obs = _score_cache_key(env, params, (o,), group)
+        if not needs_pre or p is not None:
+            key = _score_cache_key(env, params, (o, p, a), group)
+        hit = getattr(env, "_score_cache", None)
+        env._score_cache = None
+        if hit is not None and hit[2] == _lib.launch_count and hit[5] != want:
+            if key is not None and hit[0] == key:
+                return hit[3], hit[4], was_np
+            if key is None and want == "terminal" and hit[1] == key_obs:  # terminal with obs alone: the flags depend on obs only
+                return None, hit[4], was_np
+    reward, done = score_rows(env, params, o, p, a, group)
     if key is not None and not getattr(env, "accumulate_scoring_stats", False):
         env._score_cache = (key, key_obs, _lib.launch_count, reward, done, want)
     return reward, done, was_np
@@ -541,7 +562,8 @@ def score(env, params: _lib.ScoringParams, obs, pre_obs=None, action=None, want=
 def score_seq(env, params: _lib.ScoringParams, obs_seq, action=None, group=None):
     """Trajectory scoring through emei_reward_terminal_seq_*: ``obs_seq`` [T+1, n, D] (an imagined rollout),
     ``action`` [T, n, A] -> reward [T, n, 1], done bool [T, n, 1].  Equal to ``score`` on
-    ``obs = obs_seq[1:], pre_obs = obs_seq[:-1]`` flattened; every observation row is read once."""
+    ``obs = obs_seq[1:], pre_obs = obs_seq[:-1]`` flattened; every observation row is read once.  Differentiable like
+    ``score`` (``autodiff.RewardScoreSeq``, backward emei_reward_seq_vjp_*)."""
     family = params.family
     s, was_np = env._to_device(obs_seq, env.dtype)
     d = _lib.lib.emei_family_obs_dim(family)
@@ -549,7 +571,7 @@ def score_seq(env, params: _lib.ScoringParams, obs_seq, action=None, group=None)
         raise ValueError(f"obs_seq must be [T+1, n, {d}], got {tuple(s.shape)}")
     T, n = s.shape[0] - 1, s.shape[1]
     needs_pre = family in (_lib.HOPPER, _lib.HALFCHEETAH)
-    a = sumsq = None
+    a = None
     if needs_pre:
         if action is None:
             raise TypeError("get_batch_reward of this env needs the actions")
@@ -561,7 +583,21 @@ def score_seq(env, params: _lib.ScoringParams, obs_seq, action=None, group=None)
         r, dn, _ = score(env, params, s[1:].reshape(T * n, d), s[:-1].reshape(T * n, d).clone(),
                          a.reshape(T * n, -1) if needs_pre else None, group=group)
         return r.reshape(T, n, 1), dn.reshape(T, n, 1), was_np
-    if needs_pre:
+    if needs_grad(s, a):
+        from .autodiff import RewardScoreSeq
+
+        reward, done = RewardScoreSeq.apply(s, a, env, params, group)
+        return reward, done, was_np
+    reward, done = score_seq_rows(env, params, s, a, group)
+    return reward, done, was_np
+
+
+def score_seq_rows(env, params: _lib.ScoringParams, s: torch.Tensor, a, group):
+    """The kernels of one ``score_seq`` pass on a device trajectory s [T+1, n, D] whose rows keep 16-byte alignment:
+    pass 1 (Hopper / HalfCheetah: emei_sumsq_* over a) and emei_reward_terminal_seq_* -> (reward [T,n,1], done bool [T,n,1])."""
+    T, n = s.shape[0] - 1, s.shape[1]
+    sumsq = None
+    if params.family in (_lib.HOPPER, _lib.HALFCHEETAH):
         sumsq = _sumsq(env, _aligned16(a), group)
     s = _aligned16(s)
     reward = torch.empty((T, n, 1), dtype=env.dtype, device=env.device)
@@ -571,7 +607,7 @@ def score_seq(env, params: _lib.ScoringParams, obs_seq, action=None, group=None)
         env.stats.data_ptr() if getattr(env, "accumulate_scoring_stats", False) else None,
         sumsq.data_ptr() if sumsq is not None else None, n, T, ctypes.byref(params), env._stream(),
     )
-    return reward, done.view(torch.bool), was_np
+    return reward, done.view(torch.bool)
 
 
 ZERO_COPY_MAX_ENVS = 65536  # measured: scripts/probe_zero_copy_small.py, profiles/r02_zero_copy_small.txt

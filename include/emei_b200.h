@@ -410,6 +410,45 @@ int emei_reward_terminal_seq_f64(const double* obs_seq, double* reward, uint8_t*
 #define EMEI_SUMSQ_WORKSPACE_BYTES ((148 * 8 + 1) * 8)
 int emei_sumsq_f32(const float* x, int64_t n_elems, double* out, double* workspace, emei_stream_t stream);
 int emei_sumsq_f64(const double* x, int64_t n_elems, double* out, double* workspace, emei_stream_t stream);
+/* the plain sum of n_elems values: the reduction of emei_sumsq_* without the square, same workspace contract and the same
+ * run-to-run bits (the batch-wide sum of the reward cotangents that the control cost's derivative needs). */
+int emei_sum_f32(const float* x, int64_t n_elems, double* out, double* workspace, emei_stream_t stream);
+int emei_sum_f64(const double* x, int64_t n_elems, double* out, double* workspace, emei_stream_t stream);
+
+/* ---- derivatives of the scoring (vector-Jacobian products) ---------------------------------------
+ * What is differentiated: the real-valued reward emei_reward_terminal_* evaluates on the caller's rows, almost everywhere.
+ * `done` and Hopper's healthy term are piecewise constant: no gradient.  Per family (o = obs row, p = pre_obs row):
+ *   cart-pole balancing, IP / I2P balancing : constant reward, zero gradient
+ *   cart-pole swing-up    : d/do2 = -sin(o2)/2          IP swing-ups: d/do1 = sin(o1)/2
+ *   I2P swing-ups         : d/do1 = (sin o1 + sin(o1+o2))/4, d/do2 = sin(o1+o2)/4; boundary also d/do4 = -1e-2 o4, d/do5 = -2e-4 o5
+ *   Hopper, HalfCheetah   : d/do0 = fwd_w/dt, d/dp0 = -fwd_w/dt, d/da = -2 ctrl_w a summed over EVERY reward of the batch:
+ *                           g_action = -2 ctrl_w G action with G = sum of the reward cotangents (emei_sum_*; all-reduced by
+ *                           the caller when the control cost is global over a sharded batch)
+ *   charged ball          : d/do0,1 = -o0,1 / (radius rho), rho = sqrt(o0^2 + o1^2); 0 at rho = 0
+ * _f32 evaluates these in float32 (a tolerance product).  Non-finite inputs give non-finite gradients where the derivative
+ * reads them.  Validation: n < 0 (n_envs, horizon < 0) -> EMEI_ERR_BAD_SIZE; then the checks of emei_reward_terminal_*
+ * in its order (params, family -> EMEI_ERR_BAD_VARIANT, Hopper / HalfCheetah dt <= 0 -> EMEI_ERR_BAD_PARAM); n == 0 or
+ * horizon == 0 is a no-op.  obs may be NULL only for the families whose gradient does not read it (the constant rewards,
+ * Hopper, HalfCheetah); g_reward is required; a non-NULL g_action needs action and g_reward_sum and is rejected
+ * (EMEI_ERR_BAD_PARAM) for the families whose reward does not read the action.  obs, action, every gradient array: 16-byte
+ * aligned. */
+/* VJP of emei_reward_terminal_*: g_reward [n] ; g_reward_sum DEVICE double* = G ; g_obs [n,D], g_pre_obs [n,D] (dense rows),
+ * g_action [n,A] (A = emei_family_action_dim): each nullable (not written). */
+int emei_reward_vjp_f32(const float* obs, const float* action, const float* g_reward, const double* g_reward_sum, float* g_obs,
+                        float* g_pre_obs, float* g_action, int64_t n, const emei_scoring_params* p, emei_stream_t stream);
+int emei_reward_vjp_f64(const double* obs, const double* action, const double* g_reward, const double* g_reward_sum,
+                        double* g_obs, double* g_pre_obs, double* g_action, int64_t n, const emei_scoring_params* p,
+                        emei_stream_t stream);
+/* VJP of emei_reward_terminal_seq_*: obs_seq [horizon+1,n_envs,D] ; g_reward [horizon,n_envs] ;
+ * g_obs_seq [horizon+1,n_envs,D] (required, every row written once): row t = d/d obs of transition t-1 + d/d pre_obs of
+ * transition t ; g_action [horizon,n_envs,A] nullable, G summed over all horizon * n_envs rewards.
+ * n_envs * D * sizeof(real) must be a multiple of 16 (as for emei_reward_terminal_seq_*). */
+int emei_reward_seq_vjp_f32(const float* obs_seq, const float* action, const float* g_reward, const double* g_reward_sum,
+                            float* g_obs_seq, float* g_action, int64_t n_envs, int64_t horizon, const emei_scoring_params* p,
+                            emei_stream_t stream);
+int emei_reward_seq_vjp_f64(const double* obs_seq, const double* action, const double* g_reward, const double* g_reward_sum,
+                            double* g_obs_seq, double* g_action, int64_t n_envs, int64_t horizon, const emei_scoring_params* p,
+                            emei_stream_t stream);
 
 /* ---- batched initial-state sampling (counter-based Philox4x32-10; see DESIGN.md) -------------- */
 /* value(env, column) depends only on (seed, env_offset + row, column): independent of sharding. */
