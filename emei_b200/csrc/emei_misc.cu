@@ -51,12 +51,69 @@ __global__ void __launch_bounds__(kBlock) records_transpose_kernel(const E* __re
   }
 }
 
+// Wide elements (observation rows of 24, 32 or 48 bytes: 6 x float32, 4 x float64, 6 x float64) moved as K words W
+// (uint2 for 24 bytes, which a [T, n, 6] float32 tensor only aligns to 8; uint4 otherwise).  A 32 x 32 tile of 48-byte
+// elements is 50.7 KB, over the 48 KB of static shared memory, so the tile is 16 steps x 32 envs (25.3 KB at 48 bytes).
+// It stays coalesced both ways because an element is wide: a tile row read is 32 contiguous elements of in (768 to
+// 1536 bytes) and a tile row written is 16 contiguous elements of out (384 to 768 bytes), each taken by consecutive
+// threads word after word.  The shared rows are padded by one element ((32 + 1) * K words), so that the row stride is
+// K words modulo the bank width: in both phases consecutive threads touch consecutive banks.
+constexpr int kWideTileT = 16, kWideTileN = 32;
+
+template <typename W, int K>
+__global__ void __launch_bounds__(kBlock) records_transpose_wide_kernel(const W* __restrict__ in, W* __restrict__ out, int64_t T,
+                                                                        int64_t n, int64_t tiles_n, int64_t tiles) {
+  constexpr int kRow = (kWideTileN + 1) * K;  // words per shared row (one time step of the tile)
+  constexpr int kIn = kWideTileN * K;         // words per tile row read from in (one time step)
+  constexpr int kOut = kWideTileT * K;        // words per tile row written to out (one env)
+  constexpr int kWords = kWideTileT * kWideTileN * K;
+  static_assert(kWords % kBlock == 0, "whole passes over the tile");
+  __shared__ W tile[kWideTileT][kRow];
+  for (int64_t tl = blockIdx.x; tl < tiles; tl += gridDim.x) {
+    const int64_t t0 = (tl / tiles_n) * kWideTileT, i0 = (tl % tiles_n) * kWideTileN;
+#pragma unroll
+    for (int p = 0; p < kWords / kBlock; ++p) {
+      const int j = p * kBlock + threadIdx.x;
+      const int r = j / kIn, w = j % kIn;  // step r of the tile, word w of its row = word w % K of env w / K
+      const int64_t t = t0 + r;
+      if (t < T && i0 + w / K < n) tile[r][w] = in[(t * n + i0) * K + w];
+    }
+    __syncthreads();
+#pragma unroll
+    for (int p = 0; p < kWords / kBlock; ++p) {
+      const int j = p * kBlock + threadIdx.x;
+      const int c = j / kOut, w = j % kOut;  // env c of the tile, word w of its row = word w % K of step w / K
+      const int64_t i = i0 + c;
+      if (t0 + w / K < T && i < n) out[(i * T + t0) * K + w] = tile[w / K][c * K + w % K];
+    }
+    __syncthreads();
+  }
+}
+
 template <typename E>
 inline void launch_records_transpose(const void* in, void* out, int64_t T, int64_t n, cudaStream_t s) {
   const int64_t tiles_n = (n + 31) / 32, tiles = tiles_n * ((T + 31) / 32);
   const int64_t cap = static_cast<int64_t>(kNumSMs) * 8;
   const int grid = static_cast<int>(tiles < cap ? tiles : cap);
   records_transpose_kernel<E><<<grid, kBlock, 0, s>>>(static_cast<const E*>(in), static_cast<E*>(out), T, n, tiles_n, tiles);
+}
+
+template <typename W, int K>
+inline void launch_records_transpose_wide(const void* in, void* out, int64_t T, int64_t n, cudaStream_t s) {
+  const int64_t tiles_n = (n + kWideTileN - 1) / kWideTileN, tiles = tiles_n * ((T + kWideTileT - 1) / kWideTileT);
+  const int64_t cap = static_cast<int64_t>(kNumSMs) * 8;
+  const int grid = static_cast<int>(tiles < cap ? tiles : cap);
+  records_transpose_wide_kernel<W, K><<<grid, kBlock, 0, s>>>(static_cast<const W*>(in), static_cast<W*>(out), T, n, tiles_n, tiles);
+}
+
+// the alignment a record element of elem_bytes needs (that of the words it is moved in); 0: not a record element size
+inline int records_elem_align(int32_t elem_bytes) {
+  switch (elem_bytes) {
+    case 1: case 4: case 8: case 16: return elem_bytes;
+    case 24: return 8;
+    case 32: case 48: return 16;
+    default: return 0;
+  }
 }
 
 }  // namespace emei
@@ -66,18 +123,22 @@ extern "C" {
 int emei_records_transpose(const void* in, void* out, int64_t horizon, int64_t n, int32_t elem_bytes, emei_stream_t stream) {
   using namespace emei;
   if (horizon < 0 || n < 0) return EMEI_ERR_BAD_SIZE;
-  if (elem_bytes != 1 && elem_bytes != 4 && elem_bytes != 8 && elem_bytes != 16) return EMEI_ERR_BAD_PARAM;
+  const int align = records_elem_align(elem_bytes);
+  if (align == 0) return EMEI_ERR_BAD_PARAM;
   if (horizon == 0 || n == 0) return EMEI_OK;
   EMEI_CHECK_PTR(in);
   EMEI_CHECK_PTR(out);
-  if (((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) & static_cast<uintptr_t>(elem_bytes - 1)) != 0)
+  if (((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) & static_cast<uintptr_t>(align - 1)) != 0)
     return EMEI_ERR_MISALIGNED;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   switch (elem_bytes) {
     case 1: launch_records_transpose<uint8_t>(in, out, horizon, n, s); break;
     case 4: launch_records_transpose<uint32_t>(in, out, horizon, n, s); break;
     case 8: launch_records_transpose<uint2>(in, out, horizon, n, s); break;
-    default: launch_records_transpose<uint4>(in, out, horizon, n, s); break;
+    case 16: launch_records_transpose<uint4>(in, out, horizon, n, s); break;
+    case 24: launch_records_transpose_wide<uint2, 3>(in, out, horizon, n, s); break;
+    case 32: launch_records_transpose_wide<uint4, 2>(in, out, horizon, n, s); break;
+    default: launch_records_transpose_wide<uint4, 3>(in, out, horizon, n, s); break;
   }
   return launch_status();
 }

@@ -34,8 +34,8 @@ def _transpose(t: torch.Tensor, stream) -> torch.Tensor:
     elem = src.element_size()
     for d in src.shape[2:]:
         elem *= int(d)
-    if elem not in (1, 4, 8, 16):
-        raise ValueError(f"record element of {elem} bytes is not a dataset record (1, 4, 8 or 16 bytes)")
+    if elem not in (1, 4, 8, 16, 24, 32, 48):
+        raise ValueError(f"record element of {elem} bytes is not a dataset record (1, 4, 8, 16, 24, 32 or 48 bytes)")
     out = torch.empty((n, T) + tuple(src.shape[2:]), dtype=src.dtype, device=src.device)
     with torch.cuda.device(src.device):
         _lib.call("emei_records_transpose", src.data_ptr(), out.data_ptr(), T, n, elem, stream)

@@ -479,8 +479,10 @@ int emei_snapshot_copy(void* dst, const void* src, int64_t bytes, emei_stream_t 
  * The reference writes its offline datasets episode after episode (zoo/util.py:33-93,108-111: flat arrays
  * observations, next_observations, actions, rewards, dones, timeouts).  The fused rollouts record time-major
  * [horizon, n] arrays; this transposes one of them to env-major [n, horizon] (each env's trajectory, hence each
- * of its episodes, contiguous).  elem_bytes: 1 (dones, timeouts, uint8 actions), 4 (rewards, float/int32 actions),
- * 8 (int64/double actions), 16 (observation rows).  in/out aligned to elem_bytes. */
+ * of its episodes, contiguous).  elem_bytes: 1 (dones, timeouts, uint8 actions), 4 (float32 rewards, float/int32
+ * actions), 8 (float64 rewards, int64/double actions), 16 (float32 observation rows of 4), 24 (float32 rows of 6: the
+ * inverted double pendulum), 32 (float64 rows of 4), 48 (float64 rows of 6); any other size is EMEI_ERR_BAD_PARAM.
+ * in/out aligned to elem_bytes for 1, 4, 8 and 16, to 8 for 24 and to 16 for 32 and 48 (else EMEI_ERR_MISALIGNED). */
 int emei_records_transpose(const void* in, void* out, int64_t horizon, int64_t n, int32_t elem_bytes, emei_stream_t stream);
 
 /* ---- statistics --------------------------------------------------------------------------------- */

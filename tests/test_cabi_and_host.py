@@ -194,9 +194,24 @@ def test_rollout_and_transpose_validation_codes():
     _check_rollout_validation_table()
     t = lib.emei_records_transpose
     assert t(None, None, 4, -1, 4, None) == -4
-    assert t(None, None, 4, 8, 3, None) == -6          # element sizes: 1, 4, 8, 16
+    assert t(None, None, 4, 8, 3, None) == -6          # element sizes: 1, 4, 8, 16, 24, 32, 48
+    for bad in (3, 12, 20, 64):
+        assert t(None, None, 4, 8, bad, None) == -6, bad
     assert t(None, None, 0, 8, 4, None) == 0
     assert t(None, None, 4, 8, 4, None) == -1
+    # the wide observation rows (6 x float32, 4 x float64, 6 x float64): null pointers, then the alignment of the words
+    # they move in (8 bytes for 24, 16 for 32 and 48).  A misaligned address is refused before anything is launched, so
+    # these calls need no device; every call here has a null or a misaligned pointer and never launches.
+    base = 1 << 20
+    for eb in (24, 32, 48):
+        assert t(None, None, 0, 8, eb, None) == 0
+        assert t(None, None, 3, 5, eb, None) == -1, eb
+        assert t(base, None, 3, 5, eb, None) == -1, eb
+        assert t(None, base, 3, 5, eb, None) == -1, eb
+    for eb, off in ((24, 4), (24, 12), (32, 8), (32, 4), (48, 8), (48, 4)):
+        assert t(base + off, base, 3, 5, eb, None) == -5, (eb, off)
+        assert t(base, base + off, 3, 5, eb, None) == -5, (eb, off)
+    assert t(base + 8, base + 4, 3, 5, 24, None) == -5  # 8 bytes suffice for in, not 4 for out
 
 
 def test_offline_dataset_files_roundtrip(tmp_path, monkeypatch):
@@ -231,6 +246,21 @@ def test_offline_dataset_files_roundtrip(tmp_path, monkeypatch):
     except ImportError:
         with pytest.raises(ImportError):
             offline.save_dataset(ds, tmp_path / "x.h5")
+    # float64 rows (the reference-exact mode) and 6-wide rows (the inverted double pendulum, Box actions [N, 1]) keep
+    # their dtypes, shapes and bits through the file
+    for env_id, dim, dt in (("CartPoleSwingUp-v0", 4, np.float64), ("BoundaryInvertedDoublePendulumSwingUp-v0", 6, np.float32),
+                            ("ReboundInvertedDoublePendulumBalancing-v0", 6, np.float64)):
+        wide = dict(observations=rng.normal(size=(n, dim)).astype(dt), next_observations=rng.normal(size=(n, dim)).astype(dt),
+                    actions=(rng.integers(0, 2, n) if dim == 4 else rng.uniform(-1, 1, (n, 1)).astype(np.float32)),
+                    rewards=rng.normal(size=n).astype(dt), dones=(rng.random(n) < 0.1).astype(np.float32),
+                    timeouts=(rng.random(n) < 0.05).astype(np.float32))
+        env = E.make(env_id)
+        path = offline.save_dataset(wide, offline.dataset_path(env, "wide"))
+        assert path.suffix == ".npz" and env.dataset_names == ["wide.npz"]
+        back = env.get_dataset("wide.npz")
+        assert sorted(back) == sorted(wide)
+        for k in wide:
+            assert back[k].dtype == wide[k].dtype and back[k].shape == wide[k].shape and np.array_equal(back[k], wide[k]), (env_id, k)
 
 
 def test_env_params_name(golden):

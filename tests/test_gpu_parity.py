@@ -1212,17 +1212,27 @@ def test_step_kernel_large_batches_equal_scalar_rollout(env_id, cont, n):
 # ================================================================================================
 # rollout records -> the reference's dataset order (zoo/util.py:33-93,108-111)
 # ================================================================================================
-@pytest.mark.parametrize("T,n", ((1, 1), (37, 1000), (64, 33), (5, 4097)))
+@pytest.mark.parametrize("T,n", ((1, 1), (37, 1000), (64, 33), (5, 4097),
+                                 (1, 1000), (1000, 1), (45, 77),   # one step, one env; neither dimension a multiple of 16 or 32
+                                 (257, 40001)))                    # more tiles than the 148 x 8 CTAs of the grid: grid-stride loop
 def test_records_transpose_bit_exact(T, n):
-    from emei_b200 import offline
+    """every record element size: 1, 4, 8, 16 and the wide observation rows of 24 (6 x float32), 32 (4 x float64) and
+    48 bytes (6 x float64), through the C ABI and through offline._transpose"""
+    from emei_b200 import _lib, offline
 
     g = torch.Generator(device="cuda")
     g.manual_seed(T * 7919 + n)
     stream = torch.cuda.current_stream().cuda_stream
-    for shape, dtype in (((T, n, 4), torch.float32), ((T, n), torch.float32), ((T, n), torch.uint8), ((T, n), torch.int64), ((T, n), torch.bool)):
+    for shape, dtype in (((T, n, 4), torch.float32), ((T, n), torch.float32), ((T, n), torch.uint8), ((T, n), torch.int64), ((T, n), torch.bool),
+                         ((T, n), torch.float64), ((T, n, 6), torch.float32), ((T, n, 4), torch.float64), ((T, n, 6), torch.float64)):
         x = torch.randint(0, 250, shape, device="cuda", generator=g).to(dtype)
+        want = x.transpose(0, 1).contiguous()
+        elem = x.element_size() * (shape[2] if len(shape) > 2 else 1)
+        out = torch.empty_like(want)
+        assert _lib.lib.emei_records_transpose(x.data_ptr(), out.data_ptr(), T, n, elem, stream) == 0, f"{elem}-byte elements"
+        assert torch.equal(out, want), f"{elem}-byte elements"
         y = offline._transpose(x, stream)
-        assert y.dtype == x.dtype and torch.equal(y, x.transpose(0, 1).contiguous())
+        assert y.dtype == x.dtype and torch.equal(y, want)
 
 
 @pytest.mark.parametrize("env_id", ("CartPoleSwingUp-v0", "ContinuousChargedBallCentering-v0"))
