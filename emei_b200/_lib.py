@@ -5,7 +5,7 @@ raises, and every op raises ``EmeiB200Error`` on a non-zero return code.
 """
 import ctypes
 import os
-from ctypes import POINTER, Structure, c_char_p, c_double, c_int, c_int32, c_int64, c_uint64, c_void_p
+from ctypes import POINTER, Structure, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_uint64, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "csrc", "libemei_b200.so")
@@ -30,6 +30,8 @@ ACTION_DISCRETE_U8, ACTION_DISCRETE_I32, ACTION_DISCRETE_I64, ACTION_CONTINUOUS_
 
 
 SUMSQ_WORKSPACE_BYTES = (148 * 8 + 1) * 8  # EMEI_SUMSQ_WORKSPACE_BYTES
+PLAN_CEM, PLAN_MPPI = 0, 1  # EMEI_PLAN_*
+PLAN_MAX_CANDIDATES = 4096  # EMEI_PLAN_MAX_CANDIDATES
 
 
 class EmeiB200Error(RuntimeError):
@@ -124,6 +126,22 @@ class RolloutParams(Structure):
     ]
 
 
+class PlanParams(Structure):
+    _fields_ = [
+        ("seed", c_uint64),
+        ("env_offset", c_uint64),
+        ("gamma", c_double),
+        ("temperature", c_double),
+        ("momentum", c_double),
+        ("min_std", c_double),
+        ("action_low", c_float),
+        ("action_high", c_float),
+        ("method", c_int32),
+        ("elites", c_int32),
+        ("action_kind", c_int32),
+    ]
+
+
 _P = c_void_p
 _PROTOTYPES = {
     # name: (restype, argtypes)
@@ -138,6 +156,10 @@ _PROTOTYPES = {
     "emei_cartpole_trajectory_vjp": (c_int, [_P] * 7 + [c_int64, c_int64, POINTER(CartPoleParams), _P]),
     "emei_i2p_trajectory": (c_int, [_P] * 6 + [c_int64, c_int64, POINTER(I2PParams), _P]),
     "emei_i2p_trajectory_vjp": (c_int, [_P] * 7 + [c_int64, c_int64, POINTER(I2PParams), _P]),
+    "emei_cartpole_plan_eval": (c_int, [_P] * 5 + [c_int64] * 3 + [POINTER(PlanParams), POINTER(CartPoleParams), _P]),
+    "emei_i2p_plan_eval": (c_int, [_P] * 5 + [c_int64] * 3 + [POINTER(PlanParams), POINTER(I2PParams), _P]),
+    "emei_charged_ball_plan_eval": (c_int, [_P] * 7 + [c_int64] * 3 + [POINTER(PlanParams), POINTER(ChargedBallParams), _P]),
+    "emei_plan_update": (c_int, [_P] * 5 + [c_int64] * 3 + [POINTER(PlanParams), _P]),
     "emei_ip_step_noisy": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64, POINTER(CartPoleParams), POINTER(NoiseParams), _P]),
     "emei_i2p_step_noisy": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64, POINTER(I2PParams), POINTER(NoiseParams), _P]),
     "emei_cartpole_rollout_ref": (c_int, [_P] * 12 + [c_int64, POINTER(CartPoleParams), POINTER(RolloutParams), POINTER(NoiseParams), _P]),

@@ -9,6 +9,7 @@ written against the reference's ``get_batch_*`` keeps working unchanged.
 (``emei_b200.offline``); the download step (``urllib``, core.py:94-107) is out of scope -- there is no network --
 so ``dataset_names`` lists what is on disk and ``get_dataset`` raises for anything that is not.
 """
+from collections import namedtuple
 from typing import Dict, Union
 
 import numpy as np
@@ -32,6 +33,18 @@ class Freezable:
     def unfreeze(self):
         assert self.frozen, "env has unfrozen"
         self.frozen = False
+
+PlanResult = namedtuple("PlanResult", "mean std best_actions best_return returns")
+PlanResult.__doc__ = """Result of ``EmeiEnv.plan``: the refitted plan distribution ``mean`` / ``std`` [H, B] (``std`` None for discrete
+actions, whose ``mean`` is the probability of action 1), the best candidate of the last iteration (``best_actions`` [H, B],
+``best_return`` [B] float64) and that iteration's ``returns`` [B, K] (float64)."""
+
+_M64 = 0xFFFFFFFFFFFFFFFF
+
+
+def plan_iteration_seed(seed: int, i: int) -> int:
+    """The Philox key of iteration ``i`` of a plan keyed by ``seed``."""
+    return (seed * 0xD1B54A32D192ED03 + (i + 1) * 0x9E3779B97F4A7C15) & _M64
 
 
 def _torch_dtype(dtype) -> torch.dtype:
@@ -70,6 +83,7 @@ class EmeiEnv(Freezable):
         self._stats = None
         self._seed = 0
         self._reset_count = 0
+        self._plan_count = 0  # planner calls since the last explicit seed: keys plan() / get_batch_plan_returns with seed=None
         self._rollout_epoch = -1  # resets since the last explicit seed (0 = the seeded one): keys the rollout / noise streams
 
     # ------------------------------------------------------------------ engine protocol (engine.py)
@@ -229,6 +243,92 @@ class EmeiEnv(Freezable):
         actions [T,B]: the analytic families only."""
         raise NotImplementedError(f"{type(self).__name__}: no gradients, {self._no_derivatives}")
 
+    # ------------------------------------------------------------------ sampling-based planning (CEM / MPPI)
+    def _plan_setup(self, state):
+        """-> (engine, device start states, B, came_from_numpy, PlanParams with the action kind, box and env_offset)."""
+        eng = self._ensure_engine()
+        if eng is None or not hasattr(eng, "plan_eval"):
+            raise NotImplementedError(f"{type(self).__name__}: no planning, it has no dynamics kernel")
+        if state is None:
+            assert self.state is not None, "Call reset before planning from the env's state."
+            state = self.state
+        start, b, was_np = eng.plan_start(state)
+        q = _lib.PlanParams()
+        q.env_offset = int(getattr(self, "env_offset", 0))
+        q.method, q.elites, q.temperature = _lib.PLAN_CEM, 1, 1.0
+        if len(self.action_space.shape) == 0:
+            q.action_kind = _lib.ACTION_DISCRETE_U8
+        else:
+            q.action_kind = _lib.ACTION_CONTINUOUS_F32 if self.dtype == torch.float32 else _lib.ACTION_CONTINUOUS_F64
+            q.action_low, q.action_high = float(self.action_space.low.min()), float(self.action_space.high.max())
+        return eng, start, b, was_np, q
+
+    def _plan_table(self, x, b: int, what: str, horizon=None) -> torch.Tensor:
+        """mean / std as a fresh contiguous device tensor [H, B] in the env dtype ([H] is broadcast over the starts)."""
+        t, _ = self._to_device(x, self.dtype)
+        if t.dim() == 1:
+            t = t.reshape(-1, 1).expand(t.shape[0], b)
+        if t.dim() != 2 or t.shape[1] != b or (horizon is not None and t.shape[0] != horizon):
+            raise ValueError(f"{what} must be [H, B={b}] or [H], got {tuple(t.shape)}")
+        return t.clone(memory_format=torch.contiguous_format)
+
+    def get_batch_plan_returns(self, state, mean, std, candidates: int, seed=None, gamma: float = 1.0, return_actions: bool = False):
+        """Score ``candidates`` action sequences per start state in one launch: candidate k of start b draws its actions
+        around ``mean`` / ``std`` [H, B] (discrete actions: ``mean`` is the probability of action 1, ``std`` is unused) from
+        the counter-based stream of (``seed``, start, k) and is rolled out open-loop for H steps with the step arithmetic of
+        ``rollout()``.  -> ``returns`` [B, K] float64, the discounted sum of rewards up to and including the step that
+        terminates; with ``return_actions`` also the actions [H, B, K] (``actions.view(H, B*K)`` teacher-forces a rollout of
+        the candidates).  ``state``: start rows [B, D] (qpos || qvel, angles unwrapped, for the pendulums) or the charged
+        ball's state dict; ``seed=None`` draws a fresh key from the env's seed and a planner call counter of its own.  The
+        env's state, statistics and initial-state stream are not touched."""
+        eng, start, b, was_np, q = self._plan_setup(state)
+        discrete = q.action_kind == _lib.ACTION_DISCRETE_U8
+        m = self._plan_table(mean, b, "mean")
+        s = None if discrete else self._plan_table(std, b, "std", m.shape[0])
+        q.seed = self._next_plan_seed() if seed is None else int(seed) & _M64
+        q.gamma = float(gamma)
+        returns, actions = eng.plan_eval(start, m, s, int(candidates), q, bool(return_actions))
+        if return_actions:
+            return self._ret(returns, was_np), self._ret(actions, was_np)
+        return self._ret(returns, was_np)
+
+    def plan(self, horizon: int, candidates: int = 512, iterations: int = 5, method: str = "cem", elites: int = 64,
+             temperature: float = 1.0, momentum: float = 0.1, gamma: float = 1.0, mean=None, std=None, min_std: float = 0.0,
+             state=None, seed=None) -> PlanResult:
+        """Sampling-based MPC over the env's own dynamics (the loop of PETS / PlaNet / TD-MPC with the true model):
+        ``iterations`` x (score ``candidates`` sequences of ``horizon`` steps per start state, refit the plan distribution),
+        two launches per iteration.  ``method``: "cem" (refit to the ``elites`` best) or "mppi" (exponential weights with
+        ``temperature``); then ``mean <- momentum mean + (1 - momentum) fit`` and ``std <- max(momentum std + (1 - momentum)
+        fit_std, min_std)``.  ``mean`` / ``std`` [H, B] warm-start the plan (default: the centre of the action box and a
+        quarter of its width; discrete actions: probability 0.5); they are not modified.  ``state=None`` plans from the env's
+        live state (after ``reset()``); ``seed=None`` draws a fresh key from the env's seed and a planner call counter of its own
+        (a later unseeded ``reset()`` draws the same start states with or without planning), iteration i uses
+        ``plan_iteration_seed(seed, i)``.  numpy start states give numpy results.  -> ``PlanResult``."""
+        eng, start, b, was_np, q = self._plan_setup(state)
+        H, iters = int(horizon), int(iterations)
+        if H < 1 or iters < 1:
+            raise ValueError("horizon and iterations must be >= 1")
+        discrete = q.action_kind == _lib.ACTION_DISCRETE_U8
+        lo, hi = (0.0, 1.0) if discrete else (q.action_low, q.action_high)
+        m = self._plan_table(mean, b, "mean", H) if mean is not None else torch.full((H, b), 0.5 * (lo + hi), dtype=self.dtype,
+                                                                                       device=self.device)
+        s = None
+        if not discrete:
+            s = self._plan_table(std, b, "std", H) if std is not None else torch.full((H, b), 0.25 * (hi - lo), dtype=self.dtype,
+                                                                                      device=self.device)
+        methods = {"cem": _lib.PLAN_CEM, "mppi": _lib.PLAN_MPPI}
+        if method not in methods:
+            raise ValueError(f"method must be 'cem' or 'mppi', got {method!r}")
+        q.method, q.elites, q.temperature = methods[method], int(elites), float(temperature)
+        q.momentum, q.min_std, q.gamma = float(momentum), float(min_std), float(gamma)
+        base = self._next_plan_seed() if seed is None else int(seed) & _M64
+        for i in range(iters):
+            q.seed = plan_iteration_seed(base, i)
+            returns, _ = eng.plan_eval(start, m, s, int(candidates), q, False)
+            best_a, best_r = eng.plan_update(returns, m, s, q, want_best=i == iters - 1)
+        r = lambda t: self._ret(t, was_np) if t is not None else None  # noqa: E731
+        return PlanResult(r(m), r(s), r(best_a), r(best_r), r(returns))
+
     # ------------------------------------------------------------------ fused rollouts
     def rollout(self, horizon: int, actions=None, record: bool = False, auto_reset: bool = True, max_episode_steps=None):
         """``horizon`` steps of every env in ONE kernel launch: the batched counterpart of the reference's
@@ -355,9 +455,17 @@ class EmeiEnv(Freezable):
         if seed is not None:
             self._seed = int(seed) & 0xFFFFFFFFFFFFFFFF
             self._reset_count = 0
+            self._plan_count = 0
             self._rollout_epoch = 0
         else:
             self._rollout_epoch += 1
+
+    def _next_plan_seed(self):
+        """A fresh Philox key per unseeded planner call: (seed, planner call counter).  A counter of its own, so planning does
+        not shift the initial-state draws of a later unseeded reset() (``_next_sample_seed``)."""
+        s = (self._seed * 0xC2B2AE3D27D4EB4F + self._plan_count * 0x165667B19E3779F9 + 0x27D4EB2F165667C5) & 0xFFFFFFFFFFFFFFFF
+        self._plan_count += 1
+        return s
 
     def _next_sample_seed(self):
         """A fresh Philox key per sampling call: (seed, call counter) so repeated resets differ but a

@@ -77,6 +77,22 @@ inline int make_rollout(const emei_rollout_params* r, const RolloutIO<R>& io, bo
   return EMEI_OK;
 }
 
+// w[j] for a run-time j without putting the array in local memory
+__device__ __forceinline__ uint32_t select_word(const uint32_t (&w)[4], unsigned j) {
+  const uint32_t lo = (j & 1u) ? w[1] : w[0], hi = (j & 1u) ? w[3] : w[2];
+  return (j & 2u) ? hi : lo;
+}
+
+__device__ __forceinline__ double block_sum_double(double v, double* smem /*[kBlock/32]*/) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  v = warp_sum(v);
+  __syncthreads();
+  if (lane == 0) smem[warp] = v;
+  __syncthreads();
+  double t = lane < kBlock / 32 ? smem[lane] : 0.0;
+  return warp_sum(t);  // valid in every lane of every warp
+}
+
 // Philox key of the reset sample of an env's episode k (include/emei_b200.h)
 __device__ __forceinline__ unsigned long long reset_seed(unsigned long long seed_reset, int k) {
   return seed_reset + static_cast<unsigned long long>(k) * 0xD1B54A32D192ED03ull;

@@ -59,22 +59,6 @@ static __device__ __noinline__ CBRegs rollout_init_charged_ball(float radius, un
   return e;
 }
 
-// w[j] for a run-time j without putting the array in local memory
-__device__ __forceinline__ uint32_t select_word(const uint32_t (&w)[4], unsigned j) {
-  const uint32_t lo = (j & 1u) ? w[1] : w[0], hi = (j & 1u) ? w[3] : w[2];
-  return (j & 2u) ? hi : lo;
-}
-
-__device__ __forceinline__ double block_sum_double(double v, double* smem /*[kBlock/32]*/) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  v = warp_sum(v);
-  __syncthreads();
-  if (lane == 0) smem[warp] = v;
-  __syncthreads();
-  double t = lane < kBlock / 32 ? smem[lane] : 0.0;
-  return warp_sum(t);  // valid in every lane of every warp
-}
-
 // ------------------------------------------------------------------------------------------------
 // env families
 // ------------------------------------------------------------------------------------------------

@@ -28,6 +28,9 @@ _ACTION_KIND = {
     torch.float64: _lib.ACTION_CONTINUOUS_F64,
 }
 
+_KIND_DTYPE = {_lib.ACTION_DISCRETE_U8: torch.uint8, _lib.ACTION_DISCRETE_I32: torch.int32, _lib.ACTION_DISCRETE_I64: torch.int64,
+               _lib.ACTION_CONTINUOUS_F32: torch.float32, _lib.ACTION_CONTINUOUS_F64: torch.float64}
+
 
 def action_rule(env, a: torch.Tensor, continuous: bool) -> torch.Tensor:
     """The dtype and range rule of every action entry point (base_control.py:62-66 for a batch): device tensor ``a`` of
@@ -142,6 +145,32 @@ class Engine:
             rec["timeouts"] = rec["timeouts"].view(torch.bool)
         return rec
 
+    # ---- sampling-based planning (emei_*_plan_eval_* / emei_plan_update_*): the env's own state is never touched
+    def _plan_eval(self, entry: str, state_ptrs, mean: torch.Tensor, std, candidates: int, q: _lib.PlanParams, want_actions: bool):
+        """-> (returns [B, K] float64, actions [H, B, K] in the plan's action type or None) of the candidates drawn around
+        (mean, std) [H, B] from the start states behind ``state_ptrs``."""
+        env = self.env
+        H, B = mean.shape
+        returns = (torch.zeros if H == 0 else torch.empty)((B, candidates), dtype=torch.float64, device=env.device)
+        actions = torch.empty((H, B, candidates), dtype=_KIND_DTYPE[q.action_kind], device=env.device) if want_actions else None
+        self.params.action_kind = q.action_kind
+        env._call(entry, *state_ptrs, mean.data_ptr(), std.data_ptr() if std is not None else None, returns.data_ptr(),
+                  actions.data_ptr() if actions is not None else None, B, candidates, H, ctypes.byref(q), ctypes.byref(self.params),
+                  env._stream())
+        return returns, actions
+
+    def plan_update(self, returns: torch.Tensor, mean: torch.Tensor, std, q: _lib.PlanParams, want_best: bool):
+        """Refit ``mean`` / ``std`` [H, B] in place from ``returns`` [B, K] of the candidates drawn with ``q``
+        (emei_plan_update_*) -> (best_actions [H, B], best_return [B]) when ``want_best``, else (None, None)."""
+        env = self.env
+        H, B = mean.shape
+        best_a = torch.empty((H, B), dtype=_KIND_DTYPE[q.action_kind], device=env.device) if want_best else None
+        best_r = torch.empty((B,), dtype=torch.float64, device=env.device) if want_best else None
+        ptr = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
+        env._call("emei_plan_update", returns.data_ptr(), mean.data_ptr(), ptr(std), ptr(best_a), ptr(best_r), B, returns.shape[1], H,
+                  ctypes.byref(q), env._stream())
+        return best_a, best_r
+
     # freeze/unfreeze: device-side copies of the live state arrays (base_control.py:32-36)
     def snapshot(self) -> tuple:
         snaps = tuple(torch.empty_like(t) for t in self._state_arrays())
@@ -173,6 +202,7 @@ class RowStateEngine(Engine):
         self._jacobian_entry, self._vjp_entry = step_entry + "_jacobian", step_entry + "_vjp"
         self._trajectory_entry = step_entry[: -len("_step")] + "_trajectory"
         self._trajectory_vjp_entry = self._trajectory_entry + "_vjp"
+        self._plan_eval_entry = step_entry[: -len("_step")] + "_plan_eval"
         self._bufs = self._obs = self._out = None
         self._cur = 0
         self.has_state = False
@@ -328,6 +358,17 @@ class RowStateEngine(Engine):
                   g0.data_ptr(), ptr(g_act), b, T, ctypes.byref(self.params), env._stream())
         return g0, g_act
 
+    def plan_start(self, state):
+        """Start states of a plan -> (rows [B, width] on the device, B, came_from_numpy)."""
+        rows, was_np = self.env._to_device(state, self.env.dtype)
+        if rows.dim() != 2 or rows.shape[1] != self.obs_dim:
+            raise ValueError(f"state must be [B, {self.obs_dim}], got {tuple(rows.shape)}")
+        return _aligned16(rows), rows.shape[0], was_np
+
+    def plan_eval(self, rows: torch.Tensor, mean: torch.Tensor, std, candidates: int, q: _lib.PlanParams, want_actions: bool):
+        """``_plan_eval`` from start rows [B, width] (``plan_start``)."""
+        return self._plan_eval(self._plan_eval_entry, [rows.data_ptr()], mean, std, candidates, q, want_actions)
+
 
 class CartPoleEngine(RowStateEngine):
     """cart-pole family (state = observation) + analytic inverted pendulum (emei_cartpole_step_* / emei_ip_step_noisy_*)."""
@@ -442,6 +483,21 @@ class ChargedBallEngine(Engine):
 
     def _state_arrays(self):
         return [self.on_circle, self.circle, self.free]
+
+    def plan_start(self, state):
+        """Start states of a plan, a dict like ``env.state`` or a tuple (on_circle, circle, free) ->
+        ((on_circle uint8 [B], circle [B, 2], free [B, 4]) on the device, B, came_from_numpy)."""
+        env = self.env
+        parts = (state["on_circle"], state["circle_state"], state["free_state"]) if isinstance(state, dict) else tuple(state)
+        on, was_np = env._to_device(parts[0], torch.uint8)
+        b = on.numel()
+        circle = _aligned16(env._to_device(parts[1], env.dtype)[0].reshape(b, 2))
+        free = _aligned16(env._to_device(parts[2], env.dtype)[0].reshape(b, 4))
+        return (on.reshape(b), circle, free), b, was_np
+
+    def plan_eval(self, state: tuple, mean: torch.Tensor, std, candidates: int, q: _lib.PlanParams, want_actions: bool):
+        """``_plan_eval`` from start states (on_circle, circle, free) (``plan_start``)."""
+        return self._plan_eval("emei_charged_ball_plan_eval", [t.data_ptr() for t in state], mean, std, candidates, q, want_actions)
 
 
 def _aligned16(t: torch.Tensor) -> torch.Tensor:

@@ -358,6 +358,80 @@ int emei_charged_ball_rollout_ref_f64(uint8_t* on_circle_io, double* circle_io, 
                                       uint8_t* rec_dones, uint8_t* rec_timeouts, double* stats, int64_t n,
                                       const emei_charged_ball_params* p, const emei_rollout_params* r, emei_stream_t stream);
 
+/* ---- sampling-based MPC over the true dynamics (CEM / MPPI; DESIGN.md 4.10) ------------------------------
+ * One planner iteration is two launches: *_plan_eval_* scores K candidate action sequences of H steps from each of B start
+ * states, emei_plan_update_* refits the [H, B] plan distribution from their returns.  Nothing of the env moves: like the
+ * trajectory entry points this is an open-loop model query (no TimeLimit, resets, state noise or statistics).
+ * Candidate actions: drawn in-kernel from Philox4x32-10 keyed by (seed, (env_offset + b) * 2^32 + k), so results do not
+ * depend on how the start states are sharded:
+ *   continuous kinds: step t uses the Box-Muller pair of block t >> 1 (cos half for even t, sin half for odd t),
+ *     a = clamp(R(mean[t,b] + std[t,b] z)), product and sum rounded in double, clamped in R to [action_low, action_high]
+ *     (a float32 action array in a float64 plan holds that value rounded to float32);
+ *   discrete kinds: step t uses word t & 3 of block t >> 2, a = ((w >> 8) 2^-24 < float(mean[t,b])) ? 1 : 0, mean being the
+ *     probability of action 1 (std unused, may be NULL).
+ * Return R_bk = sum_{t<H} gamma^t r_t in double (ret = ret + disc r_t; disc = disc gamma; each operation rounded on its own);
+ * the reward of the step that terminates counts, later steps do not.  Per step the arithmetic is that of the env's fused
+ * rollout in the same precision (emei_cartpole_rollout_f32 / emei_charged_ball_rollout_f32 for float32 cart-pole, IP and
+ * charged ball, the *_rollout_ref_* / emei_i2p_rollout_* kernels otherwise), so the rewards of a candidate equal a
+ * teacher-forced rollout of its actions bit for bit.  The family params' action_kind is replaced by the plan's. */
+#define EMEI_PLAN_CEM 0
+#define EMEI_PLAN_MPPI 1
+#define EMEI_PLAN_MAX_CANDIDATES 4096
+typedef struct emei_plan_params {
+  uint64_t seed;       /* Philox key of the candidate actions */
+  uint64_t env_offset; /* global id of start state 0 (sharding) */
+  double gamma;        /* discount, in [0, 1] */
+  double temperature;  /* MPPI lambda, > 0 */
+  double momentum;     /* alpha in [0, 1): mean <- alpha mean + (1 - alpha) fit_mean, the same for std */
+  double min_std;      /* std floor, >= 0 */
+  float action_low, action_high; /* continuous kinds: the action box (low <= high) */
+  int32_t method;      /* EMEI_PLAN_CEM | EMEI_PLAN_MPPI */
+  int32_t elites;      /* CEM: E in [1, K] */
+  int32_t action_kind; /* EMEI_ACTION_*: discrete or continuous, and the element type of actions_out / best_actions */
+} emei_plan_params;
+
+/* eval: state0 [B,D] (cart-pole rows, or qpos || qvel with unwrapped angles, as the trajectory entry points take them;
+ * 16-byte aligned) / the charged ball's on_circle [B], circle [B,2], free [B,4] (circle and free 16-byte aligned);
+ * mean, std [H,B] in the real type; returns [B,K] double (written once); actions_out [H,B,K] in the action kind's type,
+ * nullable (so actions_out viewed as [H, B*K] is the actions array of a teacher-forced rollout of B*K envs whose state is
+ * each start repeated K times).  Validation: B < 0, H < 0 or H >= 2^31, K outside [1, 4096] -> EMEI_ERR_BAD_SIZE; NULL
+ * params; the family params as the step entry points check them; the plan params (action kind -> EMEI_ERR_BAD_ACTION_KIND;
+ * method, E outside [1, K] for CEM, temperature <= 0 for MPPI, gamma outside [0, 1], momentum outside [0, 1), min_std < 0,
+ * action_low > action_high -> EMEI_ERR_BAD_PARAM); B == 0 or H == 0 returns EMEI_OK with nothing launched; then NULL state,
+ * mean, returns (std for continuous kinds) and the alignment.  All before any launch. */
+int emei_cartpole_plan_eval_f32(const float* state0, const float* mean, const float* std, double* returns, void* actions_out, int64_t B,
+                                int64_t K, int64_t H, const emei_plan_params* plan, const emei_cartpole_params* p, emei_stream_t stream);
+int emei_cartpole_plan_eval_f64(const double* state0, const double* mean, const double* std, double* returns, void* actions_out,
+                                int64_t B, int64_t K, int64_t H, const emei_plan_params* plan, const emei_cartpole_params* p,
+                                emei_stream_t stream);
+int emei_i2p_plan_eval_f32(const float* state0, const float* mean, const float* std, double* returns, void* actions_out, int64_t B,
+                           int64_t K, int64_t H, const emei_plan_params* plan, const emei_i2p_params* p, emei_stream_t stream);
+int emei_i2p_plan_eval_f64(const double* state0, const double* mean, const double* std, double* returns, void* actions_out, int64_t B,
+                           int64_t K, int64_t H, const emei_plan_params* plan, const emei_i2p_params* p, emei_stream_t stream);
+int emei_charged_ball_plan_eval_f32(const uint8_t* on_circle, const float* circle, const float* free_state, const float* mean,
+                                    const float* std, double* returns, void* actions_out, int64_t B, int64_t K, int64_t H,
+                                    const emei_plan_params* plan, const emei_charged_ball_params* p, emei_stream_t stream);
+int emei_charged_ball_plan_eval_f64(const uint8_t* on_circle, const double* circle, const double* free_state, const double* mean,
+                                    const double* std, double* returns, void* actions_out, int64_t B, int64_t K, int64_t H,
+                                    const emei_plan_params* plan, const emei_charged_ball_params* p, emei_stream_t stream);
+/* update, one CTA per start state; reads returns [B,K], regenerates the chosen candidates' actions from the counters above
+ * (same seed, env_offset and mean / std as the eval call) and refits mean_io / std_io [H,B] in place:
+ *   CEM: the E best candidates under the total order (larger return first, ties to the smaller k, NaN below every number);
+ *        fit_mean = their mean action, fit_std = their population std (discrete: fit_mean = their frequency of action 1);
+ *   MPPI: w_k = exp((R_k - max R) / temperature) / sum (a weight that is not a number counts 0; all 0: uniform);
+ *        fit_mean = sum w a, fit_std = sqrt(sum w (a - fit_mean)^2);
+ *   both: mean <- momentum mean + (1 - momentum) fit_mean (discrete: clamped to [0, 1]);
+ *         std <- max(momentum std + (1 - momentum) fit_std, min_std).
+ * Sums are in double in a fixed order (bit-reproducible); results are rounded once to the real type.  std_io is required
+ * for continuous kinds and unused for discrete ones.  best_actions [H,B] (the action kind's type) and best_return [B]
+ * (double): the argmax candidate under the same order, each nullable.  Validation as the eval entry points, without family
+ * params and alignment.  The update needs nothing but the returns, so a caller may score candidates with a model of its own
+ * (actions_out gives it the actions) and refit with this kernel. */
+int emei_plan_update_f32(const double* returns, float* mean_io, float* std_io, void* best_actions, double* best_return, int64_t B,
+                         int64_t K, int64_t H, const emei_plan_params* plan, emei_stream_t stream);
+int emei_plan_update_f64(const double* returns, double* mean_io, double* std_io, void* best_actions, double* best_return, int64_t B,
+                         int64_t K, int64_t H, const emei_plan_params* plan, emei_stream_t stream);
+
 /* ---- model-based scoring: get_batch_reward + get_batch_terminal fused ------------------------- */
 typedef struct emei_scoring_params {
   int32_t family;                  /* EMEI_* family id */
