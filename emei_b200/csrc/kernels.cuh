@@ -129,9 +129,6 @@ __device__ __forceinline__ void add_state_noise(R (&y)[DIM], const NoiseConsts& 
   }
 }
 
-// One env step on registers: the whole of BaseControlEnv.step for one env (shared by the step kernel and the
-// reference-arithmetic rollout kernel of rollout_ref.cuh: same bits).  drive = the force (cart-pole family,
-// cartpole.py:121-122,142-143) or the raw control value (IP: clamped to ctrlrange like mj_step, then x gear).
 // cos of an observation angle in the double pendulum's scores (the fused step of i2p.cuh and the I2P scoring families share it,
 // so get_batch_reward(obs) equals the step's own reward bit for bit): float32 = the lean kernel of f32math.cuh (|error| <= 7e-8 up to
 // |x| = 1e5, libm beyond and for NaN / Inf), float64 = libm like the oracle.
@@ -143,11 +140,29 @@ __device__ __forceinline__ R cos_obs(R x) {
     return cos(x);
 }
 
+// One env step on registers: the whole of BaseControlEnv.step for one env (shared by the step kernel and the
+// reference-arithmetic rollout kernel of rollout_ref.cuh: same bits).  drive = the force (cart-pole family,
+// cartpole.py:121-122,142-143) or the raw control value (IP: clamped to ctrlrange like mj_step, then x gear).
+//
+// Both precisions take the float64 constants.  The float32 instantiation (the noisy inverted-pendulum step and the
+// reference-arithmetic float32 rollouts) runs the float64 step on the widened state and rounds once.  A float32 angle held
+// between sub-steps and re-evaluated by sincosf is re-rounded at every sub-step (1.5e-5 rad at |theta| = 300), which the
+// accelerations of a fast pole turn into 100+ envelopes of velocity error at freq_rate 4 (DESIGN.md 2).  So the state, the
+// reward and the flags are those of the float64 step (the reference's own precision) rounded to float32, and the
+// observation's angle is the wrap of the stored float32 angle: the value RefCartPole::observation gives for that state.
 template <typename R, bool IP>
-__device__ __forceinline__ void cartpole_env_step(Vec4<R>& y, R drive, const CartPoleConsts<R>& k, const NoiseConsts& z,
+__device__ __forceinline__ void cartpole_env_step(Vec4<R>& y, R drive, const CartPoleConsts<double>& k, const NoiseConsts& z,
                                                   unsigned long long env, unsigned long long substep0, R& rew, bool& notdone,
                                                   Vec4<R>& obs) {
-  if constexpr (!IP) {
+  if constexpr (sizeof(R) == 4) {
+    Vec4<double> yd = {y.x, y.y, y.z, y.w}, od;
+    double rd;
+    cartpole_env_step<double, IP>(yd, static_cast<double>(drive), k, z, env, substep0, rd, notdone, od);
+    y = {static_cast<float>(yd.x), static_cast<float>(yd.y), static_cast<float>(yd.z), static_cast<float>(yd.w)};
+    obs = y;
+    if constexpr (IP) obs.y = static_cast<float>(py_mod(static_cast<double>(y.y) + k.pi, k.two_pi) - k.pi);
+    rew = static_cast<float>(rd);
+  } else if constexpr (!IP) {
     // state = [x, x_dot, theta, theta_dot]; base_control.py:71-74
     const R force = drive;
     for (int sub = 0; sub < k.freq_rate; ++sub) {
@@ -221,7 +236,7 @@ template <typename R, bool IP>
 __global__ void __launch_bounds__(kBlock)
     cartpole_step_kernel(const R* state_in, R* state_out, R* obs_out, const void* __restrict__ action,
                          R* __restrict__ reward, uint8_t* __restrict__ done, double* stats, int64_t n,
-                         const CartPoleConsts<R> k, const NoiseConsts z) {
+                         const CartPoleConsts<double> k, const NoiseConsts z) {
   // persistent grid-stride loop; reward / done partials stay in registers and are reduced once per
   // thread (a per-env shuffle reduction makes streaming kernels MIO-bound, profiles/r01_ncu_full_c4)
   const int64_t stride = static_cast<int64_t>(gridDim.x) * kBlock;
@@ -231,7 +246,7 @@ __global__ void __launch_bounds__(kBlock)
   pdl_wait();
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * kBlock + threadIdx.x; i < n; i += stride) {
     Vec4<R> y = Vec4<R>::load(state_in + 4 * i), obs;
-    const R drive = IP ? load_ctrl<R>(action, i, k.action_kind) : load_force<R>(action, i, k.action_kind, k.force_mag);
+    const R drive = IP ? load_ctrl<R>(action, i, k.action_kind) : load_force<R>(action, i, k.action_kind, static_cast<R>(k.force_mag));
     R rew;
     bool notdone;
     cartpole_env_step<R, IP>(y, drive, k, z, z.env_offset + static_cast<unsigned long long>(i), z.substep0, rew, notdone, obs);
@@ -271,7 +286,7 @@ int cartpole_step(const R* state_in, R* state_out, R* obs_out, const void* actio
       return launch_status();
     }
   }
-  const CartPoleConsts<R> k = make_cartpole_consts<R>(*p);
+  const CartPoleConsts<double> k = make_cartpole_consts<double>(*p);
   const NoiseConsts z = make_noise_consts(noise, p->freq_rate);
   if (p->variant <= EMEI_CARTPOLE_SWINGUP)
     launch_pdl(cartpole_step_kernel<R, false>, resident_grid(cartpole_step_kernel<R, false>, n), kBlock, s, state_in, state_out, obs_out,
@@ -308,9 +323,12 @@ inline ChargedBallConsts<R> make_cb_consts(const emei_charged_ball_params& p) {
   return k;
 }
 
-// charged_ball.py:30-36
+// charged_ball.py:30-36.  float32: the cancellation-free form of the lean kernel (charged_ball_f32.cuh).  asin of the float32
+// quotient loses half its digits as |x| -> scale, and `scale * r + 1e-8f` rounds to scale * r near r = 1, which puts a landing
+// at y = 0 at +-pi/2 instead of 1.4e-4 rad away from it.
 template <typename R>
 __device__ __forceinline__ R cb_get_angle(R x, R y, const ChargedBallConsts<R>& k) {
+  if constexpr (sizeof(R) == 4) return cb_get_angle_f32(x, y, k.r, k.eps, fmaf(k.r, k.r, -1.0f), 2.0f * k.eps * k.r);
   const R scale = sqrt_r(x * x + y * y);
   const R a = asin_r(x / (scale * k.r + k.eps));
   const R angle = (y > R(0)) ? a : (k.pi - a);

@@ -50,7 +50,7 @@ __device__ __forceinline__ void ref_store_action(void* rec, size_t at, int kind,
 template <typename R, bool IP>
 struct RefCartPole {
   using Real = R;
-  using Consts = CartPoleConsts<R>;
+  using Consts = CartPoleConsts<double>;  // both precisions: cartpole_env_step takes the float64 constants
   static constexpr int kObs = 4;
   struct Buffers {
     R* state;
@@ -62,12 +62,12 @@ struct RefCartPole {
   __device__ __forceinline__ static void store(const Regs& e, const Buffers& b, int64_t i) { e.y.store(b.state + 4 * i); }
   __device__ __forceinline__ static void observation(const Regs& e, const Consts& k, R (&o)[kObs]) {
     o[0] = e.y.x, o[1] = e.y.y, o[2] = e.y.z, o[3] = e.y.w;
-    if constexpr (IP) o[1] = py_mod(e.y.y + k.pi, k.two_pi) - k.pi;  // inverted_pendulum.py:45-49
+    if constexpr (IP) o[1] = static_cast<R>(py_mod(static_cast<double>(e.y.y) + k.pi, k.two_pi) - k.pi);  // inverted_pendulum.py:45-49
   }
   __device__ __forceinline__ static R drive(const Consts& k, const void* actions, const RefAction& a, int kind) {
-    if (a.index >= 0) return IP ? load_ctrl<R>(actions, a.index, kind) : load_force<R>(actions, a.index, kind, k.force_mag);
+    if (a.index >= 0) return IP ? load_ctrl<R>(actions, a.index, kind) : load_force<R>(actions, a.index, kind, static_cast<R>(k.force_mag));
     if constexpr (IP) return static_cast<R>(a.value);
-    if (kind <= EMEI_ACTION_DISCRETE_I64) return a.value == 1.0f ? k.force_mag : -k.force_mag;
+    if (kind <= EMEI_ACTION_DISCRETE_I64) return static_cast<R>(a.value == 1.0f ? k.force_mag : -k.force_mag);
     return static_cast<R>(__fmul_rn(static_cast<float>(k.force_mag), a.value));  // load_force's float32 product
   }
   __device__ __forceinline__ static void step(Regs& e, R drv, const Consts& k, const NoiseConsts& z, unsigned long long env,
@@ -303,7 +303,7 @@ int cartpole_rollout_ref(R* state_io, int32_t* ep_step, R* ep_return, int32_t* e
   if (n == 0 || r->horizon == 0) return EMEI_OK;
   EMEI_CHECK_PTR(state_io);
   EMEI_CHECK_ALIGN16(state_io);
-  const CartPoleConsts<R> k = make_cartpole_consts<R>(*p);
+  const CartPoleConsts<double> k = make_cartpole_consts<double>(*p);
   const NoiseConsts z = make_noise_consts(noise, 1);  // substep0 = the env-step counter; the kernel scales by freq_rate
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (ip) {

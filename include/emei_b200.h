@@ -317,12 +317,16 @@ int emei_charged_ball_rollout_f32(uint8_t* on_circle_io, float* circle_io, float
  * function the step kernel calls:
  *   emei_cartpole_rollout_ref_f64 == horizon x emei_cartpole_step_f64   (z == NULL) / emei_ip_step_noisy_f64 (z != NULL)
  *   emei_cartpole_rollout_ref_f32 == horizon x emei_ip_step_noisy_f32   (z != NULL, EMEI_IP_* variants; with z == NULL it
- *        is the plain float32 evaluation of the reference's expressions, NOT the lean emei_cartpole_step_f32 bits --
- *        use emei_cartpole_rollout_f32 for those)
+ *        is the same arithmetic without noise, NOT the lean emei_cartpole_step_f32 bits -- use emei_cartpole_rollout_f32
+ *        for those)
  *   emei_i2p_rollout_{f32,f64}    == horizon x emei_i2p_step_* / emei_i2p_step_noisy_*
- *   emei_charged_ball_rollout_ref_f64 == horizon x emei_charged_ball_step_f64 (the _f32 symbol is the plain float32
- *        evaluation; emei_charged_ball_rollout_f32 is the one that equals emei_charged_ball_step_f32)
- * bit for bit, plus the bookkeeping.  z->step = env-step counter of the FIRST step of the call (step t uses step + t).
+ *   emei_charged_ball_rollout_ref_f64 == horizon x emei_charged_ball_step_f64 (emei_charged_ball_rollout_f32, not the _ref_f32
+ *        symbol, is the one that equals emei_charged_ball_step_f32)
+ * bit for bit, plus the bookkeeping.
+ * Accuracy of the two float32 _ref symbols (and of emei_ip_step_noisy_f32): the float32 envelope of the lean kernels, 1e-5 rel +
+ * 1e-6 abs per teacher-forced step against the float64 reference from the same float32 state, at any angle and freq_rate
+ * (flags exact away from their thresholds).  The cart-pole / IP step runs its sub-steps in float64 on the widened state and
+ * rounds once; the charged ball's landing angle uses the cancellation-free form of the lean kernel.  z->step = env-step counter of the FIRST step of the call (step t uses step + t).
  * In-kernel resets: the arithmetic of emei_init_uniform / emei_init_gaussian / emei_init_charged_ball in this precision
  * with seed = r->seed_reset + episode_index * 0xD1B54A32D192ED03.  Records and episode_return_io have the real type;
  * observations are [T, n, D] with D = 4 (6 for I2P: current_obs, inverted_double_pendulum.py:56-60).

@@ -1368,10 +1368,11 @@ def _noise_seed(seed):
 @pytest.mark.parametrize("fr", (1, 4))
 def test_ip_obs_noise_vs_oracle_and_philox_mirror(dtype, fr):
     """Two consecutive noisy steps against the oracle fed with the Philox mirror's draws (teacher-forced), in both
-    precisions; the (sigma_pos, sigma_vel) tuple form; sharded == unsharded."""
+    precisions, with ip_inputs' unwrapped angles; the (sigma_pos, sigma_vel) tuple form; sharded == unsharded.  float32 is
+    held to the bar of test_c1_protocol_ip_f32_teacher_forced_200_steps (1.0 x the envelope, plus half an ulp32 of the
+    variable per sub-step at freq_rate > 1); test_f32_reference_arithmetic.py covers every variant and the C1 rows."""
     n, kind = 2048, "ip_boundary_swingup"
     st, act = ip_inputs(4001, n)
-    st[: n // 8, 1] /= 30.0
     if dtype == torch.float32:
         st = st.astype(np.float32).astype(np.float64)
     p = O.InvertedPendulumParams()
@@ -1389,11 +1390,13 @@ def test_ip_obs_noise_vs_oracle_and_philox_mirror(dtype, fr):
         if dtype == torch.float64:
             assert close64(got, ref_state, 1e-11)
         else:
-            assert within32(got, ref_state, 1.5).all()
+            big = np.maximum(np.abs(cur), np.abs(ref_state)).astype(np.float32)
+            tol = 1e-6 + 1e-5 * np.abs(ref_state) + (fr * 0.5 * np.spacing(big).astype(np.float64) if fr > 1 else 0.0)
+            assert (np.abs(got - ref_state) / tol).max() <= 1.0, f"worst fraction of the envelope {(np.abs(got - ref_state) / tol).max()}"
         clean, _ = O.ip_step(cur, ctrl, 0.02, fr, True, p, libm=True)
         d = got - clean
         assert 0.5 * sig[0] < d[:, 0].std() and d[:, 2].std() > 0.5 * sig[2]  # the noise is really there
-        assert within32(rew.cpu().numpy(), O.ip_reward(kind, ref_obs), 3.0).all()
+        assert within32(rew.cpu().numpy(), O.ip_reward(kind, ref_obs)).all()
         cur = got
     # sharding: the second half of the batch as its own env with env_offset = n/2 draws the same noise
     half = E.make(IP[kind], freq_rate=fr, num_envs=n // 2, dtype=dtype, obs_noise_params=(0.01, 0.03), env_offset=n // 2)
