@@ -9,6 +9,6 @@ the C ABI in ``include/emei_b200.h``.  There is no CPU fallback.
 __version__ = "0.1.0"
 
 from . import _lib  # noqa: F401  (loads libemei_b200.so; raises if it is missing)
-from .core import EmeiEnv, Freezable, PlanResult, plan_iteration_seed  # noqa: F401
+from .core import EmeiEnv, Freezable, PlanResult, PolicySearchResult, plan_iteration_seed, policy_starts_seed  # noqa: F401
 from .envs import register_env  # noqa: F401
 from .envs.register_env import make, registry, spec  # noqa: F401

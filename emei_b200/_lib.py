@@ -32,6 +32,7 @@ ACTION_DISCRETE_U8, ACTION_DISCRETE_I32, ACTION_DISCRETE_I64, ACTION_CONTINUOUS_
 SUMSQ_WORKSPACE_BYTES = (148 * 8 + 1) * 8  # EMEI_SUMSQ_WORKSPACE_BYTES
 PLAN_CEM, PLAN_MPPI = 0, 1  # EMEI_PLAN_*
 PLAN_MAX_CANDIDATES = 4096  # EMEI_PLAN_MAX_CANDIDATES
+POLICY_MAX_DIRECTIONS, POLICY_MAX_PARAMS = 4096, 8  # EMEI_POLICY_MAX_*
 
 
 class EmeiB200Error(RuntimeError):
@@ -142,6 +143,19 @@ class PlanParams(Structure):
     ]
 
 
+class PolicyParams(Structure):
+    _fields_ = [
+        ("seed", c_uint64),
+        ("gamma", c_double),
+        ("noise", c_double),
+        ("step_size", c_double),
+        ("action_low", c_float),
+        ("action_high", c_float),
+        ("action_kind", c_int32),
+        ("top", c_int32),
+    ]
+
+
 _P = c_void_p
 _PROTOTYPES = {
     # name: (restype, argtypes)
@@ -160,6 +174,9 @@ _PROTOTYPES = {
     "emei_i2p_plan_eval": (c_int, [_P] * 5 + [c_int64] * 3 + [POINTER(PlanParams), POINTER(I2PParams), _P]),
     "emei_charged_ball_plan_eval": (c_int, [_P] * 7 + [c_int64] * 3 + [POINTER(PlanParams), POINTER(ChargedBallParams), _P]),
     "emei_plan_update": (c_int, [_P] * 5 + [c_int64] * 3 + [POINTER(PlanParams), _P]),
+    "emei_cartpole_policy_eval": (c_int, [_P] * 4 + [c_int64] * 3 + [POINTER(PolicyParams), POINTER(CartPoleParams), _P]),
+    "emei_i2p_policy_eval": (c_int, [_P] * 4 + [c_int64] * 3 + [POINTER(PolicyParams), POINTER(I2PParams), _P]),
+    "emei_charged_ball_policy_eval": (c_int, [_P] * 6 + [c_int64] * 3 + [POINTER(PolicyParams), POINTER(ChargedBallParams), _P]),
     "emei_ip_step_noisy": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64, POINTER(CartPoleParams), POINTER(NoiseParams), _P]),
     "emei_i2p_step_noisy": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64, POINTER(I2PParams), POINTER(NoiseParams), _P]),
     "emei_cartpole_rollout_ref": (c_int, [_P] * 12 + [c_int64, POINTER(CartPoleParams), POINTER(RolloutParams), POINTER(NoiseParams), _P]),
@@ -179,6 +196,8 @@ _PROTOTYPES = {
 _PLAIN = {
     "emei_cartpole_rollout_f32": (c_int, [_P] * 12 + [c_int64, POINTER(CartPoleParams), POINTER(RolloutParams), _P]),
     "emei_charged_ball_rollout_f32": (c_int, [_P] * 14 + [c_int64, POINTER(ChargedBallParams), POINTER(RolloutParams), _P]),
+    "emei_policy_perturb": (c_int, [_P, _P, c_int64, c_int64, POINTER(PolicyParams), _P]),
+    "emei_policy_update": (c_int, [_P, _P, _P, c_int64, c_int64, c_int64, POINTER(PolicyParams), _P]),
     "emei_snapshot_copy": (c_int, [_P, _P, c_int64, _P]),
     "emei_records_transpose": (c_int, [_P, _P, c_int64, c_int64, c_int32, _P]),
     "emei_stats_reset": (c_int, [_P, _P]),

@@ -46,6 +46,18 @@ def plan_iteration_seed(seed: int, i: int) -> int:
     """The Philox key of iteration ``i`` of a plan keyed by ``seed``."""
     return (seed * 0xD1B54A32D192ED03 + (i + 1) * 0x9E3779B97F4A7C15) & _M64
 
+PolicySearchResult = namedtuple("PolicySearchResult", "theta returns stats")
+PolicySearchResult.__doc__ = """Result of ``EmeiEnv.policy_search``: the linear policy ``theta`` [P] (float64, P = observation dimension + 1:
+the weights, then the bias), the last iteration's ``returns`` [2N, E] (float64; rows 2k / 2k + 1: theta +- noise delta_k) and
+per iteration ``stats`` [iterations, 4] (float64): the number of directions stepped along, the std of their returns, the best
+direction's max(r+, r-) and the mean of every finite direction return (NaN where there is none)."""
+
+
+def policy_starts_seed(seed: int) -> int:
+    """The Philox key of the start states an iteration keyed by ``seed`` draws (``policy_search``, and
+    ``get_batch_policy_returns`` with ``starts=None``)."""
+    return (seed * 0x9E3779B97F4A7C15 + 0xBF58476D1CE4E5B9) & _M64
+
 
 def _torch_dtype(dtype) -> torch.dtype:
     if isinstance(dtype, torch.dtype):
@@ -84,6 +96,8 @@ class EmeiEnv(Freezable):
         self._seed = 0
         self._reset_count = 0
         self._plan_count = 0  # planner calls since the last explicit seed: keys plan() / get_batch_plan_returns with seed=None
+        self._policy_count = 0  # unseeded policy-search calls since the last explicit seed (policy_search / get_batch_policy_returns)
+        self._sample_key = None  # set: the Philox key of the next initial-state draw instead of the reset stream's (_policy_starts)
         self._rollout_epoch = -1  # resets since the last explicit seed (0 = the seeded one): keys the rollout / noise streams
 
     # ------------------------------------------------------------------ engine protocol (engine.py)
@@ -329,6 +343,99 @@ class EmeiEnv(Freezable):
         r = lambda t: self._ret(t, was_np) if t is not None else None  # noqa: E731
         return PlanResult(r(m), r(s), r(best_a), r(best_r), r(returns))
 
+    # ------------------------------------------------------------------ policy search (linear feedback policies, ARS)
+    def _policy_setup(self):
+        """-> (engine, P, PolicyParams with the action kind and box)."""
+        eng = self._ensure_engine()
+        if eng is None or not hasattr(eng, "policy_eval"):
+            raise NotImplementedError(f"{type(self).__name__}: no policy search, it has no dynamics kernel")
+        q = _lib.PolicyParams()
+        if len(self.action_space.shape) == 0:
+            q.action_kind = _lib.ACTION_DISCRETE_U8
+        else:
+            q.action_kind = _lib.ACTION_CONTINUOUS_F32 if self.dtype == torch.float32 else _lib.ACTION_CONTINUOUS_F64
+            q.action_low, q.action_high = float(self.action_space.low.min()), float(self.action_space.high.max())
+        return eng, int(self.observation_space.shape[0]) + 1, q
+
+    def _policy_starts(self, n: int, key: int):
+        """``n`` start states from the env's initial-state distribution under Philox key ``key``, in the layout ``plan_start``
+        takes; the reset stream's counter does not move."""
+        self._sample_key = key
+        try:
+            return self._sample_init_obs(n) if hasattr(self, "_sample_init_obs") else self.get_batch_init_state(n)
+        finally:
+            self._sample_key = None
+
+    def _policy_horizon(self, horizon) -> int:
+        H = getattr(self, "max_episode_steps", None) if horizon is None else horizon
+        if H is None or int(H) < 1:
+            raise ValueError("horizon must be >= 1 (None: the env's max_episode_steps)")
+        return int(H)
+
+    def get_batch_policy_returns(self, params, starts=None, horizon=None, gamma: float = 1.0, seed=None, return_actions: bool = False):
+        """Closed-loop returns of linear feedback policies in one launch: policy c, ``params[c] = (w_0 .. w_{D-1}, b)`` (float64
+        [C, P] or [P], P = observation dimension + 1), acts ``u = b + sum_j w_j obs_j`` on the observation ``step()`` would
+        return (continuous actions: u clamped to the action box; discrete: ``u > 0``) from each of E start states for
+        ``horizon`` steps (None: ``max_episode_steps``) with the step arithmetic of ``rollout()``.  -> ``returns`` [C, E]
+        float64, the discounted sum of rewards up to and including the step that terminates; with ``return_actions`` also
+        the actions [H, C, E] (``actions.view(H, C*E)`` teacher-forces a rollout of the pairs, candidate-major).
+        ``starts``: start rows [E, D] (qpos || qvel with unwrapped angles, for the pendulums) or the charged ball's state dict;
+        None draws ``num_envs`` starts from the initial-state distribution, keyed by ``seed`` (None: a counter of the policy
+        search's own, so a later unseeded ``reset()`` draws the same states).  The env's state, statistics and initial-state
+        stream are not touched.  numpy in, numpy out."""
+        eng, P, q = self._policy_setup()
+        th, was_np = self._to_device(params, torch.float64)
+        th = th.reshape(1, -1) if th.dim() == 1 else th
+        if th.dim() != 2 or th.shape[1] != P:
+            raise ValueError(f"params must be [C, {P}] or [{P}], got {tuple(th.shape)}")
+        H = self._policy_horizon(horizon)
+        if starts is None:
+            key = self._next_policy_seed() if seed is None else int(seed) & _M64
+            starts = self._policy_starts(self.num_envs, policy_starts_seed(key))
+        start, _, st_np = eng.plan_start(starts)
+        q.gamma = float(gamma)
+        returns, actions = eng.policy_eval(start, th, H, q, bool(return_actions))
+        as_np = was_np or st_np
+        if return_actions:
+            return self._ret(returns, as_np), self._ret(actions, as_np)
+        return self._ret(returns, as_np)
+
+    def policy_search(self, horizon=None, iterations: int = 20, directions: int = 32, top=None, step_size: float = 0.02,
+                      noise: float = 0.03, episodes: int = 16, gamma: float = 1.0, theta=None, seed=None) -> PolicySearchResult:
+        """Random search over linear feedback policies (ARS V1-t, Mania, Guy & Recht 2018) on the env's own dynamics.  Each
+        of ``iterations`` draws ``episodes`` fresh start states from the initial-state distribution, perturbs ``theta``
+        along ``directions`` Gaussian directions (theta +- ``noise`` delta_k), scores the 2N policies closed loop for
+        ``horizon`` steps (None: ``max_episode_steps``) from those starts (the mean discounted return over the episodes),
+        and steps ``theta += step_size / (b sigma_R) sum (r_k+ - r_k-) delta_k`` along the ``top`` (None: all) best
+        directions, sigma_R being the std of their returns.  Four launches per iteration, no host synchronisation.
+        ``theta`` [P] warm-starts the search (default 0) and is not modified; ``seed=None`` draws a fresh key from the env's
+        seed and a counter of the search's own (a later unseeded ``reset()`` draws the same start states with or without a
+        search); iteration i is keyed by ``plan_iteration_seed(seed, i)``.  -> ``PolicySearchResult``; numpy ``theta`` in,
+        numpy out."""
+        eng, P, q = self._policy_setup()
+        H, iters, N = self._policy_horizon(horizon), int(iterations), int(directions)
+        E = int(episodes)
+        if iters < 1 or E < 1:
+            raise ValueError("iterations and episodes must be >= 1")
+        if not 1 <= N <= _lib.POLICY_MAX_DIRECTIONS:
+            raise ValueError(f"directions must be in [1, {_lib.POLICY_MAX_DIRECTIONS}], got {N}")
+        was_np = theta is not None and not isinstance(theta, torch.Tensor)
+        th = torch.zeros(P, dtype=torch.float64, device=self.device) if theta is None else self._to_device(theta, torch.float64)[0]
+        th = th.reshape(-1).clone()
+        if th.numel() != P:
+            raise ValueError(f"theta must have {P} elements, got {th.numel()}")
+        q.top, q.step_size, q.noise, q.gamma = N if top is None else int(top), float(step_size), float(noise), float(gamma)
+        base = self._next_policy_seed() if seed is None else int(seed) & _M64
+        stats = torch.empty((iters, 4), dtype=torch.float64, device=self.device)
+        returns = None
+        for i in range(iters):
+            q.seed = plan_iteration_seed(base, i)
+            start, _, _ = eng.plan_start(self._policy_starts(E, policy_starts_seed(q.seed)))
+            params = eng.policy_perturb(th, N, q)
+            returns, _ = eng.policy_eval(start, params, H, q, False)
+            eng.policy_update(returns, th, q, stats[i])
+        return PolicySearchResult(self._ret(th, was_np), self._ret(returns, was_np), self._ret(stats, was_np))
+
     # ------------------------------------------------------------------ fused rollouts
     def rollout(self, horizon: int, actions=None, record: bool = False, auto_reset: bool = True, max_episode_steps=None):
         """``horizon`` steps of every env in ONE kernel launch: the batched counterpart of the reference's
@@ -456,6 +563,7 @@ class EmeiEnv(Freezable):
             self._seed = int(seed) & 0xFFFFFFFFFFFFFFFF
             self._reset_count = 0
             self._plan_count = 0
+            self._policy_count = 0
             self._rollout_epoch = 0
         else:
             self._rollout_epoch += 1
@@ -467,9 +575,19 @@ class EmeiEnv(Freezable):
         self._plan_count += 1
         return s
 
+    def _next_policy_seed(self):
+        """A fresh Philox key per unseeded policy-search call: (seed, a counter of its own), so searching does not shift the
+        initial-state draws of a later unseeded reset()."""
+        s = (self._seed * 0x94D049BB133111EB + self._policy_count * 0xBF58476D1CE4E5B9 + 0x2545F4914F6CDD1D) & _M64
+        self._policy_count += 1
+        return s
+
     def _next_sample_seed(self):
         """A fresh Philox key per sampling call: (seed, call counter) so repeated resets differ but a
-        given (seed, call index) is reproducible and independent of sharding."""
+        given (seed, call index) is reproducible and independent of sharding.  While ``_sample_key`` is set, that key, with
+        the counter left alone (the policy search's start states)."""
+        if self._sample_key is not None:
+            return self._sample_key
         s = (self._seed * 0x9E3779B97F4A7C15 + self._reset_count * 0xD1B54A32D192ED03) & 0xFFFFFFFFFFFFFFFF
         self._reset_count += 1
         return s

@@ -348,6 +348,7 @@ constexpr uint32_t kPurposeRolloutAction = 4;  // the rollouts' random policy
 constexpr uint32_t kPurposeRolloutReset = 5;   // the float32 rollouts' lean uniform reset
 constexpr uint32_t kPurposeObsNoise = 6;       // per-sub-step state noise (bits 8..: the high word of the block index)
 constexpr uint32_t kPurposePlanAction = 7;     // the planner's candidate actions (plan.cuh)
+constexpr uint32_t kPurposePolicyPerturb = 8;  // the policy search's directions (policy.cuh)
 
 // 53-bit uniform in [0,1) from two 32-bit words (same construction as numpy's next_double)
 __host__ __device__ inline double u01_from_bits(uint32_t hi, uint32_t lo) {

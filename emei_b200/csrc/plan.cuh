@@ -56,15 +56,18 @@ __device__ __forceinline__ unsigned long long plan_env_word(const PlanConsts& c,
   return ((c.env_offset + static_cast<unsigned long long>(b)) << 32) | static_cast<unsigned long long>(k);
 }
 
-// the continuous action from the step's standard normal z: R(mean + std z) in double, then clamped in R; a float32 action
-// array in a float64 plan holds the float32 rounding of that value, and the step consumes what the array holds
+// the continuous action from the step's standard normal z: R(mean + std z) in double, then clamped in R (plan_clamp); a
+// float32 action array in a float64 plan holds the float32 rounding of that value, and the step consumes what the array holds
 template <typename R>
-__device__ __forceinline__ R plan_continuous(R mean, R std, double z, const PlanConsts& c) {
-  R a = static_cast<R>(__dadd_rn(static_cast<double>(mean), __dmul_rn(static_cast<double>(std), z)));
+__device__ __forceinline__ R plan_clamp(R a, const PlanConsts& c) {
   const R lo = static_cast<R>(c.low), hi = static_cast<R>(c.high);
   a = a < lo ? lo : (a > hi ? hi : a);
   if (sizeof(R) == 8 && c.kind == EMEI_ACTION_CONTINUOUS_F32) a = static_cast<R>(static_cast<float>(a));
   return a;
+}
+template <typename R>
+__device__ __forceinline__ R plan_continuous(R mean, R std, double z, const PlanConsts& c) {
+  return plan_clamp<R>(static_cast<R>(__dadd_rn(static_cast<double>(mean), __dmul_rn(static_cast<double>(std), z))), c);
 }
 
 __device__ __forceinline__ float plan_discrete(uint32_t word, float p) {
@@ -108,7 +111,9 @@ __device__ __forceinline__ void plan_store(void* p, int64_t i, int kind, R a) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// families: the start state's load and the rollout's step of one env, given the action value the array would hold
+// families: the start state's load and the rollout's step of one env, given the action value the array would hold; the
+// observation of the start state (observe) and of every state a step reaches (step's o) is the one the env's step()
+// returns there (the closed-loop policies of policy.cuh act on it; the plan eval discards it)
 // ---------------------------------------------------------------------------------------------
 struct PlanRowsF32 {
   const float* rows;
@@ -126,14 +131,24 @@ struct PlanCartPoleF32 {  // the lean float32 step of emei_cartpole_rollout_f32 
   using Regs = float4;
   using State = PlanRowsF32;
   static constexpr int AK = DISC ? EMEI_ACTION_DISCRETE_U8 : EMEI_ACTION_CONTINUOUS_F32;
+  static constexpr int kObs = 4;
   __device__ __forceinline__ static void load(Regs& y, const State& s, int64_t b) { y = reinterpret_cast<const float4*>(s.rows)[b]; }
-  __device__ __forceinline__ static float step(Regs& y, float a, const Consts& k, bool& terminated) {
+  // the observation step() would return in state y (CartPoleDyn::observation)
+  __device__ __forceinline__ static void observe(const Regs& y, const Consts&, float (&o)[kObs]) {
+    o[0] = y.x, o[1] = IP ? wrap_pi_f32(y.y) : y.y, o[2] = y.z, o[3] = y.w;
+  }
+  __device__ __forceinline__ static float step(Regs& y, float a, const Consts& k, bool& terminated, float (&o)[kObs]) {
     float rew;
     bool notdone;
     float4 obs;
     cartpole_step_one<IP, FR>(y, action_to_f_mt<IP, AK>(a, k), ip_flip(IP, k.variant), k, rew, notdone, obs);
     terminated = !notdone;
+    o[0] = obs.x, o[1] = obs.y, o[2] = obs.z, o[3] = obs.w;
     return rew;
+  }
+  __device__ __forceinline__ static float step(Regs& y, float a, const Consts& k, bool& terminated) {
+    float o[kObs];
+    return step(y, a, k, terminated, o);
   }
 };
 
@@ -152,9 +167,19 @@ struct PlanChargedBallF32 {  // the load and step of ChargedBallDyn (emei_charge
     e.f = reinterpret_cast<const float4*>(s.free_state)[b];
     cb_prepare(e);
   }
-  __device__ __forceinline__ static float step(Regs& e, float a, const Consts& k, bool& terminated) {
+  static constexpr int kObs = 4;
+  __device__ __forceinline__ static void observe(const Regs& e, const Consts&, float (&o)[kObs]) {
+    o[0] = e.f.x, o[1] = e.f.y, o[2] = e.f.z, o[3] = e.f.w;  // charged_ball.py:96-97
+  }
+  __device__ __forceinline__ static float step(Regs& e, float a, const Consts& k, bool& terminated, float (&o)[kObs]) {
     terminated = false;  // charged_ball.py:110-111
-    return cb_env_step<FR>(e, cb_field<AK>(a, k), k);
+    const float rew = cb_env_step<FR>(e, cb_field<AK>(a, k), k);
+    observe(e, k, o);
+    return rew;
+  }
+  __device__ __forceinline__ static float step(Regs& e, float a, const Consts& k, bool& terminated) {
+    float o[kObs];
+    return step(e, a, k, terminated, o);
   }
 };
 
@@ -167,16 +192,22 @@ struct PlanRef {
   using State = typename Fam::Buffers;
   using ActC = std::conditional_t<DISC, uint8_t, Real>;  // the element the drive reads, as a teacher-forced rollout does
   static constexpr int AK = DISC ? EMEI_ACTION_DISCRETE_U8 : (sizeof(Real) == 4 ? EMEI_ACTION_CONTINUOUS_F32 : EMEI_ACTION_CONTINUOUS_F64);
+  static constexpr int kObs = Fam::kObs;
   __device__ __forceinline__ static void load(Regs& e, const State& s, int64_t b) { Fam::load(e, s, b); }
-  __device__ __forceinline__ static Real step(Regs& e, Real a, const Consts& k, bool& terminated) {
+  __device__ __forceinline__ static void observe(const Regs& e, const Consts& k, Real (&o)[kObs]) { Fam::observation(e, k, o); }
+  __device__ __forceinline__ static Real step(Regs& e, Real a, const Consts& k, bool& terminated, Real (&o)[kObs]) {
     const ActC av = static_cast<ActC>(a);
     RefAction ra;
     ra.value = 0.f;
     ra.index = 0;
     const NoiseConsts z = {};
-    Real rew, o[Fam::kObs];
+    Real rew;
     Fam::step(e, Fam::drive(k, &av, ra, AK), k, z, 0ull, 0ull, rew, terminated, o);
     return rew;
+  }
+  __device__ __forceinline__ static Real step(Regs& e, Real a, const Consts& k, bool& terminated) {
+    Real o[kObs];
+    return step(e, a, k, terminated, o);
   }
 };
 
@@ -369,6 +400,27 @@ __device__ __forceinline__ bool plan_before(unsigned long long ka, int ia, unsig
   return ka > kb || (ka == kb && ia < ib);
 }
 
+// Sorts the Kp (a power of two) pairs (s_key, s_idx) of shared memory into plan_before order by a bitonic network.  Called by
+// every thread of the CTA; ends on a barrier.
+__device__ __forceinline__ void plan_sort(unsigned long long* s_key, uint16_t* s_idx, int Kp) {
+  const int tid = threadIdx.x;
+  for (int size = 2; size <= Kp; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int i = tid; i < (Kp >> 1); i += kBlock) {
+        const int lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
+        const unsigned long long kl = s_key[lo], kh = s_key[hi];
+        const int il = s_idx[lo], ih = s_idx[hi];
+        const bool swap = (lo & size) == 0 ? plan_before(kh, ih, kl, il) : plan_before(kl, il, kh, ih);
+        if (swap) {
+          s_key[lo] = kh, s_key[hi] = kl;
+          s_idx[lo] = static_cast<uint16_t>(ih), s_idx[hi] = static_cast<uint16_t>(il);
+        }
+      }
+      __syncthreads();
+    }
+  }
+}
+
 // The refit of start state b, one warp per Philox block of steps (S = 4 discrete / 2 continuous steps per block).
 template <typename R, bool DISC>
 __device__ __forceinline__ void plan_refit(R* mean_io, R* std_io, int64_t B, int64_t b, int64_t H, int K, int L, double W, bool cem,
@@ -478,21 +530,7 @@ __global__ void __launch_bounds__(kBlock)
     const int best = s_best;
     // ---- selection: CEM sorts (key desc, index asc) by a bitonic network; MPPI forms exp((R - max R) / lambda)
     if (cem) {
-      for (int size = 2; size <= Kp; size <<= 1) {
-        for (int stride = size >> 1; stride > 0; stride >>= 1) {
-          for (int i = tid; i < (Kp >> 1); i += kBlock) {
-            const int lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
-            const unsigned long long kl = s_key[lo], kh = s_key[hi];
-            const int il = s_idx[lo], ih = s_idx[hi];
-            const bool swap = (lo & size) == 0 ? plan_before(kh, ih, kl, il) : plan_before(kl, il, kh, ih);
-            if (swap) {
-              s_key[lo] = kh, s_key[hi] = kl;
-              s_idx[lo] = static_cast<uint16_t>(ih), s_idx[hi] = static_cast<uint16_t>(il);
-            }
-          }
-          __syncthreads();
-        }
-      }
+      plan_sort(s_key, s_idx, Kp);
     } else {
       const double rmax = r[best];
       double part = 0.0;

@@ -171,6 +171,35 @@ class Engine:
                   ctypes.byref(q), env._stream())
         return best_a, best_r
 
+    # ---- policy search (emei_*_policy_eval_* / emei_policy_perturb / emei_policy_update): the env's own state is never touched
+    def _policy_eval(self, entry: str, state_ptrs, E: int, params: torch.Tensor, H: int, q: _lib.PolicyParams, want_actions: bool):
+        """-> (returns [C, E] float64, actions [H, C, E] in the policy's action type or None) of the linear policies
+        ``params`` [C, P] (float64, contiguous) run closed loop for H steps from the E start states behind ``state_ptrs``."""
+        env = self.env
+        C = params.shape[0]
+        returns = (torch.zeros if H == 0 else torch.empty)((C, E), dtype=torch.float64, device=env.device)
+        actions = torch.empty((H, C, E), dtype=_KIND_DTYPE[q.action_kind], device=env.device) if want_actions else None
+        self.params.action_kind = q.action_kind
+        env._call(entry, *state_ptrs, params.data_ptr(), returns.data_ptr(), actions.data_ptr() if actions is not None else None, C, E,
+                  H, ctypes.byref(q), ctypes.byref(self.params), env._stream())
+        return returns, actions
+
+    def policy_perturb(self, theta: torch.Tensor, directions: int, q: _lib.PolicyParams) -> torch.Tensor:
+        """-> params [2N, P] float64: theta +- noise delta_k of the directions keyed by ``q.seed`` (emei_policy_perturb)."""
+        env = self.env
+        params = torch.empty((2 * directions, theta.numel()), dtype=torch.float64, device=env.device)
+        with torch.cuda.device(env.device):
+            _lib.call("emei_policy_perturb", theta.data_ptr(), params.data_ptr(), directions, theta.numel(), ctypes.byref(q), env._stream())
+        return params
+
+    def policy_update(self, returns: torch.Tensor, theta: torch.Tensor, q: _lib.PolicyParams, stats=None):
+        """Step ``theta`` [P] (float64) in place along the ``q.top`` best of the directions behind ``returns`` [2N, E]
+        (emei_policy_update); ``stats``: a device double[4] to write, or None."""
+        env = self.env
+        with torch.cuda.device(env.device):
+            _lib.call("emei_policy_update", returns.data_ptr(), theta.data_ptr(), stats.data_ptr() if stats is not None else None,
+                      returns.shape[0] // 2, returns.shape[1], theta.numel(), ctypes.byref(q), env._stream())
+
     # freeze/unfreeze: device-side copies of the live state arrays (base_control.py:32-36)
     def snapshot(self) -> tuple:
         snaps = tuple(torch.empty_like(t) for t in self._state_arrays())
@@ -203,6 +232,7 @@ class RowStateEngine(Engine):
         self._trajectory_entry = step_entry[: -len("_step")] + "_trajectory"
         self._trajectory_vjp_entry = self._trajectory_entry + "_vjp"
         self._plan_eval_entry = step_entry[: -len("_step")] + "_plan_eval"
+        self._policy_eval_entry = step_entry[: -len("_step")] + "_policy_eval"
         self._bufs = self._obs = self._out = None
         self._cur = 0
         self.has_state = False
@@ -369,6 +399,10 @@ class RowStateEngine(Engine):
         """``_plan_eval`` from start rows [B, width] (``plan_start``)."""
         return self._plan_eval(self._plan_eval_entry, [rows.data_ptr()], mean, std, candidates, q, want_actions)
 
+    def policy_eval(self, rows: torch.Tensor, params: torch.Tensor, H: int, q: _lib.PolicyParams, want_actions: bool):
+        """``_policy_eval`` from start rows [E, width] (``plan_start``)."""
+        return self._policy_eval(self._policy_eval_entry, [rows.data_ptr()], rows.shape[0], params, H, q, want_actions)
+
 
 class CartPoleEngine(RowStateEngine):
     """cart-pole family (state = observation) + analytic inverted pendulum (emei_cartpole_step_* / emei_ip_step_noisy_*)."""
@@ -498,6 +532,11 @@ class ChargedBallEngine(Engine):
     def plan_eval(self, state: tuple, mean: torch.Tensor, std, candidates: int, q: _lib.PlanParams, want_actions: bool):
         """``_plan_eval`` from start states (on_circle, circle, free) (``plan_start``)."""
         return self._plan_eval("emei_charged_ball_plan_eval", [t.data_ptr() for t in state], mean, std, candidates, q, want_actions)
+
+    def policy_eval(self, state: tuple, params: torch.Tensor, H: int, q: _lib.PolicyParams, want_actions: bool):
+        """``_policy_eval`` from start states (on_circle, circle, free) (``plan_start``)."""
+        return self._policy_eval("emei_charged_ball_policy_eval", [t.data_ptr() for t in state], state[0].shape[0], params, H, q,
+                                 want_actions)
 
 
 def _aligned16(t: torch.Tensor) -> torch.Tensor:

@@ -436,6 +436,72 @@ int emei_plan_update_f32(const double* returns, float* mean_io, float* std_io, v
 int emei_plan_update_f64(const double* returns, double* mean_io, double* std_io, void* best_actions, double* best_return, int64_t B,
                          int64_t K, int64_t H, const emei_plan_params* plan, emei_stream_t stream);
 
+/* ---- policy search over the true dynamics: linear feedback policies, ARS (DESIGN.md 4.11) ------------------------
+ * A policy of an env with observation dimension D (cart-pole, IP, charged ball: 4; I2P: 6) is theta = (w_0 .. w_{D-1}, c), P = D + 1
+ * doubles.  At every step it acts on the observation the env's step() returns in that state (IP: the wrapped angle; I2P: the
+ * reference's (theta + pi) % 2 * pi - pi; charged ball: the free state; the first action: the start state's observation):
+ *   u = c; u = u + w_j double(obs_j) for j = 0 .. D-1, each product and sum rounded on its own (no contraction);
+ *   continuous kinds: a = clamp(R(u)) to [action_low, action_high], clamped in R (a float32 action array in a float64 eval holds
+ *     that value rounded to float32); discrete kinds: a = u > 0 ? 1 : 0 (NaN: 0).
+ * One ARS iteration (Mania, Guy & Recht 2018, V1-t) is emei_policy_perturb (2N candidates around theta), *_policy_eval_* (their
+ * returns from E start states) and emei_policy_update (the step along the b best directions).  Nothing of the env moves. */
+#define EMEI_POLICY_MAX_DIRECTIONS 4096
+#define EMEI_POLICY_MAX_PARAMS 8
+typedef struct emei_policy_params {
+  uint64_t seed;                 /* Philox key of the directions delta_k (perturb / update) */
+  double gamma;                  /* eval: discount, in [0, 1] */
+  double noise;                  /* perturb: nu, finite and >= 0 */
+  double step_size;              /* update: alpha, finite */
+  float action_low, action_high; /* eval, continuous kinds: the action box (low <= high) */
+  int32_t action_kind;           /* eval: EMEI_ACTION_*, discrete or continuous and the element type of actions_out */
+  int32_t top;                   /* update: b, the number of directions stepped along, in [1, N] */
+} emei_policy_params;
+
+/* eval: params [C,P] double (P = D + 1); start states as the plan eval takes them: state0 [E,D] (16-byte aligned; angles
+ * unwrapped) / the charged ball's on_circle [E], circle [E,2], free [E,4] (circle and free 16-byte aligned).  Every (c, e) runs
+ * closed loop from start e for H steps; returns [C,E] double = sum_{t<H} gamma^t r_t in double (ret = ret + disc r_t; disc =
+ * disc gamma), the reward of the step that terminates counts, later steps do not; no TimeLimit, reset or noise.  actions_out
+ * [H,C,E] in the action kind's type, nullable; when given, a pair keeps stepping after it terminates, so actions_out viewed as
+ * [H, C*E] teacher-forces a rollout of C*E envs (start e of candidate c at row c*E + e, auto_reset off, no TimeLimit) whose
+ * rewards and observations are the eval's bit for bit.  Per step the arithmetic is the plan eval's, that of the env's own
+ * rollout in that precision.  The family params' action_kind is replaced by the policy's.
+ * Validation, in order: C, E < 0 or > 2^31, H < 0 or >= 2^31 -> EMEI_ERR_BAD_SIZE; NULL policy / family params; the family
+ * params; action kind (EMEI_ERR_BAD_ACTION_KIND; the double pendulum's entry points refuse discrete kinds too), gamma outside
+ * [0, 1] or action_low > action_high for a continuous kind -> EMEI_ERR_BAD_PARAM; C, E or H == 0 returns EMEI_OK with
+ * nothing launched; then NULL state, params, returns and the alignment.  All before any launch. */
+int emei_cartpole_policy_eval_f32(const float* state0, const double* params, double* returns, void* actions_out, int64_t C, int64_t E,
+                                  int64_t H, const emei_policy_params* policy, const emei_cartpole_params* p, emei_stream_t stream);
+int emei_cartpole_policy_eval_f64(const double* state0, const double* params, double* returns, void* actions_out, int64_t C, int64_t E,
+                                  int64_t H, const emei_policy_params* policy, const emei_cartpole_params* p, emei_stream_t stream);
+int emei_i2p_policy_eval_f32(const float* state0, const double* params, double* returns, void* actions_out, int64_t C, int64_t E,
+                             int64_t H, const emei_policy_params* policy, const emei_i2p_params* p, emei_stream_t stream);
+int emei_i2p_policy_eval_f64(const double* state0, const double* params, double* returns, void* actions_out, int64_t C, int64_t E,
+                             int64_t H, const emei_policy_params* policy, const emei_i2p_params* p, emei_stream_t stream);
+int emei_charged_ball_policy_eval_f32(const uint8_t* on_circle, const float* circle, const float* free_state, const double* params,
+                                      double* returns, void* actions_out, int64_t C, int64_t E, int64_t H,
+                                      const emei_policy_params* policy, const emei_charged_ball_params* p, emei_stream_t stream);
+int emei_charged_ball_policy_eval_f64(const uint8_t* on_circle, const double* circle, const double* free_state, const double* params,
+                                      double* returns, void* actions_out, int64_t C, int64_t E, int64_t H,
+                                      const emei_policy_params* policy, const emei_charged_ball_params* p, emei_stream_t stream);
+/* perturb: direction k < N draws delta_k in R^P from Philox4x32-10 keyed by (seed, k) with purpose word 8: block j gives
+ * delta_{2j} = rad cs and delta_{2j+1} = rad sn of the Box-Muller pair (the library's sampler).  Writes params [2N,P]:
+ * params[2k] = theta + nu delta_k, params[2k+1] = theta - nu delta_k, each element one rounded product and one rounded sum.
+ * theta [P] double.  Validation: N outside [1, 4096] or P outside [1, 8] -> EMEI_ERR_BAD_SIZE; NULL policy params; noise not
+ * finite or < 0 -> EMEI_ERR_BAD_PARAM; NULL theta / params. */
+int emei_policy_perturb(const double* theta, double* params, int64_t N, int64_t P, const emei_policy_params* policy,
+                        emei_stream_t stream);
+/* update (one CTA): r_k+ / r_k- = the mean over e (ascending, in double) of returns [2N,E] rows 2k / 2k+1.  Direction k is
+ * eligible when both are finite; the b' = min(top, #eligible) eligible directions with the largest max(r_k+, r_k-) (ties to the
+ * smaller k) give sigma_R, the population std of their 2b' returns, and
+ *   theta <- theta + step_size / (b' sigma_R) sum_k (r_k+ - r_k-) delta_k
+ * with delta_k regenerated from (seed, k).  When b' = 0 or sigma_R is not a finite number > 0, theta is unchanged.  Sums run in a fixed
+ * order (bit-reproducible).  stats double[4], nullable: b', sigma_R, the best eligible max(r_k+, r_k-) and the mean of every
+ * finite r_k+- (NaN where there is none).  Validation: N outside [1, 4096], E outside [1, 2^31] or P outside [1, 8] ->
+ * EMEI_ERR_BAD_SIZE; NULL policy params; top outside [1, N] or step_size not finite -> EMEI_ERR_BAD_PARAM; NULL returns /
+ * theta_io. */
+int emei_policy_update(const double* returns, double* theta_io, double* stats, int64_t N, int64_t E, int64_t P,
+                       const emei_policy_params* policy, emei_stream_t stream);
+
 /* ---- model-based scoring: get_batch_reward + get_batch_terminal fused ------------------------- */
 typedef struct emei_scoring_params {
   int32_t family;                  /* EMEI_* family id */
